@@ -588,6 +588,11 @@ static void gcc_sort(srt *a, long n) {
 
 /* exposed for unit tests */
 void orc_hash_order(const uint64_t *keys, long n, long *order) { hash_order(keys, n, order); }
+long orc_bkt_chain(uint64_t *out, long cap) {
+    long n = (long)(sizeof(BKT_CHAIN) / sizeof(BKT_CHAIN[0]));
+    for (long i = 0; i < n && i < cap; i++) out[i] = BKT_CHAIN[i];
+    return n;
+}
 void orc_gcc_sort(const float *w, long n, long *order_inout) {
     srt *a = (srt *)malloc((n + 1) * sizeof(srt));
     for (long i = 0; i < n; i++) { a[i].w = w[order_inout[i]]; a[i].id = order_inout[i]; }

@@ -17,6 +17,10 @@ def load(name):
     meta = json.loads(bytes(z["meta"]).decode())
     batch = {k[3:]: np.ascontiguousarray(z[k]) for k in z.files if k.startswith("in_")}
     ref = {k[4:]: z[k] for k in z.files if k.startswith("ref_")}
+    return meta, batch, _finish_ref(ref, batch)
+
+
+def _finish_ref(ref, batch):
     n = batch["n_mod"].size
     seqs = bytes(ref["best_sequence"]).decode().split("\n")
     if len(seqs) != n:          # all-empty edge: "".split -> ['']
@@ -24,7 +28,18 @@ def load(name):
     ref["best_sequence"] = seqs
     ref["iso_off"] = np.concatenate([[0], np.cumsum(ref["n_iso"])]).astype(np.int64)
     ref["mod_off"] = np.concatenate([[0], np.cumsum(batch["n_mod"])]).astype(np.int64)
-    return meta, batch, ref
+    return ref
+
+
+def oracle_ref(meta, batch):
+    """the C oracle run live over a host batch -> reference results in the layout load() returns (whole pep_scores
+    tables included), for test_gpu_parity.check_against_ref"""
+    import sys
+    sys.path.insert(0, GOLDEN_DIR)
+    import make_golden
+    from oracle.cscorer import OraclePyAscore
+    ref = make_golden.run_reference(meta["scorer"], meta["neutral_losses"], batch, OraclePyAscore)
+    return _finish_ref(ref, batch)
 
 
 def ref_alt(ref, i, j):

@@ -45,8 +45,10 @@ def batch_from_psms(psms):
                 aux_mass=np.concatenate(am) if am else np.zeros(0, np.float32))
 
 
-def run_reference(scorer_kw, neutral_losses, batch):
-    R = RefPyAscore(**scorer_kw)
+def run_reference(scorer_kw, neutral_losses, batch, scorer_cls=RefPyAscore):
+    """score every PSM of `batch` with the compiled reference (or another class with its surface, such as
+    oracle.cscorer.OraclePyAscore) -> per-PSM results and the whole pep_scores table in golden layout"""
+    R = scorer_cls(**scorer_kw)
     for g, m in neutral_losses:
         R.add_neutral_loss(g, m)
     n = batch["n_mod"].size
