@@ -35,9 +35,18 @@ static thread_local std::string g_create_error;
 
 namespace {
 
-struct DevBuf {
+template <cudaError_t (*Free)(void*)>
+struct OwnedMem {            // a CUDA allocation freed with its owner
     void* p = nullptr;
     size_t cap = 0;
+    OwnedMem() = default;
+    OwnedMem(OwnedMem&& o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    OwnedMem& operator=(OwnedMem&& o) noexcept { std::swap(p, o.p); std::swap(cap, o.cap); return *this; }
+    ~OwnedMem() { if (p) Free(p); }
+    template <class T> T* as() const { return (T*)p; }
+};
+
+struct DevBuf : OwnedMem<cudaFree> {
     cudaError_t ensure(size_t bytes) {
         if (bytes <= cap) return cudaSuccess;
         if (p) { cudaError_t e = cudaFree(p); p = nullptr; cap = 0; if (e != cudaSuccess) return e; }
@@ -47,15 +56,17 @@ struct DevBuf {
         if (e == cudaSuccess) cap = want;
         return e;
     }
-    void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
-    template <class T> T* as() const { return (T*)p; }
 };
 
-struct TmpBuf : DevBuf {     // function-local scratch: freed on every return path
-    TmpBuf() = default;
-    TmpBuf(const TmpBuf&) = delete;
-    TmpBuf& operator=(const TmpBuf&) = delete;
-    ~TmpBuf() { release(); }
+struct PinnedBuf : OwnedMem<cudaFreeHost> {     // page-locked host memory
+    cudaError_t ensure(size_t bytes) {
+        if (bytes <= cap) return cudaSuccess;
+        if (p) { cudaFreeHost(p); p = nullptr; cap = 0; }
+        const size_t want = bytes + bytes / 2 + 4096;
+        cudaError_t e = cudaMallocHost(&p, want);
+        if (e == cudaSuccess) cap = want;
+        return e;
+    }
 };
 
 struct PlanTotals {          // device -> host after planning a chunk
@@ -71,37 +82,19 @@ struct Slot {                // per-stream working set
     // staged inputs
     DevBuf spec_off, mz, inten, inten32, psm_spec, pep_off, pep, n_mod, max_charge, aux_off, aux_pos, aux_mass, mod_off;
     // K1
-    DevBuf rpk, rmz, rrank, rcount, ctab, chead, g_bin, g_tmp;
+    DevBuf rpk, rcount, ctab, chead, g_bin, g_tmp;
     // plan
     DevBuf psm_S, psm_status, psm_I, psm_units, iso_off, unit_off, unit_psm, totals, cub_tmp;
     // K2/K3
     DevBuf iso_lo, iso_hi, iso_n, iso_w, g_sort, g_lr, g_lists, lookups, sched, best_idx, mod_psm, tie, generic_list, generic_count, work_key, work_key2, work_val, work_sorted, rest_list, item_cnt, item_off, gen_flag, asc_cursor;
     // staged outputs
     DevBuf o_sig, o_score, o_niso, o_nsites, o_asc, o_alt, o_status;
-    PlanTotals* h_totals = nullptr;      // pinned
-    unsigned long long* h_lookups = nullptr;
+    PinnedBuf h_totals, h_lookups;       // PlanTotals, unsigned long long
     // small host batches (a single PyAscore.score call): every input array packed into one pinned block and copied
     // with one transfer, every result array read back with one; the user's (pageable) arrays are touched by memcpy only
     DevBuf d_pack, d_opack, mz32, esc, escoff, bin_list, bin_list_n;
-    unsigned char* h_pack = nullptr; size_t h_pack_cap = 0;
-    unsigned char* h_opack = nullptr; size_t h_opack_cap = 0;
+    PinnedBuf h_pack, h_opack;
     cudaEvent_t ev_plan = nullptr;
-    void release() {
-        DevBuf* all[] = {&spec_off, &mz, &inten, &inten32, &psm_spec, &pep_off, &pep, &n_mod, &max_charge, &aux_off, &aux_pos,
-                         &aux_mass, &mod_off, &rpk, &rmz, &rrank, &rcount, &ctab, &chead, &g_bin, &g_tmp, &psm_S, &psm_status, &psm_I,
-                         &psm_units, &iso_off, &unit_off, &unit_psm, &totals, &cub_tmp, &iso_lo, &iso_hi, &iso_n,
-                         &iso_w, &g_sort, &g_lr, &g_lists, &lookups, &sched, &best_idx, &mod_psm, &tie, &generic_list, &generic_count, &work_key, &work_key2, &work_val, &work_sorted, &rest_list, &item_cnt, &item_off, &gen_flag, &asc_cursor, &d_pack, &d_opack, &mz32, &esc, &escoff, &bin_list, &bin_list_n, &o_sig, &o_score, &o_niso, &o_nsites, &o_asc, &o_alt,
-                         &o_status};
-        for (DevBuf* b : all) b->release();
-        if (h_pack) cudaFreeHost(h_pack);
-        if (h_opack) cudaFreeHost(h_opack);
-        h_pack = h_opack = nullptr; h_pack_cap = h_opack_cap = 0;
-        if (h_totals) cudaFreeHost(h_totals);
-        if (h_lookups) cudaFreeHost(h_lookups);
-        if (ev_plan) cudaEventDestroy(ev_plan);
-        if (st) cudaStreamDestroy(st);
-        h_totals = nullptr; h_lookups = nullptr; ev_plan = nullptr; st = nullptr;
-    }
 };
 
 struct ChunkView {           // device-side views of the chunk in flight (kept for fetch calls)
@@ -201,21 +194,14 @@ struct HostPool {
 };
 
 struct NarrowStage {          // one of three rotating staging sets of the narrowing pass (chunk c uses set c % 3)
-    float* h_mz32 = nullptr; size_t h_mz32_cap = 0;        // pinned: narrowed m/z of the chunk,
-    double* h_esc = nullptr; size_t h_esc_cap = 0;         //   exact copies of the spectra that need them,
-    int32_t* h_escoff = nullptr; size_t h_escoff_cap = 0;  //   their per-spectrum offsets (-1: none)
+    PinnedBuf h_mz32;                                      // float: narrowed m/z of the chunk,
+    PinnedBuf h_esc;                                       //   double: exact copies of the spectra that need them,
+    PinnedBuf h_escoff;                                    //   int32_t: their per-spectrum offsets (-1: none)
     std::vector<uint8_t> flags;
     cudaEvent_t ev = nullptr;                              // the copies out of this set are done
     bool busy = false;                                     // tasks in flight on the pool
     int64_t s0 = 0, ns = 0, peak_lo = 0, npk = 0, n_esc = 0, n_flag = 0;
     bool ok = false;
-    void release() {
-        if (h_mz32) cudaFreeHost(h_mz32);
-        if (h_esc) cudaFreeHost(h_esc);
-        if (h_escoff) cudaFreeHost(h_escoff);
-        if (ev) cudaEventDestroy(ev);
-        h_mz32 = nullptr; h_esc = nullptr; h_escoff = nullptr; ev = nullptr; h_mz32_cap = h_esc_cap = h_escoff_cap = 0;
-    }
 };
 
 struct pa_scorer {
@@ -367,10 +353,6 @@ static float residue_mass_host(char c) {
 }
 
 // ---- neutral-loss variant table -----------------------------------------------------------------
-// State = capped multiplicity (0,1,2) of each distinct loss mass on the stack, 2 bits per mass.
-// For every state: PowerSetSum(stack, 2) of cpp/Util.cpp:89-160 -- sums of <=2 stack elements in
-// float32, sorted ascending, de-duplicated by exact equality.  Float addition commutes, so the
-// multiset fixes the result.
 // cpp/Util.cpp:89-160 (PowerSetSum): float32 sums of the subsets of `target` with at most max_depth
 // elements, generated in the reference's recursion order (each sum = parent + element), then sorted
 // and de-duplicated by exact equality.  max_depth is clamped to the target size; 0 then means "no
@@ -398,7 +380,6 @@ static void power_set_sums(const std::vector<float>& target, size_t max_depth, s
     sums.erase(std::unique(sums.begin(), sums.end()), sums.end());
 }
 
-// ---- neutral-loss variant table -----------------------------------------------------------------
 // State = capped multiplicity (0,1,2) of each distinct loss mass on the stack, 2 bits per mass.
 // For every state: PowerSetSum(stack, 2) of the residues' loss stack.  Only the multiset of the stack
 // matters (sums of <= 2 elements commute, and a third copy of a mass adds no new sum).
@@ -503,7 +484,7 @@ static int ensure_table(pa_scorer* s, int n_max) {
     if (want < n_max) return fail(s, PA_ERR_UNSUPPORTED, "score table beyond %d trials", PA_MAX_FRAGMENTS);
     CK(cudaDeviceSynchronize());
     size_t entries = ((size_t)want + 1) * ((size_t)want + 2) / 2;
-    TmpBuf nt;
+    DevBuf nt;
     CK(nt.ensure(entries * PA_N_TOP * sizeof(float)));
     std::vector<double> logd(want + 2);
     logd[0] = 0.;
@@ -526,9 +507,7 @@ static int ensure_table(pa_scorer* s, int n_max) {
     k_tail_table<<<rows, 128, (want + 2) * sizeof(float)>>>(a, n0, want);
     CK(cudaGetLastError());
     CK(cudaDeviceSynchronize());
-    s->d_T.release();
-    s->d_T.p = nt.p; s->d_T.cap = nt.cap;
-    nt.p = nullptr; nt.cap = 0;              // ownership moved to the scorer
+    s->d_T = std::move(nt);                  // (nt takes the old table and frees it)
     s->table_n = want;
     s->cfg.T = s->d_T.as<float>();
     s->cfg.table_n = want;
@@ -693,8 +672,8 @@ static int create_scorer(float bin_size, int n_top, const char* mod_group, float
         CK(cudaEventCreateWithFlags(&s->nstage[2].ev, cudaEventDisableTiming));
         for (int i = 0; i < 2; i++) {
             CK(cudaStreamCreateWithFlags(&s->slot[i].st, cudaStreamNonBlocking));
-            CK(cudaMallocHost(&s->slot[i].h_totals, sizeof(PlanTotals)));
-            CK(cudaMallocHost(&s->slot[i].h_lookups, sizeof(unsigned long long)));
+            CK(s->slot[i].h_totals.ensure(sizeof(PlanTotals)));
+            CK(s->slot[i].h_lookups.ensure(sizeof(unsigned long long)));
             CK(cudaEventCreateWithFlags(&s->slot[i].ev_plan, cudaEventDisableTiming));
             CK(cudaEventCreateWithFlags(&s->nstage[i].ev, cudaEventDisableTiming));
         }
@@ -750,83 +729,74 @@ extern "C" void pa_destroy(pa_scorer* s) {
     cudaSetDevice(s->device);
     cudaDeviceSynchronize();
     s->pool.stop();
-    for (int i = 0; i < 3; i++) s->nstage[i].release();
-    for (int i = 0; i < 2; i++) s->slot[i].release();
-    s->d_T.release(); s->d_logd.release(); s->d_binom.release(); s->d_nl_sums.release(); s->d_nl_nvar.release();
-    s->d_perm_pool.release(); s->d_perm_off.release(); s->d_lut.release();
+    for (NarrowStage& ns : s->nstage) if (ns.ev) cudaEventDestroy(ns.ev);
+    for (Slot& sl : s->slot) {
+        if (sl.ev_plan) cudaEventDestroy(sl.ev_plan);
+        if (sl.st) cudaStreamDestroy(sl.st);
+    }
     for (cudaEvent_t e : s->ev_pool) cudaEventDestroy(e);
     if (!s->binner_only) g_live_scorers--;
-    delete s;
+    delete s;                                          // frees every buffer
 }
 
-// ---- staging helpers ----------------------------------------------------------------------------
-template <class T>
-static cudaError_t stage_in(DevBuf& buf, const T* src, bool on_dev, int64_t lo, int64_t n, cudaStream_t st,
-                            const T** view_abs, int64_t* h2d) {
-    // returns a pointer that can be indexed with ABSOLUTE indices lo..lo+n-1
-    if (src == nullptr) { *view_abs = nullptr; return cudaSuccess; }
-    if (on_dev) { *view_abs = src; return cudaSuccess; }
-    cudaError_t e = buf.ensure((size_t)std::max<int64_t>(n, 1) * sizeof(T));
-    if (e != cudaSuccess) return e;
-    if (n > 0) {
-        e = cudaMemcpyAsync(buf.p, src + lo, (size_t)n * sizeof(T), cudaMemcpyHostToDevice, st);
-        if (e != cudaSuccess) return e;
-        *h2d += n * (int64_t)sizeof(T);
+// ---- staging ------------------------------------------------------------------------------------
+// One array of a chunk on its way to or from the device.  The device view it produces is indexed like the caller's
+// array (absolute indices lo..lo+n-1); it is null when the caller passed no array.
+struct ChunkArray {
+    const void* arr = nullptr;       // the caller's array (host or device), or null
+    int64_t lo = 0, n = 0;           // the chunk's elements [lo, lo + n)
+    size_t elem = 0;                 // element size
+    DevBuf* buf = nullptr;           // the slot's staging buffer (per-array transfers)
+    void* view = nullptr;            // the T* (T: the element type) that receives the device view
+    size_t off = 0;                  // packed transfers: offset in the block
+    ChunkArray() = default;
+    template <class T> ChunkArray(T* arr, int64_t lo, int64_t n, DevBuf& buf, T*& view)
+        : arr(arr), lo(lo), n(n), elem(sizeof(T)), buf(&buf), view(&view) {}
+    size_t bytes() const { return (size_t)std::max<int64_t>(n, 0) * elem; }
+    void set_view(const unsigned char* base) const {        // base: where element `lo` is (null: no view)
+        const unsigned char* v = base ? base - lo * (int64_t)elem : nullptr;
+        memcpy(view, &v, sizeof(v));                        // (the view's pointer type is known to the caller only)
     }
-    *view_abs = buf.as<T>() - lo;
-    return cudaSuccess;
-}
+};
 
-template <class T>
-static cudaError_t stage_out(DevBuf& buf, T* dst, bool on_dev, int64_t lo, int64_t n, T** view_abs) {
-    if (dst == nullptr) { *view_abs = nullptr; return cudaSuccess; }
-    if (on_dev) { *view_abs = dst; return cudaSuccess; }
-    cudaError_t e = buf.ensure((size_t)std::max<int64_t>(n, 1) * sizeof(T));
+// Per-array transfers.  An array on the device is used in place; a host array gets the slot's buffer, and with `h2d`
+// given (inputs) its elements are copied there and counted.
+static cudaError_t stage(const ChunkArray& a, bool on_dev, cudaStream_t st, int64_t* h2d) {
+    if (!a.arr || on_dev) {
+        a.set_view(a.arr ? (const unsigned char*)a.arr + a.lo * (int64_t)a.elem : nullptr);
+        return cudaSuccess;
+    }
+    cudaError_t e = a.buf->ensure(std::max(a.bytes(), a.elem));
     if (e != cudaSuccess) return e;
-    *view_abs = buf.as<T>() - lo;
+    if (h2d && a.n > 0) {
+        e = cudaMemcpyAsync(a.buf->p, (const unsigned char*)a.arr + a.lo * (int64_t)a.elem, a.bytes(), cudaMemcpyHostToDevice, st);
+        if (e != cudaSuccess) return e;
+        *h2d += (int64_t)a.bytes();
+    }
+    a.set_view(a.buf->as<unsigned char>());
     return cudaSuccess;
 }
 
-template <class T>
-static cudaError_t copy_out(const DevBuf& buf, T* dst, bool on_dev, int64_t lo, int64_t n, cudaStream_t st, int64_t* d2h) {
-    if (dst == nullptr || on_dev || n <= 0) return cudaSuccess;
-    *d2h += n * (int64_t)sizeof(T);
-    return cudaMemcpyAsync(dst + lo, buf.p, (size_t)n * sizeof(T), cudaMemcpyDeviceToHost, st);
+static cudaError_t copy_back(const ChunkArray& a, bool on_dev, cudaStream_t st, int64_t* d2h) {
+    if (!a.arr || on_dev || a.n <= 0) return cudaSuccess;
+    *d2h += (int64_t)a.bytes();
+    return cudaMemcpyAsync((unsigned char*)a.arr + a.lo * (int64_t)a.elem, a.buf->p, a.bytes(), cudaMemcpyDeviceToHost, st);
 }
 
 #define PA_PACK_MAX (1 << 20)            // host batches up to this many input bytes travel as one packed block
 
-static cudaError_t ensure_pinned(unsigned char*& p, size_t& cap, size_t bytes) {
-    if (bytes <= cap) return cudaSuccess;
-    if (p) { cudaFreeHost(p); p = nullptr; cap = 0; }
-    const size_t want = bytes + bytes / 2 + 4096;
-    cudaError_t e = cudaMallocHost((void**)&p, want);
-    if (e == cudaSuccess) cap = want;
-    return e;
-}
-
-template <class T> static cudaError_t ensure_pinned_t(T*& p, size_t& cap, size_t count) {
-    unsigned char* q = (unsigned char*)p;
-    size_t bytes_cap = cap * sizeof(T);
-    cudaError_t e = ensure_pinned(q, bytes_cap, count * sizeof(T));
-    p = (T*)q; cap = bytes_cap / sizeof(T);
-    return e;
-}
-
-struct PackIn {                          // cursor over the packed input block (host image + device address)
-    unsigned char* h; unsigned char* d; size_t used;
-    template <class T> const T* add(const T* src, int64_t lo, int64_t n) {      // -> device view indexed with ABSOLUTE indices
-        if (!src) return nullptr;
-        const size_t off = (used + 15) & ~(size_t)15;
-        if (n > 0) memcpy(h + off, src + lo, (size_t)n * sizeof(T));
-        used = off + (size_t)std::max<int64_t>(n, 0) * sizeof(T);
-        return (const T*)(d + off) - lo;
+// Packed transfers of a small host batch: the arrays the caller passed are laid out in one block from byte `used` on,
+// each at a 16-byte aligned offset, with their device views in the block at `dev`.  Returns the block's size.
+static size_t pack_layout(ChunkArray* list, size_t count, size_t used, unsigned char* dev) {
+    for (size_t i = 0; i < count; i++) {
+        ChunkArray& a = list[i];
+        if (!a.arr) { a.set_view(nullptr); continue; }
+        a.off = (used + 15) & ~(size_t)15;
+        a.set_view(dev + a.off);
+        used = a.off + a.bytes();
     }
-};
-
-struct PackOut {                         // one packed result array: where it sits in the block, where it goes on the host
-    size_t off, bytes; void* dst;
-};
+    return used;
+}
 
 // (pa_host.cpp: vectorised with the host compiler's AVX2 when the CPU has it)
 void pa_narrow_spectra(const double* mz, const int64_t* spec_off, int64_t sa, int64_t sb, int64_t peak_base,
@@ -841,46 +811,32 @@ extern "C" int64_t pa_narrow_mz(const double* mz, const int64_t* spec_off, int64
     return n;
 }
 
-// ---- chunk boundaries of a device-resident batch --------------------------------------------------
-// Chunks a device-resident batch is cut into (the two streams alternate).  Measured on config 2 (1 M PSMs):
-// 1 chunk 91.5 M PSM/s, 2 chunks 94.1 M, 4 chunks 84.0 M, 8 chunks 70.2 M -- the persistent kernels of two
-// chunks cannot share an SM (registers / shared memory), so more chunks only add launches and tails.  One
-// chunk keeps the per-kernel event times free of overlap, which the roofline arithmetic relies on.
-#ifndef PA_DEV_CHUNKS
-#define PA_DEV_CHUNKS 1
-#endif
-#define PA_DEV_CHUNK_MIN 65536          // ... as long as each keeps at least this many PSMs
-#define PA_DEV_CHUNKS_MAX 16
+// ---- range ends of a device-resident batch --------------------------------------------------------
+// A device-resident batch is scored as one chunk.  Measured on config 2 (1 M PSMs): 1 chunk 91.5 M PSM/s, 2 chunks
+// 94.1 M, 4 chunks 84.0 M, 8 chunks 70.2 M -- the persistent kernels of two chunks cannot share an SM (registers /
+// shared memory), so more chunks only add launches and tails.  One chunk keeps the per-kernel event times free of
+// overlap, which the roofline arithmetic relies on.
 struct DevBounds {
-    int n;                              // boundaries 0..n (n = number of chunks)
-    int bad;                            // psm_spec decreasing or out of range somewhere
+    int bad;                            // see k_check_batch
     int max_peaks;                      // largest spectrum of the batch
-    int pad;
     int64_t n_aux;                      // fixed-mod entries of the range
-    int64_t p[PA_DEV_CHUNKS_MAX + 1];       // first PSM of chunk c (p[n] = n_psm)
-    int64_t s0[PA_DEV_CHUNKS_MAX + 1];      // first spectrum chunk c references
-    int64_t s1[PA_DEV_CHUNKS_MAX + 1];      // one past the last spectrum chunk c-1 references
-    int64_t peak0[PA_DEV_CHUNKS_MAX + 1], peak1[PA_DEV_CHUNKS_MAX + 1];     // spec_off at s0 / s1
-    int64_t pep[PA_DEV_CHUNKS_MAX + 1], mod[PA_DEV_CHUNKS_MAX + 1];         // pep_off / mod_off at p
+    int64_t s0, s1;                     // first spectrum the range references, one past the last
+    int64_t peak0, peak1;               // spec_off at s0 / s1
+    int64_t pep0, pep1, mod0, mod1;     // pep_off / mod_off at p_lo / p_hi
 };
 
+// Range ends of the non-empty PSM range [p_lo, p_hi): one thread, so that the host needs one copy, not one per value.
 __global__ void k_dev_bounds(const int64_t* spec_off, const int32_t* psm_spec, const int32_t* pep_off,
                              const int32_t* aux_off, const int64_t* mod_off, int64_t p_lo, int64_t p_hi, int64_t n_spec,
-                             int C, int64_t per, DevBounds* o) {
-    const int c = threadIdx.x;
-    if (c == 0) {
-        o->n = C;
-        o->n_aux = aux_off ? (int64_t)aux_off[p_hi] - (int64_t)aux_off[p_lo] : 0;
-    }
-    if (c > C) return;
-    const int64_t p = p_lo + (int64_t)c * per < p_hi ? p_lo + (int64_t)c * per : p_hi;
-    int64_t s0 = p < p_hi ? (int64_t)psm_spec[p] : (p_hi > p_lo ? (int64_t)psm_spec[p_hi - 1] + 1 : 0);
-    int64_t s1 = p > p_lo ? (int64_t)psm_spec[p - 1] + 1 : 0;
+                             DevBounds* o) {
+    int64_t s0 = psm_spec[p_lo], s1 = (int64_t)psm_spec[p_hi - 1] + 1;
     s0 = s0 < 0 ? 0 : (s0 > n_spec ? n_spec : s0);
     s1 = s1 < 0 ? 0 : (s1 > n_spec ? n_spec : s1);
-    o->p[c] = p; o->s0[c] = s0; o->s1[c] = s1;
-    o->peak0[c] = spec_off[s0]; o->peak1[c] = spec_off[s1];
-    o->pep[c] = pep_off[p]; o->mod[c] = mod_off[p];
+    o->n_aux = aux_off ? (int64_t)aux_off[p_hi] - (int64_t)aux_off[p_lo] : 0;
+    o->s0 = s0; o->s1 = s1;
+    o->peak0 = spec_off[s0]; o->peak1 = spec_off[s1];
+    o->pep0 = pep_off[p_lo]; o->pep1 = pep_off[p_hi];
+    o->mod0 = mod_off[p_lo]; o->mod1 = mod_off[p_hi];
 }
 
 // Consistency of a device-resident batch (the host path checks the same things per chunk): `bad` bit 0 =
@@ -912,13 +868,12 @@ struct ChunkState {              // what the back half of a chunk needs from the
     const int64_t* mod_off_abs = nullptr;
     cudaEvent_t e_bin0, e_bin1, e_plan1, e_cnt0, e_cnt1, e_sel1, e_asc1;
     uint64_t* o_sig; float* o_score; int64_t* o_niso; int32_t* o_nsites; float* o_asc; uint64_t* o_alt; int32_t* o_status;
+    ChunkArray res[7];               // the result arrays (views: the o_* above)
     bool single_chunk = false;       // the call has one chunk
-    bool packed = false;             // inputs / outputs travel as one block each (small host batch)
-    std::vector<PackOut> pack_out;
-    size_t pack_out_bytes = 0;
+    bool packed = false;             // inputs travel as one block (small host batch)
+    bool packed_res = false;         // ... and so do the results, in a block of this size:
+    size_t packed_res_bytes = 0;
 };
-
-struct ChunkEnds { int64_t peak_lo, peak_hi, pep_lo, pep_hi; };   // range ends of a device-resident chunk
 
 // Narrowing of the m/z of host chunk `r` into staging set `ns`: narrow_begin hands the per-spectrum work to the pool and
 // returns; narrow_end waits for it and lays out the exact copies.  The pipeline runs it one chunk ahead of the copies.
@@ -932,13 +887,13 @@ static int narrow_begin(pa_scorer* s, NarrowStage& ns, const pa_batch* in, const
     for (int64_t q = r.s0; q < r.s1; q++)
         if (in->spec_off[q + 1] < in->spec_off[q]) return PA_OK;
     CK(cudaEventSynchronize(ns.ev));                      // the chunk that used this set three chunks ago has left it
-    CK(ensure_pinned_t(ns.h_mz32, ns.h_mz32_cap, (size_t)ns.npk));
-    CK(ensure_pinned_t(ns.h_escoff, ns.h_escoff_cap, (size_t)ns.ns));
+    CK(ns.h_mz32.ensure((size_t)ns.npk * 4));
+    CK(ns.h_escoff.ensure((size_t)ns.ns * 4));
     ns.flags.resize((size_t)ns.ns);
     if (s->pool.th.empty()) s->pool.start(std::max(1, s->host_threads));
     const int tasks = (int)std::min<int64_t>(ns.ns, (int64_t)s->host_threads * 4);
     const double* mzh = in->mz; const int64_t* offh = in->spec_off;
-    float* o32 = ns.h_mz32; uint8_t* fl = ns.flags.data() - r.s0;
+    float* o32 = ns.h_mz32.as<float>(); uint8_t* fl = ns.flags.data() - r.s0;
     const float bsz = s->bin_size;
     const int64_t s0 = r.s0, nsp = ns.ns, peak_lo = ns.peak_lo, npk = ns.npk;
     s->pool.run_async(tasks, [=](int t) {
@@ -964,14 +919,15 @@ static int narrow_end(pa_scorer* s, NarrowStage& ns, const pa_batch* in) {
     for (int64_t q = 0; q < ns.ns; q++)
         if (ns.flags[q]) { ns.n_esc += in->spec_off[ns.s0 + q + 1] - in->spec_off[ns.s0 + q]; ns.n_flag++; }
     if (ns.n_esc * 4 > ns.npk) return PA_OK;              // m/z that sit on bin boundaries wholesale: nothing to gain
-    CK(ensure_pinned_t(ns.h_esc, ns.h_esc_cap, (size_t)std::max<int64_t>(ns.n_esc, 1)));
+    CK(ns.h_esc.ensure((size_t)std::max<int64_t>(ns.n_esc, 1) * 8));
+    int32_t* escoff = ns.h_escoff.as<int32_t>();
     int64_t eo = 0;
     for (int64_t q = 0; q < ns.ns; q++) {
-        ns.h_escoff[q] = -1;
+        escoff[q] = -1;
         if (!ns.flags[q]) continue;
         const int64_t o = in->spec_off[ns.s0 + q], P = in->spec_off[ns.s0 + q + 1] - o;
-        ns.h_escoff[q] = (int32_t)eo;
-        memcpy(ns.h_esc + eo, in->mz + o, (size_t)P * 8);
+        escoff[q] = (int32_t)eo;
+        memcpy(ns.h_esc.as<double>() + eo, in->mz + o, (size_t)P * 8);
         eo += P;
     }
     ns.ok = true;
@@ -979,14 +935,14 @@ static int narrow_end(pa_scorer* s, NarrowStage& ns, const pa_batch* in) {
 }
 
 static int chunk_front(pa_scorer* s, int si, const pa_batch* in, bool in_dev, const ChunkRange& r, int64_t mod_lo,
-                       int64_t mod_hi, int max_peaks, ChunkState& cs, const ChunkEnds* ends_dev, NarrowStage* nst = nullptr) {
+                       int64_t mod_hi, int max_peaks, ChunkState& cs, const DevBounds* ends_dev, NarrowStage* nst = nullptr) {
     Slot& sl = s->slot[si];
     cudaStream_t st = sl.st;
     const int64_t np = r.p1 - r.p0, ns = r.s1 - r.s0;
     int64_t peak_lo, peak_hi, pep_lo, pep_hi, aux_lo = 0, aux_hi = 0;
     if (in_dev) {
-        // offsets live on the device: pa_score_batch fetched the range ends of every chunk in one go
-        peak_lo = ends_dev->peak_lo; peak_hi = ends_dev->peak_hi; pep_lo = ends_dev->pep_lo; pep_hi = ends_dev->pep_hi;
+        // offsets live on the device: score_impl fetched the range ends in one go
+        peak_lo = ends_dev->peak0; peak_hi = ends_dev->peak1; pep_lo = ends_dev->pep0; pep_hi = ends_dev->pep1;
     } else {
         peak_lo = in->spec_off[r.s0]; peak_hi = in->spec_off[r.s1];
         pep_lo = in->pep_off[r.p0]; pep_hi = in->pep_off[r.p1];
@@ -996,46 +952,39 @@ static int chunk_front(pa_scorer* s, int si, const pa_batch* in, bool in_dev, co
     cs.r = r; cs.mod_lo = mod_lo; cs.mod_hi = mod_hi;
     int64_t* h2d = &s->ctr.bytes_h2d;
     PaBatchDev& b = cs.b;
-    const double *v_mz, *v_int = nullptr;
+    const double *v_mz = nullptr, *v_int = nullptr;
     const float* v_int32 = nullptr;
-    const int64_t n_aux = aux_hi - aux_lo;
-    const size_t pack_bytes = (size_t)(ns + 1) * 8 + (size_t)npk * (in->inten32 ? 12 : 16) + (size_t)np * 12 + (size_t)(np + 1) * 16 +
-                              (size_t)(pep_hi - pep_lo) + (size_t)n_aux * 8 + 16 * 16;
+    ChunkArray ins[] = {
+        {in->spec_off, r.s0, ns + 1, sl.spec_off, b.spec_off},
+        {in->mz, peak_lo, npk, sl.mz, v_mz},
+        in->inten32 ? ChunkArray(in->inten32, peak_lo, npk, sl.inten32, v_int32) : ChunkArray(in->inten, peak_lo, npk, sl.inten, v_int),
+        {in->psm_spec, r.p0, np, sl.psm_spec, b.psm_spec},
+        {in->pep_off, r.p0, np + 1, sl.pep_off, b.pep_off},
+        {in->pep, pep_lo, pep_hi - pep_lo, sl.pep, b.pep},
+        {in->n_mod, r.p0, np, sl.n_mod, b.n_mod},
+        {in->max_charge, r.p0, np, sl.max_charge, b.max_charge},
+        {in->aux_off, r.p0, np + 1, sl.aux_off, b.aux_off},
+        {in->aux_off ? in->aux_pos : nullptr, aux_lo, aux_hi - aux_lo, sl.aux_pos, b.aux_pos},
+        {in->aux_off ? in->aux_mass : nullptr, aux_lo, aux_hi - aux_lo, sl.aux_mass, b.aux_mass},
+        {in->mod_off, r.p0, np + 1, sl.mod_off, cs.mod_off_abs},
+    };
+    const ChunkArray& mz_in = ins[1];
+    // packed block bound: every array at full size, the absent ones too, and 16 bytes of alignment for each
+    size_t pack_bytes = 16 * 16;
+    for (const ChunkArray& a : ins) pack_bytes += (size_t)a.n * a.elem;
     bool narrowed = false;
     cs.packed = !in_dev && cs.single_chunk && pack_bytes <= PA_PACK_MAX && s->narrow_mode != 1 && !(nst != nullptr && nst->busy);
     if (cs.packed) {
-        CK(ensure_pinned(sl.h_pack, sl.h_pack_cap, pack_bytes));
+        CK(sl.h_pack.ensure(pack_bytes));
         CK(sl.d_pack.ensure(pack_bytes));
-        PackIn pk{sl.h_pack, sl.d_pack.as<unsigned char>(), 0};
-        b.spec_off = pk.add(in->spec_off, r.s0, ns + 1);
-        v_mz = pk.add(in->mz, peak_lo, npk);
-        if (in->inten32) v_int32 = pk.add(in->inten32, peak_lo, npk); else v_int = pk.add(in->inten, peak_lo, npk);
-        b.psm_spec = pk.add(in->psm_spec, r.p0, np);
-        b.pep_off = pk.add(in->pep_off, r.p0, np + 1);
-        b.pep = pk.add(in->pep, pep_lo, pep_hi - pep_lo);
-        b.n_mod = pk.add(in->n_mod, r.p0, np);
-        b.max_charge = pk.add(in->max_charge, r.p0, np);
-        b.aux_off = pk.add(in->aux_off, r.p0, np + 1);
-        b.aux_pos = in->aux_off ? pk.add(in->aux_pos, aux_lo, n_aux) : nullptr;
-        b.aux_mass = in->aux_off ? pk.add(in->aux_mass, aux_lo, n_aux) : nullptr;
-        cs.mod_off_abs = pk.add(in->mod_off, r.p0, np + 1);
-        CK(cudaMemcpyAsync(sl.d_pack.p, sl.h_pack, pk.used, cudaMemcpyHostToDevice, st));
-        *h2d += (int64_t)pk.used;
+        const size_t used = pack_layout(ins, sizeof(ins) / sizeof(ins[0]), 0, sl.d_pack.as<unsigned char>());
+        for (const ChunkArray& a : ins)
+            if (a.arr && a.n > 0) memcpy(sl.h_pack.as<unsigned char>() + a.off, (const unsigned char*)a.arr + a.lo * (int64_t)a.elem, a.bytes());
+        CK(cudaMemcpyAsync(sl.d_pack.p, sl.h_pack.p, used, cudaMemcpyHostToDevice, st));
+        *h2d += (int64_t)used;
     } else {
-    CK(stage_in(sl.spec_off, in->spec_off, in_dev, r.s0, ns + 1, st, &b.spec_off, h2d));
-    if (in->inten32) CK(stage_in(sl.inten32, in->inten32, in_dev, peak_lo, npk, st, &v_int32, h2d));
-    else CK(stage_in(sl.inten, in->inten, in_dev, peak_lo, npk, st, &v_int, h2d));
-    CK(stage_in(sl.psm_spec, in->psm_spec, in_dev, r.p0, np, st, &b.psm_spec, h2d));
-    CK(stage_in(sl.pep_off, in->pep_off, in_dev, r.p0, np + 1, st, &b.pep_off, h2d));
-    CK(stage_in(sl.pep, in->pep, in_dev, pep_lo, pep_hi - pep_lo, st, &b.pep, h2d));
-    CK(stage_in(sl.n_mod, in->n_mod, in_dev, r.p0, np, st, &b.n_mod, h2d));
-    CK(stage_in(sl.max_charge, in->max_charge, in_dev, r.p0, np, st, &b.max_charge, h2d));
-    CK(stage_in(sl.aux_off, in->aux_off, in_dev, r.p0, np + 1, st, &b.aux_off, h2d));
-    if (in->aux_off) {
-        CK(stage_in(sl.aux_pos, in->aux_pos, in_dev, aux_lo, aux_hi - aux_lo, st, &b.aux_pos, h2d));
-        CK(stage_in(sl.aux_mass, in->aux_mass, in_dev, aux_lo, aux_hi - aux_lo, st, &b.aux_mass, h2d));
-    } else { b.aux_pos = nullptr; b.aux_mass = nullptr; }
-    CK(stage_in(sl.mod_off, in->mod_off, in_dev, r.p0, np + 1, st, &cs.mod_off_abs, h2d));
+    for (const ChunkArray& a : ins)
+        if (&a != &mz_in) CK(stage(a, in_dev, st, h2d));
     // host batches: the m/z array goes over the link as float32 wherever the host proved that nothing the kernels
     // derive from it changes (narrow_begin / narrow_end); spectra that failed the proof come with an exact copy.  It goes
     // last: the chunk's other arrays are on the wire while the pool finishes the chunk's narrowing.
@@ -1044,16 +993,15 @@ static int chunk_front(pa_scorer* s, int si, const pa_batch* in, bool in_dev, co
         CK(sl.mz32.ensure((size_t)std::max<int64_t>(npk, 1) * 4));
         CK(sl.escoff.ensure((size_t)ns * 4));
         CK(sl.esc.ensure((size_t)std::max<int64_t>(nst->n_esc, 1) * 8));
-        CK(cudaMemcpyAsync(sl.mz32.p, nst->h_mz32, (size_t)npk * 4, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(sl.escoff.p, nst->h_escoff, (size_t)ns * 4, cudaMemcpyHostToDevice, st));
-        if (nst->n_esc > 0) CK(cudaMemcpyAsync(sl.esc.p, nst->h_esc, (size_t)nst->n_esc * 8, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(sl.mz32.p, nst->h_mz32.p, (size_t)npk * 4, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(sl.escoff.p, nst->h_escoff.p, (size_t)ns * 4, cudaMemcpyHostToDevice, st));
+        if (nst->n_esc > 0) CK(cudaMemcpyAsync(sl.esc.p, nst->h_esc.p, (size_t)nst->n_esc * 8, cudaMemcpyHostToDevice, st));
         CK(cudaEventRecord(nst->ev, st));
         *h2d += npk * 4 + ns * 4 + nst->n_esc * 8;
         s->ctr.n_spec_exact += nst->n_flag;
         narrowed = true;
-        v_mz = nullptr;
     }
-    if (!narrowed) CK(stage_in(sl.mz, in->mz, in_dev, peak_lo, npk, st, &v_mz, h2d));
+    if (!narrowed) CK(stage(mz_in, in_dev, st, h2d));
     }
     // PSM-indexed views become chunk-relative
     b.psm_spec += r.p0; b.pep_off += r.p0; b.n_mod += r.p0; b.max_charge += r.p0;
@@ -1145,7 +1093,7 @@ static int chunk_front(pa_scorer* s, int si, const pa_batch* in, bool in_dev, co
     s->ctr.kernel_launches += 2;
     CK(cudaMemcpyAsync(&dt->total_iso, sl.iso_off.as<int64_t>() + np, sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
     CK(cudaMemcpyAsync(&dt->total_units, sl.unit_off.as<int32_t>() + np, sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
-    CK(cudaMemcpyAsync(sl.h_totals, dt, sizeof(PlanTotals), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(sl.h_totals.p, dt, sizeof(PlanTotals), cudaMemcpyDeviceToHost, st));
     CK(cudaEventRecord(cs.e_plan1, st));
     CK(cudaEventRecord(sl.ev_plan, st));
     return PA_OK;
@@ -1157,7 +1105,7 @@ static int chunk_back(pa_scorer* s, int si, const pa_results* out, bool out_dev,
     const ChunkRange& r = cs.r;
     const int64_t np = r.p1 - r.p0;
     CK(cudaEventSynchronize(sl.ev_plan));
-    PlanTotals T = *sl.h_totals;
+    PlanTotals T = *sl.h_totals.as<PlanTotals>();
     const int64_t total_iso = T.total_iso;
     const int n_units = T.total_units;
     // tables that depend on what the chunk contains
@@ -1222,40 +1170,23 @@ static int chunk_back(pa_scorer* s, int si, const pa_results* out, bool out_dev,
     CK(cudaEventRecord(cs.e_cnt1, st));
     // outputs
     const int64_t nm = cs.mod_hi - cs.mod_lo;
-    const bool pack_results = cs.packed && !out_dev && (size_t)np * 32 + (size_t)nm * 12 + 8 * 16 <= PA_PACK_MAX;
-    if (pack_results) {
-        size_t used = 0;
-        auto slot_of = [&](void* dst, int64_t lo, int64_t n, size_t elem) -> unsigned char* {      // view with absolute indices
-            if (!dst) return nullptr;
-            const size_t off = (used + 15) & ~(size_t)15;
-            used = off + (size_t)std::max<int64_t>(n, 0) * elem;
-            cs.pack_out.push_back({off, (size_t)std::max<int64_t>(n, 0) * elem, (unsigned char*)dst + (size_t)lo * elem});
-            return (unsigned char*)nullptr + off - (size_t)lo * elem;      // offset relative to the block, rebased below
-        };
-        const size_t bound = (size_t)np * 32 + (size_t)nm * 12 + 8 * 16;
-        CK(sl.d_opack.ensure(bound));
-        CK(ensure_pinned(sl.h_opack, sl.h_opack_cap, bound));
-        unsigned char* base = sl.d_opack.as<unsigned char>();
-        auto rebase = [&](unsigned char* rel) { return rel == nullptr ? nullptr : base + (size_t)(rel - (unsigned char*)nullptr); };
-        // (a NULL result pointer means "skip": slot_of returns nullptr and so does rebase -- but an offset of 0 must
-        // not be mistaken for it, so the block starts with 16 bytes of padding)
-        used = 16;
-        cs.o_sig = (uint64_t*)rebase(slot_of(out->best_sig, r.p0, np, 8));
-        cs.o_score = (float*)rebase(slot_of(out->best_score, r.p0, np, 4));
-        cs.o_niso = (int64_t*)rebase(slot_of(out->n_iso, r.p0, np, 8));
-        cs.o_nsites = (int32_t*)rebase(slot_of(out->n_sites, r.p0, np, 4));
-        cs.o_asc = (float*)rebase(slot_of(out->ascores, cs.mod_lo, nm, 4));
-        cs.o_alt = (uint64_t*)rebase(slot_of(out->alt_sites, cs.mod_lo, nm, 8));
-        cs.o_status = (int32_t*)rebase(slot_of(out->psm_status, r.p0, np, 4));
-        cs.pack_out_bytes = used;
+    ChunkArray* res = cs.res;
+    res[0] = {out->best_sig, r.p0, np, sl.o_sig, cs.o_sig};
+    res[1] = {out->best_score, r.p0, np, sl.o_score, cs.o_score};
+    res[2] = {out->n_iso, r.p0, np, sl.o_niso, cs.o_niso};
+    res[3] = {out->n_sites, r.p0, np, sl.o_nsites, cs.o_nsites};
+    res[4] = {out->ascores, cs.mod_lo, nm, sl.o_asc, cs.o_asc};
+    res[5] = {out->alt_sites, cs.mod_lo, nm, sl.o_alt, cs.o_alt};
+    res[6] = {out->psm_status, r.p0, np, sl.o_status, cs.o_status};
+    const size_t res_bound = (size_t)np * 32 + (size_t)nm * 12 + 8 * 16;
+    cs.packed_res = cs.packed && !out_dev && res_bound <= PA_PACK_MAX;
+    if (cs.packed_res) {
+        CK(sl.d_opack.ensure(res_bound));
+        CK(sl.h_opack.ensure(res_bound));
+        // (the results start at byte 16 of the block: the read-back that bytes_d2h reports keeps its size)
+        cs.packed_res_bytes = pack_layout(res, 7, 16, sl.d_opack.as<unsigned char>());
     } else {
-    CK(stage_out(sl.o_sig, out->best_sig, out_dev, r.p0, np, &cs.o_sig));
-    CK(stage_out(sl.o_score, out->best_score, out_dev, r.p0, np, &cs.o_score));
-    CK(stage_out(sl.o_niso, out->n_iso, out_dev, r.p0, np, &cs.o_niso));
-    CK(stage_out(sl.o_nsites, out->n_sites, out_dev, r.p0, np, &cs.o_nsites));
-    CK(stage_out(sl.o_asc, out->ascores, out_dev, cs.mod_lo, cs.mod_hi - cs.mod_lo, &cs.o_asc));
-    CK(stage_out(sl.o_alt, out->alt_sites, out_dev, cs.mod_lo, cs.mod_hi - cs.mod_lo, &cs.o_alt));
-    CK(stage_out(sl.o_status, out->psm_status, out_dev, r.p0, np, &cs.o_status));
+        for (int i = 0; i < 7; i++) CK(stage(res[i], out_dev, st, nullptr));
     }
     CK(sl.best_idx.ensure((size_t)std::max<int64_t>(np, 1) * 4));
     CK(sl.mod_psm.ensure((size_t)std::max<int64_t>(nm, 1) * 4));
@@ -1357,17 +1288,11 @@ static int chunk_back(pa_scorer* s, int si, const pa_results* out, bool out_dev,
     }
     CK(cudaEventRecord(cs.e_asc1, st));
     int64_t* d2h = &s->ctr.bytes_d2h;
-    if (pack_results) {
-        CK(cudaMemcpyAsync(sl.h_opack, sl.d_opack.p, cs.pack_out_bytes, cudaMemcpyDeviceToHost, st));
-        *d2h += (int64_t)cs.pack_out_bytes;
+    if (cs.packed_res) {         // (score_impl copies the block into the caller's arrays once the stream is done)
+        CK(cudaMemcpyAsync(sl.h_opack.p, sl.d_opack.p, cs.packed_res_bytes, cudaMemcpyDeviceToHost, st));
+        *d2h += (int64_t)cs.packed_res_bytes;
     } else {
-    CK(copy_out(sl.o_sig, out->best_sig, out_dev, r.p0, np, st, d2h));
-    CK(copy_out(sl.o_score, out->best_score, out_dev, r.p0, np, st, d2h));
-    CK(copy_out(sl.o_niso, out->n_iso, out_dev, r.p0, np, st, d2h));
-    CK(copy_out(sl.o_nsites, out->n_sites, out_dev, r.p0, np, st, d2h));
-    CK(copy_out(sl.o_asc, out->ascores, out_dev, cs.mod_lo, cs.mod_hi - cs.mod_lo, st, d2h));
-    CK(copy_out(sl.o_alt, out->alt_sites, out_dev, cs.mod_lo, cs.mod_hi - cs.mod_lo, st, d2h));
-    CK(copy_out(sl.o_status, out->psm_status, out_dev, r.p0, np, st, d2h));
+        for (int i = 0; i < 7; i++) CK(copy_back(res[i], out_dev, st, d2h));
     }
     s->ctr.n_isoforms += total_iso;
     if (keep) {
@@ -1430,49 +1355,33 @@ static int score_impl(pa_scorer* s, const pa_batch* in, const pa_results* out, i
     std::vector<ChunkRange> chunks;
     std::vector<int> chunk_maxp;
     std::vector<int64_t> mod_lo, mod_hi;
-    std::vector<ChunkEnds> ends_dev;
-    int dev_max_peaks = 512;
+    DevBounds hb;
     if (in_dev) {
-        // Device-resident batch: PA_DEV_CHUNKS chunks that alternate between the two streams (see the note at
-        // PA_DEV_CHUNKS: one by default).  One small kernel gathers every range end the host needs, a second
-        // checks the CSR arrays (and that psm_spec is non-decreasing: cutting on PSM indices relies on it), a
+        // Device-resident batch: one chunk (see DevBounds).  One small kernel gathers the range ends the host needs,
+        // a second checks the CSR arrays (and that psm_spec is non-decreasing: the spectrum range relies on it), a
         // third finds the largest spectrum: one device -> host copy instead of one per value.
-        int C = keep ? 1 : (int)std::max<int64_t>(1, std::min<int64_t>(PA_DEV_CHUNKS, n_range / PA_DEV_CHUNK_MIN));
-        const int64_t per = (n_range + C - 1) / C;
         DevBuf& tb = s->slot[0].totals;
         CK(tb.ensure(sizeof(PlanTotals) + sizeof(DevBounds)));
         DevBounds* d_b = (DevBounds*)tb.p;
         CK(cudaMemset(d_b, 0, sizeof(DevBounds)));
-        k_dev_bounds<<<1, 32>>>(in->spec_off, in->psm_spec, in->pep_off, in->aux_off, in->mod_off, p_lo, p_hi, in->n_spec, C, per, d_b);
+        k_dev_bounds<<<1, 1>>>(in->spec_off, in->psm_spec, in->pep_off, in->aux_off, in->mod_off, p_lo, p_hi, in->n_spec, d_b);
         k_check_batch<<<(unsigned)std::min<int64_t>((std::max(n_range, in->n_spec) + 255) / 256, 1184), 256>>>(
             in->psm_spec, in->pep_off, in->aux_off, in->n_mod, in->mod_off, in->spec_off, p_lo, p_hi, in->n_spec, &d_b->bad);
         k_max_peaks<<<(unsigned)((in->n_spec + 255) / 256), 256>>>(in->spec_off, in->n_spec, &d_b->max_peaks);
         CK(cudaGetLastError());
         s->ctr.kernel_launches += 3;
-        DevBounds hb;
         CK(cudaMemcpy(&hb, d_b, sizeof(DevBounds), cudaMemcpyDeviceToHost));
         if (hb.bad & 2) return fail(s, PA_ERR_ARG, "inconsistent batch: an offset array is not a non-decreasing CSR index or mod_off does not follow n_mod");
         if (hb.n_aux > 0 && (!in->aux_pos || !in->aux_mass)) return fail(s, PA_ERR_ARG, "aux_off is not empty but aux_pos / aux_mass is NULL");
-        dev_max_peaks = hb.max_peaks;
-        const bool unordered = (hb.bad & 1) != 0;
-        if (unordered) C = 1;                    // unordered PSM -> spectrum map: one chunk over everything
-        for (int c = 0; c < C; c++) {
-            const int a = (C == 1) ? 0 : c, z = (C == 1) ? hb.n : c + 1;       // boundary indices
-            ChunkRange r = {hb.p[a], hb.p[z], unordered ? 0 : hb.s0[a], unordered ? in->n_spec : hb.s1[z]};
-            if (r.p1 <= r.p0) continue;
-            chunks.push_back(r);
-            ChunkEnds e;
-            if (unordered) {
-                int64_t pk[2];
-                CK(cudaMemcpy(&pk[0], in->spec_off, 8, cudaMemcpyDeviceToHost));
-                CK(cudaMemcpy(&pk[1], in->spec_off + in->n_spec, 8, cudaMemcpyDeviceToHost));
-                e = {pk[0], pk[1], hb.pep[a], hb.pep[z]};
-            } else e = {hb.peak0[a], hb.peak1[z], hb.pep[a], hb.pep[z]};
-            ends_dev.push_back(e);
-            mod_lo.push_back(hb.mod[a]); mod_hi.push_back(hb.mod[z]);
-            chunk_maxp.push_back(dev_max_peaks);
-            s->ctr.n_peaks += e.peak_hi - e.peak_lo;
+        if (hb.bad & 1) {                        // unordered PSM -> spectrum map: the chunk takes every spectrum
+            hb.s0 = 0; hb.s1 = in->n_spec;
+            CK(cudaMemcpy(&hb.peak0, in->spec_off, 8, cudaMemcpyDeviceToHost));
+            CK(cudaMemcpy(&hb.peak1, in->spec_off + in->n_spec, 8, cudaMemcpyDeviceToHost));
         }
+        chunks.push_back({p_lo, p_hi, hb.s0, hb.s1});
+        mod_lo.push_back(hb.mod0); mod_hi.push_back(hb.mod1);
+        chunk_maxp.push_back(hb.max_peaks);
+        s->ctr.n_peaks += hb.peak1 - hb.peak0;
     } else {
         // one branch-free pass (the compiler vectorises it): PSMs in spectrum order, indices in range
         int bad = 0;
@@ -1543,7 +1452,7 @@ static int score_impl(pa_scorer* s, const pa_batch* in, const pa_results* out, i
         rc = narrow_begin(s, nstage(0), in, chunks[0]);           // (chunk_front waits for it, after the chunk's other copies)
         if (rc != PA_OK) return bail(rc);
     }
-    rc = chunk_front(s, 0, in, in_dev, chunks[0], mod_lo[0], mod_hi[0], chunk_maxp[0], cs[0], in_dev ? &ends_dev[0] : nullptr,
+    rc = chunk_front(s, 0, in, in_dev, chunks[0], mod_lo[0], mod_hi[0], chunk_maxp[0], cs[0], in_dev ? &hb : nullptr,
                      may_narrow ? &nstage(0) : nullptr);
     if (rc != PA_OK) return bail(rc);
     if (may_narrow && chunks.size() > 1) { rc = narrow_begin(s, nstage(1), in, chunks[1]); if (rc != PA_OK) return bail(rc); }
@@ -1555,7 +1464,7 @@ static int score_impl(pa_scorer* s, const pa_batch* in, const pa_results* out, i
             }
             // slot (c+1)&1 was last used by chunk c-1: its stream order keeps buffers safe
             rc = chunk_front(s, (int)((c + 1) & 1), in, in_dev, chunks[c + 1], mod_lo[c + 1], mod_hi[c + 1],
-                             chunk_maxp[c + 1], cs[c + 1], in_dev ? &ends_dev[c + 1] : nullptr, may_narrow ? &nstage(c + 1) : nullptr);
+                             chunk_maxp[c + 1], cs[c + 1], in_dev ? &hb : nullptr, may_narrow ? &nstage(c + 1) : nullptr);
             if (rc != PA_OK) return bail(rc);
             if (may_narrow && c + 2 < chunks.size()) { rc = narrow_begin(s, nstage(c + 2), in, chunks[c + 2]); if (rc != PA_OK) return bail(rc); }
         }
@@ -1563,14 +1472,16 @@ static int score_impl(pa_scorer* s, const pa_batch* in, const pa_results* out, i
         if (rc != PA_OK) return bail(rc);
     }
     for (int i = 0; i < 2; i++)
-        CK(cudaMemcpyAsync(s->slot[i].h_lookups, s->slot[i].lookups.p, 8, cudaMemcpyDeviceToHost, s->slot[i].st));
+        CK(cudaMemcpyAsync(s->slot[i].h_lookups.p, s->slot[i].lookups.p, 8, cudaMemcpyDeviceToHost, s->slot[i].st));
     CK(cudaStreamSynchronize(s->slot[0].st));
     CK(cudaStreamSynchronize(s->slot[1].st));
     CK(cudaEventRecord(e_all1, s->slot[0].st));
     CK(cudaEventSynchronize(e_all1));
     for (size_t c = 0; c < chunks.size(); c++)       // packed results: from the pinned block into the caller's arrays
-        for (const PackOut& po : cs[c].pack_out)
-            if (po.bytes) memcpy(po.dst, s->slot[c & 1].h_opack + po.off, po.bytes);
+        if (cs[c].packed_res)
+            for (const ChunkArray& a : cs[c].res)
+                if (a.arr && a.n > 0)
+                    memcpy((unsigned char*)a.arr + a.lo * (int64_t)a.elem, s->slot[c & 1].h_opack.as<unsigned char>() + a.off, a.bytes());
     // counters
     for (size_t c = 0; c < chunks.size(); c++) {
         float ms = 0.f;
@@ -1581,7 +1492,7 @@ static int score_impl(pa_scorer* s, const pa_batch* in, const pa_results* out, i
         cudaEventElapsedTime(&ms, cs[c].e_sel1, cs[c].e_asc1); s->ctr.ms_ascore += ms;
     }
     cudaEventElapsedTime(&s->ctr.ms_total, e_all0, e_all1);
-    s->ctr.n_fragment_lookups = (int64_t)(*s->slot[0].h_lookups) + (int64_t)(*s->slot[1].h_lookups);
+    s->ctr.n_fragment_lookups = (int64_t)*s->slot[0].h_lookups.as<unsigned long long>() + (int64_t)*s->slot[1].h_lookups.as<unsigned long long>();
     if (narrow_trial && s->narrow_state < 3) {
         const double rate = (double)call_peaks / std::chrono::duration<double>(std::chrono::steady_clock::now() - t_call).count();
         if (s->narrow_state == 1) s->narrow_rate_on = rate;
@@ -1679,7 +1590,7 @@ extern "C" int64_t pa_fetch_pep_scores(pa_scorer* s, int64_t psm, int64_t cap, u
     CK(cudaMemcpy(&k, s->kept.b.n_mod + q, 4, cudaMemcpyDeviceToHost));
     const int64_t I = off[1] - off[0];
     if (I <= 0 || status != PA_PSM_OK) return 0;
-    TmpBuf d_sig, d_cnt, d_sc, d_w, d_tot;
+    DevBuf d_sig, d_cnt, d_sc, d_w, d_tot;
     CK(d_sig.ensure(I * 8)); CK(d_cnt.ensure(I * PA_N_TOP * 4)); CK(d_sc.ensure(I * PA_N_TOP * 4));
     CK(d_w.ensure(I * 4)); CK(d_tot.ensure(I * 4));
     k_export_psm<<<(unsigned)((I + 127) / 128), 128>>>(s->cfg, off[0], I, S, k, s->kept.iso, d_sig.as<uint64_t>(),
@@ -1692,7 +1603,6 @@ extern "C" int64_t pa_fetch_pep_scores(pa_scorer* s, int64_t psm, int64_t cap, u
     CK(cudaMemcpy(h_sc.data(), d_sc.p, I * PA_N_TOP * 4, cudaMemcpyDeviceToHost));
     CK(cudaMemcpy(h_w.data(), d_w.p, I * 4, cudaMemcpyDeviceToHost));
     CK(cudaMemcpy(h_tot.data(), d_tot.p, I * 4, cudaMemcpyDeviceToHost));
-    d_sig.release(); d_cnt.release(); d_sc.release(); d_w.release(); d_tot.release();
     // listing order: hash-iteration order, then std::sort by descending weighted score unless
     // the PSM is unambiguous (cpp/Ascore.cpp:263-269)
     std::vector<uint32_t> order(I);
@@ -1726,7 +1636,7 @@ extern "C" int pa_calculate_ambiguity(pa_scorer* s, int64_t psm, uint64_t sig_a,
     PaAmbArgs a;
     a.psm = psm - s->kept.psm_lo; a.sigA = sig_a; a.sigB = sig_b; a.wA = weighted_a; a.wB = weighted_b;
     memcpy(a.scA, scores_a, sizeof(a.scA)); memcpy(a.scB, scores_b, sizeof(a.scB));
-    TmpBuf d_out, d_lists;
+    DevBuf d_out, d_lists;
     CK(d_out.ensure(4));
     a.list_stride = 32;
     while (a.list_stride < s->kept.max_list) a.list_stride <<= 1;
@@ -1735,7 +1645,6 @@ extern "C" int pa_calculate_ambiguity(pa_scorer* s, int64_t psm, uint64_t sig_a,
     k_ambiguity<<<1, 32, sizeof(SelSmem)>>>(s->cfg, s->kept.b, a);
     CK(cudaGetLastError());
     CK(cudaMemcpy(out, d_out.p, 4, cudaMemcpyDeviceToHost));
-    d_out.release(); d_lists.release();
     return PA_OK;
 }
 
@@ -1856,24 +1765,24 @@ extern "C" int pa_bin_spectra_ex(pa_scorer* s, int64_t n_spec, const int64_t* sp
     cudaStream_t st = sl.st;
     const int64_t lo = spec_off[0], npk = spec_off[n_spec] - lo;
     const size_t npk1 = (size_t)std::max<int64_t>(npk, 1);
-    int64_t dummy = 0;
-    const int64_t* v_off; const double *v_mz, *v_int;
-    CK(stage_in(sl.spec_off, spec_off, false, 0, n_spec + 1, st, &v_off, &dummy));
-    CK(stage_in(sl.mz, mz, false, lo, npk, st, &v_mz, &dummy));
-    CK(stage_in(sl.inten, inten, false, lo, npk, st, &v_int, &dummy));
-    CK(sl.rpk.ensure(npk1 * sizeof(float2))); CK(sl.rmz.ensure(npk1 * 4)); CK(sl.rrank.ensure(npk1));
+    PaBinArgs ba;
+    int64_t h2d = 0;
+    for (const ChunkArray& a : {ChunkArray(spec_off, 0, n_spec + 1, sl.spec_off, ba.spec_off), ChunkArray(mz, lo, npk, sl.mz, ba.mz),
+                                ChunkArray(inten, lo, npk, sl.inten, ba.inten)})
+        CK(stage(a, false, st, &h2d));
+    DevBuf rmz, rrank;
+    CK(sl.rpk.ensure(npk1 * sizeof(float2))); CK(rmz.ensure(npk1 * 4)); CK(rrank.ensure(npk1));
     CK(sl.g_bin.ensure(npk1 * 4)); CK(sl.g_tmp.ensure(npk1));
     CK(sl.rcount.ensure((size_t)n_spec * 4));
     CK(sl.ctab.ensure((size_t)n_spec * PA_NCELL)); CK(sl.chead.ensure((size_t)n_spec * sizeof(float2)));
     const bool extra = out_index || out_bin || out_bounds;
-    TmpBuf d_index, d_bin, d_bounds;
+    DevBuf d_index, d_bin, d_bounds;
     if (extra) { CK(d_index.ensure(npk1 * 4)); CK(d_bin.ensure(npk1 * 4)); CK(d_bounds.ensure((size_t)n_spec * 12)); }
     int64_t m = 0;
     for (int64_t q = 0; q < n_spec; q++) m = std::max<int64_t>(m, spec_off[q + 1] - spec_off[q]);
-    PaBinArgs ba;
-    ba.spec_off = v_off; ba.mz = v_mz; ba.inten = v_int; ba.inten32 = nullptr; ba.peak_base = 0; ba.n_spec = n_spec;
+    ba.inten32 = nullptr; ba.peak_base = 0; ba.n_spec = n_spec;
     ba.mz32 = nullptr; ba.esc_off = nullptr; ba.mz_esc = nullptr;
-    ba.rpk = sl.rpk.as<float2>() - lo; ba.rmz = sl.rmz.as<float>() - lo; ba.rrank = sl.rrank.as<uint8_t>() - lo;
+    ba.rpk = sl.rpk.as<float2>() - lo; ba.rmz = rmz.as<float>() - lo; ba.rrank = rrank.as<uint8_t>() - lo;
     ba.g_bin = sl.g_bin.as<int32_t>() - lo; ba.g_tmp = sl.g_tmp.as<uint8_t>() - lo;
     ba.rcount = sl.rcount.as<int32_t>(); ba.bin_size = s->bin_size; ba.n_top = s->n_top;
     ba.ctab = sl.ctab.as<uint8_t>(); ba.chead = sl.chead.as<float2>();
@@ -1887,14 +1796,13 @@ extern "C" int pa_bin_spectra_ex(pa_scorer* s, int64_t n_spec, const int64_t* sp
     ba.cap = cap;
     k_bin_topn<false><<<blocks, wpb * 32, smem, st>>>(ba);
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(out_mz + lo, sl.rmz.p, (size_t)npk * 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaMemcpyAsync(out_rank + lo, sl.rrank.p, (size_t)npk, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(out_mz + lo, rmz.p, (size_t)npk * 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(out_rank + lo, rrank.p, (size_t)npk, cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(out_count, sl.rcount.p, (size_t)n_spec * 4, cudaMemcpyDeviceToHost, st));
     if (out_index) CK(cudaMemcpyAsync(out_index + lo, d_index.p, (size_t)npk * 4, cudaMemcpyDeviceToHost, st));
     if (out_bin) CK(cudaMemcpyAsync(out_bin + lo, d_bin.p, (size_t)npk * 4, cudaMemcpyDeviceToHost, st));
     if (out_bounds) CK(cudaMemcpyAsync(out_bounds, d_bounds.p, (size_t)n_spec * 12, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
-    d_index.release(); d_bin.release(); d_bounds.release();
     return PA_OK;
 }
 
@@ -1906,7 +1814,7 @@ extern "C" int pa_bin_spectra(pa_scorer* s, int64_t n_spec, const int64_t* spec_
 // ---- single-peptide probes ------------------------------------------------------------------------
 // One peptide (+ fixed mods) staged as a 1-PSM chunk without a spectrum, for the probe kernels.
 struct ProbePsm {
-    TmpBuf buf;
+    DevBuf buf;
     PaBatchDev b;
 };
 
@@ -1946,7 +1854,7 @@ extern "C" int pa_fragment_table(pa_scorer* s, const uint8_t* pep, int32_t len, 
     ProbePsm pp;
     int rc = stage_probe_psm(s, pep, len, aux_pos, aux_mass, n_aux, std::max(charge, 1), pp);
     if (rc != PA_OK) return rc;
-    TmpBuf d_mz, d_nv;
+    DevBuf d_mz, d_nv;
     CK(d_mz.ensure((size_t)len * 16 * 4)); CK(d_nv.ensure((size_t)len * 4));
     CK(cudaMemset(d_mz.p, 0, (size_t)len * 16 * 4));
     PaFragArgs a;
@@ -1955,7 +1863,6 @@ extern "C" int pa_fragment_table(pa_scorer* s, const uint8_t* pep, int32_t len, 
     CK(cudaGetLastError());
     CK(cudaMemcpy(out_mz, d_mz.p, (size_t)len * 16 * 4, cudaMemcpyDeviceToHost));
     CK(cudaMemcpy(out_nvar, d_nv.p, (size_t)len * 4, cudaMemcpyDeviceToHost));
-    d_mz.release(); d_nv.release(); pp.buf.release();
     return PA_OK;
 }
 
@@ -1976,7 +1883,7 @@ extern "C" int pa_site_determining_ions(pa_scorer* s, const uint8_t* pep, int32_
     a.sig_a = sig_a; a.sig_b = sig_b; a.type = fragment_type; a.max_charge = max_charge;
     a.list_stride = 32;
     while (a.list_stride < per_type) a.list_stride <<= 1;
-    TmpBuf d_a, d_b, d_cnt, d_lists;
+    DevBuf d_a, d_b, d_cnt, d_lists;
     CK(d_a.ensure((size_t)a.list_stride * 4)); CK(d_b.ensure((size_t)a.list_stride * 4)); CK(d_cnt.ensure(8));
     if (per_type > PA_LCAP) CK(d_lists.ensure((size_t)4 * a.list_stride * sizeof(float)));
     a.out_a = d_a.as<float>(); a.out_b = d_b.as<float>(); a.counts = d_cnt.as<int32_t>(); a.g_lists = d_lists.as<float>();
@@ -1988,7 +1895,6 @@ extern "C" int pa_site_determining_ions(pa_scorer* s, const uint8_t* pep, int32_
     *n_a = cnt[0]; *n_b = cnt[1];
     if (std::min(cnt[0], cap) > 0) CK(cudaMemcpy(out_a, d_a.p, (size_t)std::min(cnt[0], cap) * 4, cudaMemcpyDeviceToHost));
     if (std::min(cnt[1], cap) > 0) CK(cudaMemcpy(out_b, d_b.p, (size_t)std::min(cnt[1], cap) * 4, cudaMemcpyDeviceToHost));
-    d_a.release(); d_b.release(); d_cnt.release(); d_lists.release(); pp.buf.release();
     return PA_OK;
 }
 
@@ -2008,7 +1914,7 @@ extern "C" int pa_log_math(pa_scorer* s, int32_t op, int32_t n, const float* x, 
     std::vector<double> logd(max_tr + 2);
     logd[0] = 0.;
     for (int m = 1; m <= max_tr + 1; m++) logd[m] = std::log((double)m);
-    TmpBuf d_in0, d_in1, d_logd, d_out;
+    DevBuf d_in0, d_in1, d_logd, d_out;
     CK(d_in0.ensure((size_t)n * 4)); CK(d_in1.ensure((size_t)n * 4)); CK(d_out.ensure((size_t)n * 4));
     CK(d_logd.ensure(logd.size() * 8));
     CK(cudaMemcpy(d_in0.p, op == 0 ? (const void*)x : (const void*)k, (size_t)n * 4, cudaMemcpyHostToDevice));
@@ -2025,7 +1931,6 @@ extern "C" int pa_log_math(pa_scorer* s, int32_t op, int32_t n, const float* x, 
     k_math_probe<<<(n + 127) / 128, 128>>>(a);
     CK(cudaGetLastError());
     CK(cudaMemcpy(out, d_out.p, (size_t)n * 4, cudaMemcpyDeviceToHost));
-    d_in0.release(); d_in1.release(); d_logd.release(); d_out.release();
     return PA_OK;
 }
 
