@@ -50,11 +50,15 @@ enum {
 
 /* Peak depth of a scoring handle.  The reference's weight vector has 10 entries (cpp/Ascore.cpp:15-19): n_top < 10 reads
  * out of bounds there; for n_top > 10 the PepScores, the isoform order, best_sequence and the alternative sites are
- * those of n_top = 10 (deeper ranks only add count / score columns and can move the depth calculateAmbiguity picks,
- * cpp/Ascore.cpp:165-175 -- shown on the compiled reference by tests/test_oracle_vs_ref.py::
- * test_reference_behaviour_for_n_top_above_10).  pa_create therefore takes n_top = 10 only -- the value
- * pyascore/__main__.py:69 hard-codes -- and reports anything else as PA_ERR_UNSUPPORTED. */
+ * those of n_top = 10, while deeper ranks add count / score columns for depths 10 .. n_top-1 and can move the depth
+ * calculateAmbiguity picks (cpp/Ascore.cpp:165-175 -- shown on the compiled reference by tests/test_oracle_vs_ref.py::
+ * test_reference_behaviour_for_n_top_above_10), so an Ascore may be computed at a depth >= 10.  pa_create takes
+ * PA_N_TOP <= n_top <= PA_MAX_N_TOP and computes all of that as the reference does; n_top < 10 (out-of-bounds reads in
+ * the reference) and n_top > 64 (beyond the tested envelope) are PA_ERR_UNSUPPORTED.  pyascore/__main__.py:69
+ * hard-codes n_top = 10.  Per-depth arrays of the ABI (pa_fetch_pep_scores, pa_calculate_ambiguity, pa_tail_table)
+ * are n_top wide. */
 #define PA_N_TOP 10
+#define PA_MAX_N_TOP 64
 #define PA_MAX_PEPTIDE 126
 #define PA_MAX_SITES 63
 #define PA_MAX_ISOFORMS (1ll << 26)
@@ -63,7 +67,7 @@ enum {
 
 /* Replaces PyAscore.__cinit__ (Ascore.pyx:64-73): BinnedSpectra(bin_size, n_top) +
  * ModifiedPeptide(mod_group, mod_mass, mz_error, fragment_types) + Ascore().
- * `device` is the CUDA ordinal.  n_top must be 10 (see PA_N_TOP). */
+ * `device` is the CUDA ordinal.  n_top in PA_N_TOP .. PA_MAX_N_TOP (see PA_N_TOP). */
 int pa_create(float bin_size, int n_top, const char* mod_group, float mod_mass, float mz_error,
               const char* fragment_types, int device, pa_scorer** out);
 
@@ -158,13 +162,14 @@ int pa_shard_ranges_for(const char* mod_group, int32_t n_types, int32_t nl_varia
 /* Replaces the pep_scores property (Ascore.pyx:240-252 -> cpp/Ascore.cpp:281-303) for PSM
  * `psm` of the last batch scored with PA_KEEP_ISOFORMS.  Rows come in the reference's order
  * (libstdc++ hash-iteration order + std::sort by descending weighted score).
- * sig: bit j = site j; counts/scores: [cap x PA_N_TOP] row-major.  Returns the number of isoforms
+ * sig: bit j = site j; counts/scores: [cap x n_top] row-major (the scorer's n_top).  Returns the number of isoforms
  * (>= 0; only min(cap, n) rows are written) or a negative pa_status. */
 int64_t pa_fetch_pep_scores(pa_scorer* s, int64_t psm, int64_t cap, uint64_t* sig, int32_t* counts,
                             float* scores, float* weighted, int32_t* total_fragments);
 
 /* Replaces PyAscore.calculate_ambiguity (Ascore.pyx:208-230 -> cpp/Ascore.cpp:157-210) against
- * the peptide/spectrum of PSM `psm` of the kept batch. */
+ * the peptide/spectrum of PSM `psm` of the kept batch.  scores_a / scores_b: the n_top depth scores of the two
+ * isoforms (a pep_scores row of the scorer's n_top). */
 int pa_calculate_ambiguity(pa_scorer* s, int64_t psm, uint64_t sig_a, const float* scores_a, float weighted_a,
                            uint64_t sig_b, const float* scores_b, float weighted_b, float* out);
 
@@ -219,7 +224,7 @@ int pa_log_math(pa_scorer* s, int32_t op, int32_t n, const float* x, const float
 int64_t pa_power_set_sums(const float* target, int32_t n, int32_t max_depth, float* out, int64_t cap);
 
 /* Stage probe: the score table |-10 log10 P(X >= k)| for depth d (0-based), n trials, k hits
- * (cpp/Util.cpp:47-83 + cpp/Ascore.cpp:127-133).  out[(n*(n+1)/2 + k)*PA_N_TOP + d], n <= n_max. */
+ * (cpp/Util.cpp:47-83 + cpp/Ascore.cpp:127-133).  out[(n*(n+1)/2 + k)*n_top + d], n <= n_max, d < the scorer's n_top. */
 int pa_tail_table(pa_scorer* s, int32_t n_max, float* out);
 
 typedef struct {
@@ -232,6 +237,8 @@ typedef struct {
                                            time the call spent waiting for the m/z narrowing pass (pa_narrow_mz) of a chunk */
     int64_t n_chunks;                   /* chunks the batch was cut into: every stage launches once per chunk */
     int64_t n_spec_exact;               /* spectra whose m/z kept an exact float64 copy beside the narrowed batch (pa_narrow_mz) */
+    int64_t launches_deep;              /* n_top > 10 only: launches of the depth 10 .. n_top-1 counting kernel (K2d), also in */
+    float ms_deep;                      /*   kernel_launches, and its CUDA-event time; both 0 for n_top = 10 */
 } pa_counters_t;
 
 /* Counters of the last pa_score_batch (roofline arithmetic: SURVEY.md section 8d). */

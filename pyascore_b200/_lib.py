@@ -10,7 +10,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # PYASCORE_B200_LIB selects another build of the same library (tuning variants under build/)
 SO_PATH = os.environ.get("PYASCORE_B200_LIB") or os.path.join(_HERE, "libpyascore_b200.so")
 
-PA_N_TOP = 10
+PA_N_TOP = 10          # depths the reference weights (and the default scoring depth)
+PA_MAX_N_TOP = 64      # deepest n_top a scorer takes (include/pyascore_b200.h)
 PA_KEEP_ISOFORMS = 1
 
 PSM_STATUS = {
@@ -39,7 +40,8 @@ class PaCounters(C.Structure):
                                          "n_fragment_lookups", "bytes_h2d", "bytes_d2h", "kernel_launches")] + \
                [(n, C.c_float) for n in ("ms_bin", "ms_plan", "ms_count", "ms_select", "ms_total")] + \
                [(n, C.c_int64) for n in ("launches_bin", "launches_count", "launches_select", "launches_ascore")] + \
-               [(n, C.c_float) for n in ("ms_ascore", "ms_narrow_wait")] + [("n_chunks", C.c_int64), ("n_spec_exact", C.c_int64)]
+               [(n, C.c_float) for n in ("ms_ascore", "ms_narrow_wait")] + [("n_chunks", C.c_int64), ("n_spec_exact", C.c_int64)] + \
+               [("launches_deep", C.c_int64), ("ms_deep", C.c_float)]
 
 
 EXPORTS = ["pa_create", "pa_add_neutral_loss", "pa_destroy", "pa_last_error", "pa_score_batch",

@@ -104,7 +104,8 @@ def _check(name, a):
 
 
 class Scorer:
-    """One pa_scorer: PyAscore's constructor arguments (Ascore.pyx:64-73) + a CUDA device."""
+    """One pa_scorer: PyAscore's constructor arguments (Ascore.pyx:64-73) + a CUDA device.  n_top: 10 .. 64
+    (_lib.PA_N_TOP .. _lib.PA_MAX_N_TOP); the per-depth arrays of the probes below are n_top wide."""
 
     def __init__(self, bin_size, n_top, mod_group, mod_mass, mz_error=.5, fragment_types="by", device=0):
         self.L = _lib.load()
@@ -119,6 +120,7 @@ class Scorer:
         self.h = h
         self.device = int(device)
         self.mod_group = mod_group
+        self.n_top = int(n_top)
 
     def close(self):
         if getattr(self, "h", None):
@@ -241,7 +243,7 @@ class Scorer:
         return omz, ork, ocnt[:n]
 
     def tail_table(self, n_max):
-        out = np.zeros(((n_max + 1) * (n_max + 2) // 2, _lib.PA_N_TOP), np.float32)
+        out = np.zeros(((n_max + 1) * (n_max + 2) // 2, self.n_top), np.float32)
         rc = self.L.pa_tail_table(self.h, n_max, out.ctypes.data)
         if rc != 0:
             self._raise(rc)
@@ -253,8 +255,8 @@ class Scorer:
         if n < 0:
             self._raise(int(n))
         sig = np.zeros(n, np.uint64)
-        cnt = np.zeros((n, _lib.PA_N_TOP), np.int32)
-        sc = np.zeros((n, _lib.PA_N_TOP), np.float32)
+        cnt = np.zeros((n, self.n_top), np.int32)
+        sc = np.zeros((n, self.n_top), np.float32)
         w = np.zeros(n, np.float32)
         tot = np.zeros(n, np.int32)
         if n:
@@ -267,8 +269,8 @@ class Scorer:
     def calculate_ambiguity(self, psm, sig_a, scores_a, w_a, sig_b, scores_b, w_b):
         sa = np.ascontiguousarray(scores_a, np.float32)
         sb = np.ascontiguousarray(scores_b, np.float32)
-        if sa.size != _lib.PA_N_TOP or sb.size != _lib.PA_N_TOP:
-            raise ValueError("scores must have %d entries" % _lib.PA_N_TOP)
+        if sa.size != self.n_top or sb.size != self.n_top:
+            raise ValueError("scores must have n_top = %d entries" % self.n_top)
         out = C.c_float()
         rc = self.L.pa_calculate_ambiguity(self.h, psm, int(sig_a), sa.ctypes.data, w_a, int(sig_b), sb.ctypes.data,
                                            w_b, C.byref(out))

@@ -39,10 +39,11 @@ __global__ void k_asc_item_count(PaAscArgs a, PaAscItemArgs it) {
 }
 
 // Ambiguity of the best isoform of entry t against its comp-th tied competitor (cpp/Ascore.cpp:157-210).
-// Returns false when a merge does not cover the shape (-> generic kernel).
-template <int NQ>
+// Returns false when a merge does not cover the shape (-> generic kernel).  DEEP: a scorer with n_top > 10, whose depth
+// argmax goes on over depths 10 .. n_top-1 (scores from dp.T at the K2d counts dp.cnt).
+template <int NQ, bool DEEP>
 __device__ __forceinline__ bool asc_pair(const PaCfg& cfg, const PaBatchDev& b, const PaAscArgs& a, int64_t t, int comp,
-                                         float& amb) {
+                                         float& amb, const PaDeep& dp) {
     const int32_t p = a.mod_psm[t];
     const int j = (int)(a.mod_lo + t - a.mod_off[p]);
     const int S = a.psm_S[p], k = b.n_mod[p];
@@ -107,21 +108,31 @@ __device__ __forceinline__ bool asc_pair(const PaCfg& cfg, const PaBatchDev& b, 
                                          __ldg(cfg.T + pa_tab_index(nfB, pa_cum_get(loB, hiB, d), d)));
             if (diff > max_diff) { max_diff = diff; depth = d; }
         }
+        if constexpr (DEEP) {
+            const uint16_t* cA = dp.cnt + (size_t)(ib + best) * dp.nd;
+            const uint16_t* cB = dp.cnt + (size_t)(ib + ci) * dp.nd;
+            for (int dd = 0; dd < dp.nd; dd++) {
+                const float diff = __fsub_rn(__ldg(dp.T + pa_tab_index_deep(nfA, cA[dd], dd, dp.nd)),
+                                             __ldg(dp.T + pa_tab_index_deep(nfB, cB[dd], dd, dp.nd)));
+                if (diff > max_diff) { max_diff = diff; depth = PA_N_TOP + dd; }
+            }
+        }
     }
     int hitsA = 0, hitsB = 0, trialsA = 0, trialsB = 0;
     for (int ti = 0; ti < cfg.n_types; ti++)
         if (!asc_merge_type<NQ>(cfg, q, pk, cfg.types[ti], alo, ahi, blo, bhi, depth, hitsA, trialsA, hitsB, trialsB))
             return false;
-    amb = __fsub_rn(__ldg(cfg.T + pa_tab_index(trialsA, hitsA, depth)), __ldg(cfg.T + pa_tab_index(trialsB, hitsB, depth)));
+    if constexpr (DEEP) amb = __fsub_rn(pa_depth_score(cfg.T, dp, trialsA, hitsA, depth), pa_depth_score(cfg.T, dp, trialsB, hitsB, depth));
+    else amb = __fsub_rn(__ldg(cfg.T + pa_tab_index(trialsA, hitsA, depth)), __ldg(cfg.T + pa_tab_index(trialsB, hitsB, depth)));
     return true;
 }
 
 #ifndef PA_ASC3_GRAB
 #define PA_ASC3_GRAB 1           // rounds of 32 pairs a warp takes per visit to the cursor
 #endif
-template <int NQ, int CLS>
+template <int NQ, int CLS, bool DEEP>
 __global__ void __launch_bounds__(128, (NQ <= 1 ? PA_ASC_MINBLOCKS : (NQ <= 2 ? PA_ASC2_MINBLOCKS : (NQ <= 4 ? PA_ASC4_MINBLOCKS : PA_ASC12_MINBLOCKS))))
-k_ascore_pairs(PaCfg cfg, PaBatchDev b, PaAscArgs a, PaAscItemArgs it) {
+k_ascore_pairs(PaCfg cfg, PaBatchDev b, PaAscArgs a, PaAscItemArgs it, PaDeep deep) {
     const int lane = threadIdx.x & 31;
     int64_t first = 0;                       // classes are contiguous in the sorted entry list, hence in the pair numbering
 #pragma unroll
@@ -142,7 +153,9 @@ k_ascore_pairs(PaCfg cfg, PaBatchDev b, PaAscArgs a, PaAscItemArgs it) {
             while (hi - lo > 1) { const int64_t mid = (lo + hi) >> 1; if ((int64_t)it.item_off[mid] <= g) lo = mid; else hi = mid; }
             const int64_t t = a.work_sorted[lo];
             float amb;
-            if (asc_pair<NQ>(cfg, b, a, t, (int)(g - it.item_off[lo]), amb)) {
+            // (`deep` is the last parameter, and the n_top = 10 form does not read it: its code stays that of the kernel
+            // before the parameter existed)
+            if (asc_pair<NQ, DEEP>(cfg, b, a, t, (int)(g - it.item_off[lo]), amb, DEEP ? deep : PaDeep())) {
                 if (a.ascores) asc_atomic_min(a.ascores + a.mod_lo + t, amb);
             } else if (atomicExch(it.gen_flag + t, 1) == 0)
                 a.generic_list[atomicAdd(a.generic_count, 1)] = (int32_t)t;

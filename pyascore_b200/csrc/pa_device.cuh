@@ -403,3 +403,21 @@ __device__ __forceinline__ int pa_nl_bump(int state, int idx) {   // idx 1-based
 __device__ __forceinline__ size_t pa_tab_index(int n, int k, int d) {
     return ((size_t)n * (size_t)(n + 1) / 2 + (size_t)k) * PA_N_TOP + (size_t)d;
 }
+
+// Depths 10 .. n_top-1 of a scorer with n_top > 10.  The score table of those depths is a second table beside T, with
+// the same rows: T_deep[(n(n+1)/2 + k) * nd + (d - 10)], nd = n_top - 10.  Per isoform of a chunk, K2d stores the
+// cumulative counts of those depths: cnt[(iso_off[p] + idx) * nd + (d - 10)].  nd = 0: a scorer of n_top = 10.
+struct PaDeep {
+    const float* T;
+    const uint16_t* cnt;
+    int nd;
+};
+
+__device__ __forceinline__ size_t pa_tab_index_deep(int n, int k, int dd, int nd) {
+    return ((size_t)n * (size_t)(n + 1) / 2 + (size_t)k) * (size_t)nd + (size_t)dd;
+}
+
+// score of depth d (0 .. n_top-1) at n trials and k hits
+__device__ __forceinline__ float pa_depth_score(const float* T, const PaDeep& dp, int n, int k, int d) {
+    return d < PA_N_TOP ? __ldg(T + pa_tab_index(n, k, d)) : __ldg(dp.T + pa_tab_index_deep(n, k, d - PA_N_TOP, dp.nd));
+}

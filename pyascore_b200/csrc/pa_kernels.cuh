@@ -4,6 +4,7 @@
 //                        spectra that are the rule (pa_bin_rows.cuh); k_bin_topn takes the ones it declines
 //   P1  k_plan           one thread per PSM: validation, #sites, #isoforms, work units
 //   K2  k_count_score    one warp per unit of <=1024 positional isoforms: fragments, matches, PepScore
+//   K2d k_count_deep     n_top > 10 only: one warp per K2 unit, lane per isoform: cumulative counts of depths 10..n_top-1
 //   K3a k_select_thread  one thread per PSM: reference-order best isoform, tied competitors per site,
 //                        sort keys of the Ascore entries; k_select (one warp per PSM) for the PSMs it declines
 //   K3b k_ascore_pairs   one thread per (PSM, modified site, tied competitor) pair, pairs handed out from a global
@@ -18,14 +19,21 @@
 // K0: score table  T[(n(n+1)/2 + k) * 10 + d] = | -10 * log10 P(X >= k) |,  X ~ Binomial(n, p_d)
 // cpp/Util.cpp:28-83 + cpp/Ascore.cpp:23-36, :127-133, in the reference's float32 rounding order.
 // logd[m] = log((double)m) and lps/lpf = logf(p_d), (float)log(1-p_d) are host constants from the
-// platform libm (the reference gets them from the same place).
+// platform libm (the reference gets them from the same place).  One thread per depth: depths 0..9 go to T, depths
+// 10 .. n_top-1 of a scorer with n_top > 10 to T_deep (PaDeep).
 // ---------------------------------------------------------------------------------------------
 struct PaTailArgs {
     float* T;
     const double* logd;
-    float lps[PA_N_TOP], lpf[PA_N_TOP];
+    float lps[PA_MAX_N_TOP], lpf[PA_MAX_N_TOP];
     double log10e;
+    float* T_deep;
+    int n_top;
 };
+
+__device__ __forceinline__ float* pa_tail_cell(const PaTailArgs& a, int n, int k, int d) {
+    return d < PA_N_TOP ? a.T + pa_tab_index(n, k, d) : a.T_deep + pa_tab_index_deep(n, k, d - PA_N_TOP, a.n_top - PA_N_TOP);
+}
 
 __global__ void __launch_bounds__(128) k_tail_table(PaTailArgs a, int n0, int n1) {
     extern __shared__ float s_lbc[];
@@ -39,16 +47,16 @@ __global__ void __launch_bounds__(128) k_tail_table(PaTailArgs a, int n0, int n1
         s_lbc[k] = c;
     }
     __syncthreads();
-    if (threadIdx.x < PA_N_TOP) {
+    if (threadIdx.x < a.n_top) {
         const int d = threadIdx.x;
         const float lps = a.lps[d], lpf = a.lpf[d];
         float tail = __int_as_float(0xff800000);   // -inf
-        a.T[pa_tab_index(n, 0, d)] = fabsf(__fmul_rn(-10.f, __double2float_rn(__dmul_rn(a.log10e, 0.0))));
+        *pa_tail_cell(a, n, 0, d) = fabsf(__fmul_rn(-10.f, __double2float_rn(__dmul_rn(a.log10e, 0.0))));
         for (int k = n; k >= 1; k--) {
             float pmf = __fadd_rn(__fadd_rn(s_lbc[k], __fmul_rn((float)k, lps)), __fmul_rn((float)(n - k), lpf));
             tail = pa_log_sum(tail, pmf);
             float l10 = __double2float_rn(__dmul_rn(a.log10e, (double)tail));
-            a.T[pa_tab_index(n, k, d)] = fabsf(__fmul_rn(-10.f, l10));
+            *pa_tail_cell(a, n, k, d) = fabsf(__fmul_rn(-10.f, l10));
         }
     }
 }
@@ -603,13 +611,11 @@ struct PaCountArgs {
 #define PA_K2_GRAB 4
 #endif
 // One fragment position: every neutral-loss variant and charge of running sum `run`, matched
-// against the staged peaks; adds the packed per-rank increments (`lut[r]`, lut[10] = 0 for "no
-// match") and returns the number of fragments emitted.
-template <bool HAS_NL, bool EGH>
-__device__ __forceinline__ int pa_emit_step(const PaCfg& cfg, const PsmInfo& info, const float* s_nl, float run,
-                                            int nls, double a1, double a2, double zm1, double zm2,
-                                            const ulonglong2* lut, unsigned long long& clo,
-                                            unsigned long long& chi) {
+// against the staged peaks; hands the rank of each fragment's match (255: none) to `hit` and
+// returns the number of fragments emitted.
+template <bool HAS_NL, bool EGH, class Hit>
+__device__ __forceinline__ int pa_emit_ranks(const PaCfg& cfg, const PsmInfo& info, const float* s_nl, float run,
+                                             int nls, double a1, double a2, double zm1, double zm2, Hit& hit) {
     const int Z = info.Z;
     int nv = 1;
     if (HAS_NL) nv = ((const uint8_t*)(s_nl + 256 * 16))[nls];       // variant counts sit behind the sums in shared memory
@@ -621,21 +627,9 @@ __device__ __forceinline__ int pa_emit_step(const PaCfg& cfg, const PsmInfo& inf
         if (HAS_NL) base = __fsub_rn(run, s_nl[nls * 16 + v]);
         const double d = __dsub_rn(__dadd_rn((double)base, a1), a2);
         // charge z: (d + z * 1.007825) / z  (cpp/ModifiedPeptide.cpp:585-587); 1 and 2 are unrolled
-        {
-            const int rk = pa_match_rank<EGH>(info, __double2float_rn(__dadd_rn(d, zm1)), cfg.err, cfg.err_gt_half);
-            const ulonglong2 inc = lut[rk < 10 ? rk : 10];
-            clo += inc.x; chi += inc.y;
-        }
-        if (Z >= 2) {
-            const int rk = pa_match_rank<EGH>(info, __double2float_rn(__dmul_rn(__dadd_rn(d, zm2), 0.5)), cfg.err, cfg.err_gt_half);
-            const ulonglong2 inc = lut[rk < 10 ? rk : 10];
-            clo += inc.x; chi += inc.y;
-        }
-        for (int z = 3; z <= Z; z++) {
-            const int rk = pa_match_rank<EGH>(info, pa_charge_mz(d, z), cfg.err, cfg.err_gt_half);
-            const ulonglong2 inc = lut[rk < 10 ? rk : 10];
-            clo += inc.x; chi += inc.y;
-        }
+        hit(pa_match_rank<EGH>(info, __double2float_rn(__dadd_rn(d, zm1)), cfg.err, cfg.err_gt_half));
+        if (Z >= 2) hit(pa_match_rank<EGH>(info, __double2float_rn(__dmul_rn(__dadd_rn(d, zm2), 0.5)), cfg.err, cfg.err_gt_half));
+        for (int z = 3; z <= Z; z++) hit(pa_match_rank<EGH>(info, pa_charge_mz(d, z), cfg.err, cfg.err_gt_half));
     }
     return nv * Z;
 }
@@ -643,14 +637,13 @@ __device__ __forceinline__ int pa_emit_step(const PaCfg& cfg, const PsmInfo& inf
 // Walk ion type `type` of the isoform with residue mask (mlo,mhi) from step `f` on, where the
 // float32 running sum / neutral-loss state before step f are (run, nls): the reference's
 // sequential adds are replayed for steps [f, s0) and fragments are emitted and matched for
-// steps [s0, s1).  Returns packed non-cumulative per-rank counts.
-template <bool HAS_NL, bool EGH>
-__device__ __forceinline__ void pa_walk_isoform(const PaCfg& cfg, const PsmSmem* sm, const PsmInfo& info,
-                                                const float* s_nl, uint64_t mlo, uint64_t mhi, char type, int f,
-                                                float run, int nls, int s0, int s1, const ulonglong2* lut,
-                                                unsigned long long& clo, unsigned long long& chi, uint32_t& nfrag) {
+// steps [s0, s1), each match's rank handed to `hit`.  Returns the number of fragments emitted.
+template <bool HAS_NL, bool EGH, class Hit>
+__device__ __forceinline__ uint32_t pa_walk_ranks(const PaCfg& cfg, const PsmSmem* sm, const PsmInfo& info,
+                                                  const float* s_nl, uint64_t mlo, uint64_t mhi, char type, int f,
+                                                  float run, int nls, int s0, int s1, Hit& hit) {
     const int L = info.L;
-    clo = 0; chi = 0; nfrag = 0;
+    uint32_t nfrag = 0;
     const bool fwd = (type == 'b' || type == 'c');
     double a1, a2;
     pa_type_consts(type, a1, a2);
@@ -676,12 +669,28 @@ __device__ __forceinline__ void pa_walk_isoform(const PaCfg& cfg, const PsmSmem*
             int idx = sm->nlidx[i][st];
             if (idx) nls = pa_nl_bump(nls, idx);
         }
-        nfrag += pa_emit_step<HAS_NL, EGH>(cfg, info, s_nl, run, nls, a1, a2, zm1, zm2, lut, clo, chi);
+        nfrag += pa_emit_ranks<HAS_NL, EGH>(cfg, info, s_nl, run, nls, a1, a2, zm1, zm2, hit);
     }
+    return nfrag;
+}
+
+// The same with packed non-cumulative per-rank counts of depths 0..9 (`lut[r]`, lut[10] = 0 for "no match" and for
+// the ranks >= 10).
+template <bool HAS_NL, bool EGH>
+__device__ __forceinline__ void pa_walk_isoform(const PaCfg& cfg, const PsmSmem* sm, const PsmInfo& info,
+                                                const float* s_nl, uint64_t mlo, uint64_t mhi, char type, int f,
+                                                float run, int nls, int s0, int s1, const ulonglong2* lut,
+                                                unsigned long long& clo, unsigned long long& chi, uint32_t& nfrag) {
+    clo = 0; chi = 0;
+    auto add = [&](int rk) {
+        const ulonglong2 inc = lut[rk < 10 ? rk : 10];
+        clo += inc.x; chi += inc.y;
+    };
+    nfrag = pa_walk_ranks<HAS_NL, EGH>(cfg, sm, info, s_nl, mlo, mhi, type, f, run, nls, s0, s1, add);
 }
 
 // ---- the walk of the common case: staged peaks with a cell index, 2 <= L <= 64 ------------------------------
-// Same arithmetic as pa_walk_isoform / pa_emit_step / pa_match_rank, fewer instructions per step: the residue states of
+// Same arithmetic as pa_walk_isoform / pa_emit_ranks / pa_match_rank, fewer instructions per step: the residue states of
 // the walk come off a 64-bit word one bit per step (reversed up front for the y-side walks) instead of a variable shift of
 // a 128-bit mask, the residue table is followed by a running shared-memory address, the peaks need no "are they staged"
 // test per lookup, and the increment table is read through a 32-bit shared address.
@@ -941,6 +950,60 @@ __global__ void __launch_bounds__(256, PA_K2_MINBLOCKS) k_count_score(PaCfg cfg,
     }
     for (int o = 16; o > 0; o >>= 1) lookups += __shfl_xor_sync(PA_FULL, lookups, o);
     if (lane == 0 && lookups) atomicAdd(a.n_lookups, lookups);
+}
+
+// ---------------------------------------------------------------------------------------------
+// K2d (n_top > 10 only, after K2): cumulative counts of depths 10 .. n_top-1 for every isoform of the chunk,
+// cnt_d = cnt_9 + sum of the ranks 10..d, with cnt_9 from K2.  One warp per K2 unit, one lane per isoform walking
+// every ion type with the reference's arithmetic (pa_walk_ranks); the ranks >= 10 go to the lane's own histogram in
+// shared memory.  K2 sees these ranks as "no match" (lut[10]), so its depth 0-9 counts and PepScores stand.
+// ---------------------------------------------------------------------------------------------
+struct PaDeepCountArgs {
+    int64_t n_units;
+    const int32_t* unit_psm;
+    const int32_t* unit_off;
+    const int64_t* iso_off;
+    const int32_t* psm_S;
+    const unsigned long long* iso_hi;   // K2's packed cumulative counts of depths 5..9
+    uint16_t* cnt;                      // [total isoforms * nd]
+    int nd;                             // n_top - 10
+};
+
+template <bool HAS_NL>
+__global__ void __launch_bounds__(128) k_count_deep(PaCfg cfg, PaBatchDev b, PaDeepCountArgs a) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    __shared__ float s_nl[HAS_NL ? 256 * 16 + 64 : 1];   // as in k_count_score
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5, wpb = blockDim.x >> 5;
+    if (HAS_NL) {
+        for (int i = threadIdx.x; i < 256 * 16; i += blockDim.x) s_nl[i] = cfg.nl_sums[i];
+        for (int i = threadIdx.x; i < 256; i += blockDim.x) ((uint8_t*)(s_nl + 256 * 16))[i] = cfg.nl_nvar[i];
+    }
+    __syncthreads();
+    const int nd = a.nd;
+    PsmSmem* sm = (PsmSmem*)smem_raw + wib;
+    uint16_t* hist = (uint16_t*)((PsmSmem*)smem_raw + wpb) + (size_t)(wib * 32 + lane) * nd;
+    auto add = [&](int rk) { if (rk >= PA_N_TOP && rk < PA_N_TOP + nd) hist[rk - PA_N_TOP]++; };
+    int64_t cur = -1;
+    PsmInfo info;
+    for (int64_t u = (int64_t)blockIdx.x * wpb + wib; u < a.n_units; u += (int64_t)gridDim.x * wpb) {
+        const int64_t p = a.unit_psm[u];
+        if (p != cur) { pa_setup_psm(cfg, b, p, sm, info, true); cur = p; }
+        const int64_t I = a.iso_off[p + 1] - a.iso_off[p];
+        const int S = a.psm_S[p];
+        const int64_t first = (int64_t)(u - a.unit_off[p]) * PA_UNIT;
+        const int cnt = (int)((I - first < PA_UNIT) ? I - first : PA_UNIT);
+        const int steps = (info.L == 1) ? 1 : info.L - 1;
+        for (int q = lane; q < cnt; q += 32) {
+            for (int d = 0; d < nd; d++) hist[d] = 0;
+            uint64_t mlo, mhi;
+            pa_sites_to_mask(sm, pa_unrank(cfg.binom, S, info.k, (uint32_t)(first + q)), mlo, mhi);
+            for (int t = 0; t < cfg.n_types; t++)
+                pa_walk_ranks<HAS_NL, true>(cfg, sm, info, s_nl, mlo, mhi, cfg.types[t], 0, 0.f, 0, 0, steps, add);
+            const int64_t g = a.iso_off[p] + first + q;
+            int c = (int)((a.iso_hi[g] >> 48) & 0xfffull);       // cumulative count of depth 9
+            for (int d = 0; d < nd; d++) { c += hist[d]; a.cnt[g * nd + d] = (uint16_t)c; }
+        }
+    }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1334,10 +1397,14 @@ __device__ __forceinline__ void pa_sdi_type(const PaCfg& cfg, SelSmem* sm, const
     __syncwarp();
 }
 
-// cpp/Ascore.cpp:157-210.  scA/scB: the ten depth scores of the two isoforms (lane-uniform arrays).
+// cpp/Ascore.cpp:157-210.  scA/scB: the depth scores of the two isoforms (lane-uniform arrays): ten, or with DEEP
+// (a scorer with n_top > 10) 10 + dp.nd, the argmax running over all of them and the final scores of a depth >= 10
+// coming from dp.T.
+template <bool DEEP>
 __device__ __forceinline__ float pa_ambiguity(const PaCfg& cfg, SelSmem* sm, const PsmInfo& info, uint64_t bitsA,
                                               const float* scA, float wA, uint64_t bitsB, const float* scB,
-                                              float wB, float* raw0, float* raw1, float* srt0, float* srt1) {
+                                              float wB, float* raw0, float* raw1, float* srt0, float* srt1,
+                                              const PaDeep& dp) {
     if ((double)fabsf(__fsub_rn(wA, wB)) < 1e-6) return 0.f;
     float max_diff = 0.f;
     int depth = 0;
@@ -1346,6 +1413,11 @@ __device__ __forceinline__ float pa_ambiguity(const PaCfg& cfg, SelSmem* sm, con
         float diff = __fsub_rn(scA[d], scB[d]);
         if (diff > max_diff) { max_diff = diff; depth = d; }
     }
+    if (DEEP)
+        for (int d = PA_N_TOP; d < PA_N_TOP + dp.nd; d++) {
+            float diff = __fsub_rn(scA[d], scB[d]);
+            if (diff > max_diff) { max_diff = diff; depth = d; }
+        }
     uint64_t alo, ahi, blo, bhi;
     pa_sites_to_mask(&sm->psm, bitsA, alo, ahi);
     pa_sites_to_mask(&sm->psm, bitsB, blo, bhi);
@@ -1353,6 +1425,7 @@ __device__ __forceinline__ float pa_ambiguity(const PaCfg& cfg, SelSmem* sm, con
     for (int t = 0; t < cfg.n_types; t++)
         pa_sdi_type(cfg, sm, info, cfg.types[t], alo, ahi, blo, bhi, raw0, raw1, srt0, srt1, depth, hitsA,
                     trialsA, hitsB, trialsB);
+    if (DEEP) return __fsub_rn(pa_depth_score(cfg.T, dp, trialsA, hitsA, depth), pa_depth_score(cfg.T, dp, trialsB, hitsB, depth));
     const float sA = __ldg(cfg.T + pa_tab_index(trialsA, hitsA, depth));
     const float sB = __ldg(cfg.T + pa_tab_index(trialsB, hitsB, depth));
     return __fsub_rn(sA, sB);
@@ -1362,6 +1435,12 @@ __device__ __forceinline__ void pa_depth_scores(const PaCfg& cfg, unsigned long 
                                                 int n, float* sc) {
 #pragma unroll
     for (int d = 0; d < PA_N_TOP; d++) sc[d] = __ldg(cfg.T + pa_tab_index(n, pa_cum_get(lo, hi, d), d));
+}
+
+// depths 10 .. n_top-1 of isoform g (K2d counts), into sc[10 ..]
+__device__ __forceinline__ void pa_deep_scores(const PaDeep& dp, int64_t g, int n, float* sc) {
+    for (int dd = 0; dd < dp.nd; dd++)
+        sc[PA_N_TOP + dd] = __ldg(dp.T + pa_tab_index_deep(n, dp.cnt[(size_t)g * dp.nd + dd], dd, dp.nd));
 }
 
 // position of the n-th set bit (n counted from 0) of a 128-bit mask
@@ -2105,9 +2184,11 @@ __device__ __forceinline__ int asc_site_pos(const PaCfg& cfg, const AscPep& q, i
 #endif
 #include "pa_ascore.cuh"
 
-// K3c: generic (warp-cooperative, list-materialising) Ascore for the entries k_ascore queued.
+// K3c: generic (warp-cooperative, list-materialising) Ascore for the entries k_ascore queued.  DEEP: n_top > 10 (see
+// asc_pair); `deep` comes last so that the parameters of the n_top = 10 form keep their offsets.
+template <bool DEEP>
 __global__ void __launch_bounds__(256) k_ascore_generic(PaCfg cfg, PaBatchDev b, PaAscArgs a, float* g_lists,
-                                                         int64_t list_stride) {
+                                                         int64_t list_stride, PaDeep deep) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5, wpb = blockDim.x >> 5;
     SelSmem* sm = (SelSmem*)smem_raw + wib;
@@ -2126,8 +2207,9 @@ __global__ void __launch_bounds__(256) k_ascore_generic(PaCfg cfg, PaBatchDev b,
         uint64_t rem = best_bits;
         for (int jj = 0; jj < j; jj++) rem &= rem - 1;
         const int site = __ffsll((long long)rem) - 1;
-        float scBest[PA_N_TOP];
+        float scBest[DEEP ? PA_MAX_N_TOP : PA_N_TOP];
         pa_depth_scores(cfg, a.iso.lo[ib + best], a.iso.hi[ib + best], (int)a.iso.nfrag[ib + best], scBest);
+        if (DEEP) pa_deep_scores(deep, ib + best, (int)a.iso.nfrag[ib + best], scBest);
         const float wbest = a.iso.w[ib + best];
         float* raw0 = sm->raw[0]; float* raw1 = sm->raw[1]; float* srt0 = sm->srt[0]; float* srt1 = sm->srt[1];
         long long per_type = (long long)(info.L > 1 ? info.L - 1 : 1) * cfg.nvar_cap * info.Z;
@@ -2140,10 +2222,11 @@ __global__ void __launch_bounds__(256) k_ascore_generic(PaCfg cfg, PaBatchDev b,
             const int u = __ffsll((long long)tt) - 1;
             const uint64_t cb = (best_bits & ~(1ull << site)) | (1ull << u);
             const uint32_t ci = pa_rank(cfg.binom, S, k, cb);
-            float scC[PA_N_TOP];
+            float scC[DEEP ? PA_MAX_N_TOP : PA_N_TOP];
             pa_depth_scores(cfg, a.iso.lo[ib + ci], a.iso.hi[ib + ci], (int)a.iso.nfrag[ib + ci], scC);
-            const float amb = pa_ambiguity(cfg, sm, info, best_bits, scBest, wbest, cb, scC, a.iso.w[ib + ci],
-                                           raw0, raw1, srt0, srt1);
+            if (DEEP) pa_deep_scores(deep, ib + ci, (int)a.iso.nfrag[ib + ci], scC);
+            const float amb = pa_ambiguity<DEEP>(cfg, sm, info, best_bits, scBest, wbest, cb, scC, a.iso.w[ib + ci],
+                                                 raw0, raw1, srt0, srt1, deep);
             asc = amb < asc ? amb : asc;
         }
         if (lane == 0 && a.ascores) a.ascores[a.mod_lo + t] = asc;
@@ -2154,17 +2237,19 @@ __global__ void __launch_bounds__(256) k_ascore_generic(PaCfg cfg, PaBatchDev b,
 // ---------------------------------------------------------------------------------------------
 // export of one PSM's per-isoform table (pep_scores) and a stand-alone ambiguity call
 // ---------------------------------------------------------------------------------------------
+// counts / scores rows are n_top = 10 + dp.nd wide
 __global__ void k_export_psm(PaCfg cfg, int64_t ib, int64_t I, int S, int k, PaIso iso, uint64_t* sig,
-                             int32_t* counts, float* scores, float* weighted, int32_t* total) {
+                             int32_t* counts, float* scores, float* weighted, int32_t* total, PaDeep dp) {
     int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= I) return;
     unsigned long long lo = iso.lo[ib + q], hi = iso.hi[ib + q];
     int n = (int)iso.nfrag[ib + q];
+    const int w = PA_N_TOP + dp.nd;
     sig[q] = pa_unrank(cfg.binom, S, k, (uint32_t)q);
-    for (int d = 0; d < PA_N_TOP; d++) {
-        int c = pa_cum_get(lo, hi, d);
-        counts[q * PA_N_TOP + d] = c;
-        scores[q * PA_N_TOP + d] = cfg.T[pa_tab_index(n, c, d)];
+    for (int d = 0; d < w; d++) {
+        int c = d < PA_N_TOP ? pa_cum_get(lo, hi, d) : dp.cnt[(size_t)(ib + q) * dp.nd + (d - PA_N_TOP)];
+        counts[q * w + d] = c;
+        scores[q * w + d] = pa_depth_score(cfg.T, dp, n, c, d);
     }
     weighted[q] = iso.w[ib + q];
     total[q] = n;
@@ -2173,11 +2258,12 @@ __global__ void k_export_psm(PaCfg cfg, int64_t ib, int64_t I, int S, int k, PaI
 struct PaAmbArgs {
     int64_t psm;
     uint64_t sigA, sigB;
-    float scA[PA_N_TOP], scB[PA_N_TOP];
+    float scA[PA_MAX_N_TOP], scB[PA_MAX_N_TOP];   // n_top entries
     float wA, wB;
     float* out;
     float* g_lists;
     int64_t list_stride;
+    PaDeep deep;                                   // nd = 0 for n_top = 10
 };
 
 __global__ void __launch_bounds__(32) k_ambiguity(PaCfg cfg, PaBatchDev b, PaAmbArgs a) {
@@ -2191,6 +2277,6 @@ __global__ void __launch_bounds__(32) k_ambiguity(PaCfg cfg, PaBatchDev b, PaAmb
         float* g = a.g_lists;
         raw0 = g; raw1 = g + a.list_stride; srt0 = g + 2 * a.list_stride; srt1 = g + 3 * a.list_stride;
     }
-    float r = pa_ambiguity(cfg, sm, info, a.sigA, a.scA, a.wA, a.sigB, a.scB, a.wB, raw0, raw1, srt0, srt1);
+    float r = pa_ambiguity<true>(cfg, sm, info, a.sigA, a.scA, a.wA, a.sigB, a.scB, a.wB, raw0, raw1, srt0, srt1, a.deep);
     if ((threadIdx.x & 31) == 0) *a.out = r;
 }

@@ -86,7 +86,7 @@ struct Slot {                // per-stream working set
     // plan
     DevBuf psm_S, psm_status, psm_I, psm_units, iso_off, unit_off, unit_psm, totals, cub_tmp;
     // K2/K3
-    DevBuf iso_lo, iso_hi, iso_n, iso_w, g_sort, g_lr, g_lists, lookups, sched, best_idx, mod_psm, tie, generic_list, generic_count, work_key, work_key2, work_val, work_sorted, rest_list, item_cnt, item_off, gen_flag, asc_cursor;
+    DevBuf iso_lo, iso_hi, iso_n, iso_w, iso_deep, g_sort, g_lr, g_lists, lookups, sched, best_idx, mod_psm, tie, generic_list, generic_count, work_key, work_key2, work_val, work_sorted, rest_list, item_cnt, item_off, gen_flag, asc_cursor;
     // staged outputs
     DevBuf o_sig, o_score, o_niso, o_nsites, o_asc, o_alt, o_status;
     PinnedBuf h_totals, h_lookups;       // PlanTotals, unsigned long long
@@ -104,6 +104,7 @@ struct ChunkView {           // device-side views of the chunk in flight (kept f
     const int32_t* psm_S = nullptr;
     const int32_t* psm_status = nullptr;
     PaIso iso;
+    const uint16_t* iso_deep = nullptr;    // n_top > 10: K2d counts
     int max_list = 0;
     bool valid = false;
     int slot = 0;
@@ -210,14 +211,16 @@ struct pa_scorer {
     std::string mod_group, frag_types;
     float bin_size = 100.f, mod_mass = 0.f, err = 0.5f;
     int n_top = PA_N_TOP;
+    int n_deep = 0;                        // scoring depths beyond 10: n_top - 10 (0 for a binner, whose n_top only bins)
     float nl_mass[256];
     bool nl_has[256];
     std::vector<float> nl_values;          // distinct non-zero loss masses, index+1 = device index
     bool nl_dirty = true;
     PaCfg cfg;
     DevBuf d_T, d_logd, d_binom, d_nl_sums, d_nl_nvar, d_perm_pool, d_perm_off, d_lut;
+    DevBuf d_T_deep;                       // n_top > 10: score table of depths 10 .. n_top-1 (PaDeep), same rows as d_T
     int table_n = -1;
-    float lps[PA_N_TOP], lpf[PA_N_TOP];
+    float lps[PA_MAX_N_TOP], lpf[PA_MAX_N_TOP];
     std::vector<int64_t> perm_off;         // [64*64]
     std::vector<uint32_t> perm_pool;
     bool perm_dirty = true;
@@ -484,8 +487,10 @@ static int ensure_table(pa_scorer* s, int n_max) {
     if (want < n_max) return fail(s, PA_ERR_UNSUPPORTED, "score table beyond %d trials", PA_MAX_FRAGMENTS);
     CK(cudaDeviceSynchronize());
     size_t entries = ((size_t)want + 1) * ((size_t)want + 2) / 2;
-    DevBuf nt;
+    const int nd = s->n_deep;                    // depths of the second table (PaDeep); 0 for n_top = 10
+    DevBuf nt, nt_deep;
     CK(nt.ensure(entries * PA_N_TOP * sizeof(float)));
+    if (nd > 0) CK(nt_deep.ensure(entries * nd * sizeof(float)));
     std::vector<double> logd(want + 2);
     logd[0] = 0.;
     for (int m = 1; m <= want + 1; m++) logd[m] = std::log((double)m);
@@ -494,13 +499,15 @@ static int ensure_table(pa_scorer* s, int n_max) {
     PaTailArgs a;
     a.T = nt.as<float>();
     a.logd = s->d_logd.as<double>();
-    for (int d = 0; d < PA_N_TOP; d++) { a.lps[d] = s->lps[d]; a.lpf[d] = s->lpf[d]; }
+    for (int d = 0; d < PA_N_TOP + nd; d++) { a.lps[d] = s->lps[d]; a.lpf[d] = s->lpf[d]; }
+    a.T_deep = nt_deep.as<float>(); a.n_top = PA_N_TOP + nd;
     volatile double one = 1.0;
     a.log10e = std::log10(std::exp(one));      // cpp/Util.cpp:82
     int n0 = 0;
     if (s->table_n >= 0) {                     // keep the rows already built
         size_t old_entries = ((size_t)s->table_n + 1) * ((size_t)s->table_n + 2) / 2;
         CK(cudaMemcpy(nt.p, s->d_T.p, old_entries * PA_N_TOP * sizeof(float), cudaMemcpyDeviceToDevice));
+        if (nd > 0) CK(cudaMemcpy(nt_deep.p, s->d_T_deep.p, old_entries * nd * sizeof(float), cudaMemcpyDeviceToDevice));
         n0 = s->table_n + 1;
     }
     int rows = want - n0 + 1;
@@ -508,6 +515,7 @@ static int ensure_table(pa_scorer* s, int n_max) {
     CK(cudaGetLastError());
     CK(cudaDeviceSynchronize());
     s->d_T = std::move(nt);                  // (nt takes the old table and frees it)
+    s->d_T_deep = std::move(nt_deep);
     s->table_n = want;
     s->cfg.T = s->d_T.as<float>();
     s->cfg.table_n = want;
@@ -605,9 +613,10 @@ static int create_scorer(float bin_size, int n_top, const char* mod_group, float
     pa_scorer* s = nullptr;
     if (!out || !mod_group || !fragment_types) return fail(nullptr, PA_ERR_ARG, "NULL argument");
     *out = nullptr;
-    if (binner_only ? (n_top < 1 || n_top > 254) : (n_top != PA_N_TOP))
-        return fail(nullptr, PA_ERR_UNSUPPORTED, "n_top must be %d (the reference's score weights have %d entries: "
-                    "smaller n_top reads out of bounds there, larger is ignored)", PA_N_TOP, PA_N_TOP);
+    if (binner_only ? (n_top < 1 || n_top > 254) : (n_top < PA_N_TOP || n_top > PA_MAX_N_TOP))
+        return fail(nullptr, PA_ERR_UNSUPPORTED, "n_top must be in %d..%d: below %d the reference reads past the end of its "
+                    "%d score weights; above %d is beyond what the oracle models and beyond the tested envelope",
+                    PA_N_TOP, PA_MAX_N_TOP, PA_N_TOP, PA_N_TOP, PA_MAX_N_TOP);
     if (!(bin_size > 0.f)) return fail(nullptr, PA_ERR_ARG, "bin_size must be positive");
     size_t nt = strlen(fragment_types);
     if (nt == 0 || nt > 7) return fail(nullptr, PA_ERR_ARG, "fragment_types must hold 1..7 characters");
@@ -639,13 +648,14 @@ static int create_scorer(float bin_size, int n_top, const char* mod_group, float
     cudaDeviceGetAttribute(&s->sm_count, cudaDevAttrMultiProcessorCount, device);
     s->mod_group = mod_group; s->frag_types = fragment_types;
     s->bin_size = bin_size; s->mod_mass = mod_mass; s->err = mz_error; s->n_top = n_top;
+    s->n_deep = binner_only ? 0 : n_top - PA_N_TOP;
     memset(s->nl_mass, 0, sizeof(s->nl_mass));
     memset(s->nl_has, 0, sizeof(s->nl_has));
     memset(&s->ctr, 0, sizeof(s->ctr));
     memset(&s->cfg, 0, sizeof(s->cfg));
     s->perm_off.assign(64 * 64, -1);
     // cpp/Ascore.cpp:23-36 + cpp/Util.cpp:52-55 (platform libm, like the reference)
-    for (int d = 1; d <= PA_N_TOP; d++) {
+    for (int d = 1; d <= PA_N_TOP + s->n_deep; d++) {
         float p = (float)((double)((2 * mz_error) * (float)d) / 100.);
         s->lps[d - 1] = logf(p);
         s->lpf[d - 1] = (float)log(1. - (double)p);
@@ -677,8 +687,14 @@ static int create_scorer(float bin_size, int n_top, const char* mod_group, float
             CK(cudaEventCreateWithFlags(&s->slot[i].ev_plan, cudaEventDisableTiming));
             CK(cudaEventCreateWithFlags(&s->nstage[i].ev, cudaEventDisableTiming));
         }
-        CK(cudaFuncSetAttribute(k_ascore_generic, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        CK(cudaFuncSetAttribute(k_ascore_pairs<PA_MAXSTREAM, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(AscSm)));
+        CK(cudaFuncSetAttribute(k_ascore_generic<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+        CK(cudaFuncSetAttribute(k_ascore_pairs<PA_MAXSTREAM, 3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(AscSm)));
+        if (s->n_deep > 0) {
+            CK(cudaFuncSetAttribute(k_ascore_generic<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            CK(cudaFuncSetAttribute(k_ascore_pairs<PA_MAXSTREAM, 3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(AscSm)));
+            CK(cudaFuncSetAttribute(k_count_deep<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+            CK(cudaFuncSetAttribute(k_count_deep<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+        }
         CK(cudaFuncSetAttribute(k_bin_topn<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
         CK(cudaFuncSetAttribute(k_bin_topn<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
         for (int v = 0; v < 4; v++)
@@ -867,6 +883,7 @@ struct ChunkState {              // what the back half of a chunk needs from the
     int64_t mod_lo = 0, mod_hi = 0;
     const int64_t* mod_off_abs = nullptr;
     cudaEvent_t e_bin0, e_bin1, e_plan1, e_cnt0, e_cnt1, e_sel1, e_asc1;
+    cudaEvent_t e_deep1 = nullptr;   // n_top > 10: end of K2d (which starts at e_cnt1)
     uint64_t* o_sig; float* o_score; int64_t* o_niso; int32_t* o_nsites; float* o_asc; uint64_t* o_alt; int32_t* o_status;
     ChunkArray res[7];               // the result arrays (views: the o_* above)
     bool single_chunk = false;       // the call has one chunk
@@ -1168,6 +1185,33 @@ static int chunk_back(pa_scorer* s, int si, const pa_results* out, bool out_dev,
         s->ctr.kernel_launches++; s->ctr.launches_count++;
     }
     CK(cudaEventRecord(cs.e_cnt1, st));
+    // K2d: depths 10 .. n_top-1 (n_top > 10 only)
+    PaDeep deep;
+    deep.nd = s->n_deep; deep.T = s->d_T_deep.as<float>(); deep.cnt = nullptr;
+    if (deep.nd > 0) {
+        CK(sl.iso_deep.ensure((size_t)std::max<int64_t>(total_iso, 1) * deep.nd * sizeof(uint16_t)));
+        deep.cnt = sl.iso_deep.as<uint16_t>();
+        cs.e_deep1 = next_event(s);
+        if (n_units > 0) {
+            PaDeepCountArgs da;
+            da.n_units = n_units; da.unit_psm = sl.unit_psm.as<int32_t>(); da.unit_off = sl.unit_off.as<int32_t>();
+            da.iso_off = sl.iso_off.as<int64_t>(); da.psm_S = sl.psm_S.as<int32_t>(); da.iso_hi = iso.hi;
+            da.cnt = sl.iso_deep.as<uint16_t>(); da.nd = deep.nd;
+            const int wpb = 4;
+            const size_t smem = wpb * (sizeof(PsmSmem) + 32 * deep.nd * sizeof(uint16_t));
+            const int64_t want = ((int64_t)n_units + wpb - 1) / wpb;
+            if (s->cfg.has_nl) {
+                const int blocks = (int)std::min<int64_t>(want, (int64_t)s->sm_count * resident_blocks(k_count_deep<true>, wpb * 32, smem));
+                k_count_deep<true><<<blocks, wpb * 32, smem, st>>>(s->cfg, cs.b, da);
+            } else {
+                const int blocks = (int)std::min<int64_t>(want, (int64_t)s->sm_count * resident_blocks(k_count_deep<false>, wpb * 32, smem));
+                k_count_deep<false><<<blocks, wpb * 32, smem, st>>>(s->cfg, cs.b, da);
+            }
+            CK(cudaGetLastError());
+            s->ctr.kernel_launches++; s->ctr.launches_deep++;
+        }
+        CK(cudaEventRecord(cs.e_deep1, st));
+    }
     // outputs
     const int64_t nm = cs.mod_hi - cs.mod_lo;
     ChunkArray* res = cs.res;
@@ -1267,9 +1311,15 @@ static int chunk_back(pa_scorer* s, int si, const pa_results* out, bool out_dev,
         ts = sl.cub_tmp.cap;
         CK(cub::DeviceScan::ExclusiveSum(sl.cub_tmp.p, ts, ia.item_cnt, sl.item_off.as<int32_t>(), (int)(nm + 1), st));
         s->ctr.kernel_launches += 2;
+        // (n_top > 10: the DEEP instantiations, whose depth argmax goes on over depths 10 .. n_top-1)
 #define PA_PAIRS_LAUNCH(NQ, CLS, SMEM) { \
-            const int blocks = (int)std::min<int64_t>(ab, (int64_t)s->sm_count * resident_blocks(k_ascore_pairs<NQ, CLS>, 128, SMEM)); \
-            k_ascore_pairs<NQ, CLS><<<blocks, 128, SMEM, st>>>(s->cfg, cs.b, aa, ia); }
+            if (deep.nd > 0) { \
+                const int blocks = (int)std::min<int64_t>(ab, (int64_t)s->sm_count * resident_blocks(k_ascore_pairs<NQ, CLS, true>, 128, SMEM)); \
+                k_ascore_pairs<NQ, CLS, true><<<blocks, 128, SMEM, st>>>(s->cfg, cs.b, aa, ia, deep); \
+            } else { \
+                const int blocks = (int)std::min<int64_t>(ab, (int64_t)s->sm_count * resident_blocks(k_ascore_pairs<NQ, CLS, false>, 128, SMEM)); \
+                k_ascore_pairs<NQ, CLS, false><<<blocks, 128, SMEM, st>>>(s->cfg, cs.b, aa, ia, deep); \
+            } }
         if (!s->cfg.has_nl) {
             PA_PAIRS_LAUNCH(1, 0, 0) PA_PAIRS_LAUNCH(2, 1, 0) PA_PAIRS_LAUNCH(4, 2, 0)
             s->ctr.kernel_launches += 3;
@@ -1282,7 +1332,8 @@ static int chunk_back(pa_scorer* s, int si, const pa_results* out, bool out_dev,
         int64_t stride = 32;
         while (stride < T.max_list) stride <<= 1;
         if (T.max_list > PA_LCAP) CK(sl.g_lists.ensure((size_t)blocks * wpb * 4 * stride * sizeof(float)));
-        k_ascore_generic<<<blocks, wpb * 32, wpb * sizeof(SelSmem), st>>>(s->cfg, cs.b, aa, sl.g_lists.as<float>(), stride);
+        if (deep.nd > 0) k_ascore_generic<true><<<blocks, wpb * 32, wpb * sizeof(SelSmem), st>>>(s->cfg, cs.b, aa, sl.g_lists.as<float>(), stride, deep);
+        else k_ascore_generic<false><<<blocks, wpb * 32, wpb * sizeof(SelSmem), st>>>(s->cfg, cs.b, aa, sl.g_lists.as<float>(), stride, deep);
         CK(cudaGetLastError());
         s->ctr.kernel_launches += 2; s->ctr.launches_ascore += 2;
     }
@@ -1299,6 +1350,7 @@ static int chunk_back(pa_scorer* s, int si, const pa_results* out, bool out_dev,
         s->kept.b = cs.b; s->kept.n_psm = np; s->kept.psm_lo = r.p0;
         s->kept.iso_off = sl.iso_off.as<int64_t>(); s->kept.psm_S = sl.psm_S.as<int32_t>();
         s->kept.psm_status = sl.psm_status.as<int32_t>(); s->kept.iso = iso; s->kept.max_list = T.max_list;
+        s->kept.iso_deep = deep.cnt;
         s->kept.valid = true; s->kept.slot = si;
     }
     return PA_OK;
@@ -1488,7 +1540,8 @@ static int score_impl(pa_scorer* s, const pa_batch* in, const pa_results* out, i
         cudaEventElapsedTime(&ms, cs[c].e_bin0, cs[c].e_bin1); s->ctr.ms_bin += ms;
         cudaEventElapsedTime(&ms, cs[c].e_bin1, cs[c].e_plan1); s->ctr.ms_plan += ms;
         cudaEventElapsedTime(&ms, cs[c].e_cnt0, cs[c].e_cnt1); s->ctr.ms_count += ms;
-        cudaEventElapsedTime(&ms, cs[c].e_cnt1, cs[c].e_sel1); s->ctr.ms_select += ms;
+        if (cs[c].e_deep1) { cudaEventElapsedTime(&ms, cs[c].e_cnt1, cs[c].e_deep1); s->ctr.ms_deep += ms; }
+        cudaEventElapsedTime(&ms, cs[c].e_deep1 ? cs[c].e_deep1 : cs[c].e_cnt1, cs[c].e_sel1); s->ctr.ms_select += ms;
         cudaEventElapsedTime(&ms, cs[c].e_sel1, cs[c].e_asc1); s->ctr.ms_ascore += ms;
     }
     cudaEventElapsedTime(&s->ctr.ms_total, e_all0, e_all1);
@@ -1590,17 +1643,20 @@ extern "C" int64_t pa_fetch_pep_scores(pa_scorer* s, int64_t psm, int64_t cap, u
     CK(cudaMemcpy(&k, s->kept.b.n_mod + q, 4, cudaMemcpyDeviceToHost));
     const int64_t I = off[1] - off[0];
     if (I <= 0 || status != PA_PSM_OK) return 0;
+    const int64_t D = PA_N_TOP + s->n_deep;   // row width of counts / scores: the scorer's n_top
+    PaDeep deep;
+    deep.nd = s->n_deep; deep.T = s->d_T_deep.as<float>(); deep.cnt = s->kept.iso_deep;
     DevBuf d_sig, d_cnt, d_sc, d_w, d_tot;
-    CK(d_sig.ensure(I * 8)); CK(d_cnt.ensure(I * PA_N_TOP * 4)); CK(d_sc.ensure(I * PA_N_TOP * 4));
+    CK(d_sig.ensure(I * 8)); CK(d_cnt.ensure(I * D * 4)); CK(d_sc.ensure(I * D * 4));
     CK(d_w.ensure(I * 4)); CK(d_tot.ensure(I * 4));
     k_export_psm<<<(unsigned)((I + 127) / 128), 128>>>(s->cfg, off[0], I, S, k, s->kept.iso, d_sig.as<uint64_t>(),
-                                                        d_cnt.as<int32_t>(), d_sc.as<float>(), d_w.as<float>(), d_tot.as<int32_t>());
+                                                        d_cnt.as<int32_t>(), d_sc.as<float>(), d_w.as<float>(), d_tot.as<int32_t>(), deep);
     CK(cudaGetLastError());
-    std::vector<uint64_t> h_sig(I); std::vector<int32_t> h_cnt(I * PA_N_TOP), h_tot(I);
-    std::vector<float> h_sc(I * PA_N_TOP), h_w(I);
+    std::vector<uint64_t> h_sig(I); std::vector<int32_t> h_cnt(I * D), h_tot(I);
+    std::vector<float> h_sc(I * D), h_w(I);
     CK(cudaMemcpy(h_sig.data(), d_sig.p, I * 8, cudaMemcpyDeviceToHost));
-    CK(cudaMemcpy(h_cnt.data(), d_cnt.p, I * PA_N_TOP * 4, cudaMemcpyDeviceToHost));
-    CK(cudaMemcpy(h_sc.data(), d_sc.p, I * PA_N_TOP * 4, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(h_cnt.data(), d_cnt.p, I * D * 4, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(h_sc.data(), d_sc.p, I * D * 4, cudaMemcpyDeviceToHost));
     CK(cudaMemcpy(h_w.data(), d_w.p, I * 4, cudaMemcpyDeviceToHost));
     CK(cudaMemcpy(h_tot.data(), d_tot.p, I * 4, cudaMemcpyDeviceToHost));
     // listing order: hash-iteration order, then std::sort by descending weighted score unless
@@ -1619,8 +1675,8 @@ extern "C" int64_t pa_fetch_pep_scores(pa_scorer* s, int64_t psm, int64_t cap, u
     for (int64_t i = 0; i < I && i < cap; i++) {
         uint32_t id = order[i];
         if (sig) sig[i] = h_sig[id];
-        if (counts) memcpy(counts + i * PA_N_TOP, &h_cnt[id * PA_N_TOP], PA_N_TOP * 4);
-        if (scores) memcpy(scores + i * PA_N_TOP, &h_sc[id * PA_N_TOP], PA_N_TOP * 4);
+        if (counts) memcpy(counts + i * D, &h_cnt[id * D], D * 4);
+        if (scores) memcpy(scores + i * D, &h_sc[id * D], D * 4);
         if (weighted) weighted[i] = h_w[id];
         if (total_fragments) total_fragments[i] = h_tot[id];
     }
@@ -1635,7 +1691,8 @@ extern "C" int pa_calculate_ambiguity(pa_scorer* s, int64_t psm, uint64_t sig_a,
     CK(cudaSetDevice(s->device));
     PaAmbArgs a;
     a.psm = psm - s->kept.psm_lo; a.sigA = sig_a; a.sigB = sig_b; a.wA = weighted_a; a.wB = weighted_b;
-    memcpy(a.scA, scores_a, sizeof(a.scA)); memcpy(a.scB, scores_b, sizeof(a.scB));
+    memcpy(a.scA, scores_a, (PA_N_TOP + s->n_deep) * sizeof(float)); memcpy(a.scB, scores_b, (PA_N_TOP + s->n_deep) * sizeof(float));
+    a.deep.nd = s->n_deep; a.deep.T = s->d_T_deep.as<float>(); a.deep.cnt = s->kept.iso_deep;
     DevBuf d_out, d_lists;
     CK(d_out.ensure(4));
     a.list_stride = 32;
@@ -1949,7 +2006,16 @@ extern "C" int pa_tail_table(pa_scorer* s, int32_t n_max, float* out) {
     int rc = ensure_table(s, n_max);
     if (rc != PA_OK) return rc;
     size_t entries = ((size_t)n_max + 1) * ((size_t)n_max + 2) / 2;
-    CK(cudaMemcpy(out, s->d_T.p, entries * PA_N_TOP * sizeof(float), cudaMemcpyDeviceToHost));
+    const int nd = s->n_deep;
+    if (nd == 0) {
+        CK(cudaMemcpy(out, s->d_T.p, entries * PA_N_TOP * sizeof(float), cudaMemcpyDeviceToHost));
+        return PA_OK;
+    }
+    // rows of n_top: depths 0..9 from T, 10 .. n_top-1 from T_deep (strided copies straight into the caller's rows)
+    CK(cudaMemcpy2D(out, (size_t)(PA_N_TOP + nd) * sizeof(float), s->d_T.p, PA_N_TOP * sizeof(float), PA_N_TOP * sizeof(float),
+                    entries, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy2D(out + PA_N_TOP, (size_t)(PA_N_TOP + nd) * sizeof(float), s->d_T_deep.p, nd * sizeof(float), nd * sizeof(float),
+                    entries, cudaMemcpyDeviceToHost));
     return PA_OK;
 }
 
