@@ -1050,16 +1050,10 @@ struct PaSelArgs {
     uint16_t* work_key;          // [entries] sort key of each mod entry: stream class << 10 | (1023 - estimated merge
     int32_t* work_val;           // [entries]   trips), PA_WORK_NONE = no site-determining-ion comparison needed; identity
     int* work_count;             // [4] entries per stream class (k_ascore)
-    const int32_t* order;        // optional visiting order of the PSMs (null = input order)
-    unsigned long long* next_psm;    // work cursor (zeroed before the launch)
-    int32_t* rest_list;              // PSMs k_select_thread leaves to k_select (large isoform sets, tied top scores)
-    int* rest_count;
-    const int* n_psm_dev;            // k_select: number of PSMs to visit when it is only known on the device (else null)
-    int grab;                        // PSMs per visit to the cursor: 1 .. PA_SEL_GRAB; negative: no reservation ahead
+    unsigned long long* next_psm;    // k_select's cursor into rest_list (zeroed before the launch)
+    int32_t* rest_list;              // PSMs k_select_thread declines, for k_select (large isoform sets, tied top scores)
+    int* rest_count;                 // their number (zeroed before the launch)
 };
-#ifndef PA_SEL_GRAB
-#define PA_SEL_GRAB 16
-#endif
 #define PA_WORK_BITS 13
 #ifndef PA_WORK_SHIFT
 #define PA_WORK_SHIFT 5      // low bits of the trip estimate dropped from the key (coarser classes keep more input order)
@@ -1067,8 +1061,8 @@ struct PaSelArgs {
 #define PA_WORK_NONE 0x1fffu
 
 // --- libstdc++ std::sort (introsort + final insertion sort), comparator a.w > b.w ------------
-// bits/stl_algo.h of GCC 13, as in SURVEY.md appendix A.2.  Elements are (float w, uint32 id)
-// packed in 64 bits: w in the high word.  Run by ONE lane.
+// bits/stl_algo.h of GCC 13, as in SURVEY.md appendix A.2: the steps that decide its first element.
+// Elements are (float w, uint32 id) packed in 64 bits: w in the high word.  The heap sort is run by ONE lane.
 __device__ __forceinline__ float srt_w(unsigned long long e) { return __int_as_float((int)(e >> 32)); }
 #define SRT_CMP(x, y) (srt_w(x) > srt_w(y))
 
@@ -1101,61 +1095,6 @@ __device__ void srt_heap_sort(unsigned long long* a, long n) {
         a[last] = a[0];
         srt_adjust_heap(a, 0, last, v);
     }
-}
-
-__device__ __forceinline__ void srt_linear_insert(unsigned long long* a, long i) {
-    unsigned long long v = a[i];
-    long j = i - 1;
-    while (SRT_CMP(v, a[j])) { a[j + 1] = a[j]; j--; }
-    a[j + 1] = v;
-}
-
-__device__ __forceinline__ void srt_insertion(unsigned long long* a, long first, long last) {
-    for (long i = first + 1; i < last; i++) {
-        if (SRT_CMP(a[i], a[first])) {
-            unsigned long long v = a[i];
-            for (long j = i; j > first; j--) a[j] = a[j - 1];
-            a[first] = v;
-        } else srt_linear_insert(a, i);
-    }
-}
-
-__device__ void pa_gcc_sort(unsigned long long* a, long n) {
-    if (n < 2) return;
-    long lg = 0;
-    for (long t = n; t > 1; t >>= 1) lg++;
-    // __introsort_loop with an explicit stack instead of recursion (the recursion is on the right part)
-    long stk_first[64], stk_last[64], stk_depth[64];
-    int sp = 0;
-    stk_first[0] = 0; stk_last[0] = n; stk_depth[0] = 2 * lg; sp = 1;
-    while (sp > 0) {
-        sp--;
-        long first = stk_first[sp], last = stk_last[sp], depth = stk_depth[sp];
-        // the reference processes [cut,last) recursively FIRST, then loops on [first,cut).  The
-        // order in which disjoint ranges are partitioned does not change the result.
-        while (last - first > 16) {
-            if (depth == 0) { srt_heap_sort(a + first, last - first); break; }
-            --depth;
-            long mid = first + (last - first) / 2;
-            long x = first + 1, y = mid, z = last - 1, pick;
-            if (SRT_CMP(a[x], a[y])) { if (SRT_CMP(a[y], a[z])) pick = y; else if (SRT_CMP(a[x], a[z])) pick = z; else pick = x; }
-            else if (SRT_CMP(a[x], a[z])) pick = x; else if (SRT_CMP(a[y], a[z])) pick = z; else pick = y;
-            { unsigned long long t = a[first]; a[first] = a[pick]; a[pick] = t; }
-            long f = first + 1, l = last;
-            for (;;) {
-                while (SRT_CMP(a[f], a[first])) f++;
-                --l;
-                while (SRT_CMP(a[first], a[l])) l--;
-                if (!(f < l)) break;
-                { unsigned long long t = a[f]; a[f] = a[l]; a[l] = t; }
-                f++;
-            }
-            if (sp < 64) { stk_first[sp] = f; stk_last[sp] = last; stk_depth[sp] = depth; sp++; }
-            last = f;
-        }
-    }
-    if (n > 16) { srt_insertion(a, 0, 16); for (long i = 16; i < n; i++) srt_linear_insert(a, i); }
-    else srt_insertion(a, 0, n);
 }
 
 // Only the element std::sort would leave at index 0 is needed on the device (the full listing
@@ -1453,6 +1392,29 @@ __device__ __forceinline__ int pa_nth_set(uint64_t lo, uint64_t hi, int n) {
     return base + __ffsll((long long)x) - 1;
 }
 
+// K3a, the Ascore-0 shortcut: every tied competitor has exactly the score m; within 1e-6 of the best score wb the
+// ambiguity is 0 without looking at any ion (cpp/Ascore.cpp:161-163), so the Ascore (the minimum over the tie set)
+// is 0.
+__device__ __forceinline__ bool pa_asc_zero(float wb, float m) { return (double)fabsf(__fsub_rn(wb, m)) < 1e-6; }
+
+// K3a, the sort key of an Ascore entry that goes to k_ascore: stream class `cls` (so that the lanes of a k_ascore
+// warp run the same code), then the estimated number of merge trips, longest first -- per tied competitor one trip
+// per residue plus three per residue between the two sites, times the charges -- and the host sorts the entries by
+// it, so that the lanes of a warp also finish together.  pos(s) is the residue index of site s.
+template <class Pos>
+__device__ __forceinline__ uint32_t pa_work_key(const PaCfg& cfg, int Z, int L, int site, uint64_t tie, Pos pos,
+                                                int& cls) {
+    cls = cfg.has_nl ? 3 : (Z == 1 ? 0 : (Z == 2 ? 1 : (Z <= 4 ? 2 : 3)));
+    int work = 0;
+    const int ps = pos(site);
+    for (uint64_t tt = tie; tt; tt &= tt - 1) {
+        const int pu = pos(__ffsll((long long)tt) - 1);
+        work += (L - 1) + 3 * (pu > ps ? pu - ps : ps - pu);
+    }
+    work *= Z < 8 ? Z : 8;
+    return ((uint32_t)cls << 10) | (((uint32_t)(1023 - (work > 1023 ? 1023 : work)) >> PA_WORK_SHIFT) << PA_WORK_SHIFT);
+}
+
 // K3a, common case: one THREAD per PSM.  A PSM of config-2 size has a dozen isoforms and a handful of
 // sites: a warp per PSM spends its instructions on reductions over mostly empty lanes.  A thread walks
 // the same steps serially (best isoform, per modified site the tied best competitors, Ascore-0 shortcut,
@@ -1529,7 +1491,7 @@ __global__ void __launch_bounds__(128) k_select_thread(PaCfg cfg, PaBatchDev b, 
                 if (a.best_sig) a.best_sig[p] = best_bits;
                 if (a.best_score) a.best_score[p] = wb;
                 a.best_idx[p] = best;
-                // residues that are sites, for the merge-length estimate (see k_select)
+                // residues that are sites, for the merge-length estimate (see pa_work_key)
                 const int pep0 = b.pep_off[p], L = b.pep_off[p + 1] - pep0;
                 uint64_t slo = 0, shi = 0;
                 if (a.ascores)
@@ -1558,21 +1520,12 @@ __global__ void __launch_bounds__(128) k_select_thread(PaCfg cfg, PaBatchDev b, 
                     a.mod_psm[mo + j - a.mod_lo] = (int32_t)p;
                     if (a.ascores) {
                         uint32_t key = PA_WORK_NONE;
-                        // every tied competitor has exactly the score m; within 1e-6 of the best score the
-                        // ambiguity is 0 without looking at any ion (cpp/Ascore.cpp:161-163)
-                        if ((double)fabsf(__fsub_rn(wb, m)) < 1e-6) a.ascores[mo + j] = 0.f;
+                        if (pa_asc_zero(wb, m)) a.ascores[mo + j] = 0.f;
                         else {
-                            const int Z = b.max_charge[p];
-                            const int cls = cfg.has_nl ? 3 : (Z == 1 ? 0 : (Z == 2 ? 1 : (Z <= 4 ? 2 : 3)));
+                            int cls;
+                            key = pa_work_key(cfg, b.max_charge[p], L, site, tie,
+                                              [&](int s) { return pa_nth_set(slo, shi, s); }, cls);
                             atomicAdd(&s_cls[cls], 1);
-                            int work = 0;
-                            const int ps = pa_nth_set(slo, shi, site);
-                            for (uint64_t tt = tie; tt; tt &= tt - 1) {
-                                const int pu = pa_nth_set(slo, shi, __ffsll((long long)tt) - 1);
-                                work += (L - 1) + 3 * (pu > ps ? pu - ps : ps - pu);
-                            }
-                            work *= Z < 8 ? Z : 8;
-                            key = ((uint32_t)cls << 10) | (((uint32_t)(1023 - (work > 1023 ? 1023 : work)) >> PA_WORK_SHIFT) << PA_WORK_SHIFT);
                         }
                         a.work_key[mo + j - a.mod_lo] = (uint16_t)key;
                         a.work_val[mo + j - a.mod_lo] = (int32_t)(mo + j - a.mod_lo);
@@ -1585,64 +1538,38 @@ __global__ void __launch_bounds__(128) k_select_thread(PaCfg cfg, PaBatchDev b, 
     if (threadIdx.x < 4 && s_cls[threadIdx.x]) atomicAdd(a.work_count + threadIdx.x, s_cls[threadIdx.x]);
 }
 
-// K3a: warp per PSM.  Best isoform in the reference's order + per modified site the set of tied
-// best competitors (= alternative sites).  The Ascore of every (PSM, site) entry is then computed
-// by k_ascore (thread per entry) or, for the rare shapes that kernel does not cover, k_ascore_generic.
+// K3a for the PSMs k_select_thread declines: one WARP per PSM, taken from rest_list.  Every PSM here has status
+// OK, I > 0 and k < S, and either more than PA_SEL_THREAD_MAX isoforms or a top score tied among more than 16
+// isoforms (where the reference's std::sort order decides).  Best isoform in the reference's order + per modified
+// site the set of tied best competitors (= alternative sites).  The thread kernel writes nothing for these PSMs, so
+// their status, n_iso and n_sites are written here too.
 __global__ void __launch_bounds__(256) k_select(PaCfg cfg, PaBatchDev b, PaSelArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5, wpb = blockDim.x >> 5;
+    const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     unsigned long long* s_sort = (unsigned long long*)smem_raw + (size_t)wib * PA_SORTCAP;
     __shared__ uint8_t s_pos_all[8][64];              // per warp: residue index of each site of the current PSM
     uint8_t* s_pos = s_pos_all[wib];
     int qn0 = 0, qn1 = 0, qn2 = 0, qn3 = 0;           // Ascore entries found per stream class (lane-uniform)
-    const int64_t gw = (int64_t)blockIdx.x * wpb + wib, nw = (int64_t)gridDim.x * wpb;
     const float INF = __int_as_float(0x7f800000);
 
-    // Warps take runs of `grab` consecutive PSMs from a global cursor (the cost per PSM grows with
-    // its isoform count, so a static split leaves warps idle).
-    (void)gw; (void)nw;
-    unsigned long long pend = 0;
-    const int grab = a.grab < 0 ? -a.grab : a.grab;
-    if (lane == 0) pend = atomicAdd(a.next_psm, (unsigned long long)grab);
-    int64_t run0 = (int64_t)__shfl_sync(PA_FULL, pend, 0);
-    const bool ahead = a.grab > 0;                    // see k_count_score
-    const int64_t n_visit = a.n_psm_dev ? (int64_t)*a.n_psm_dev : a.n_psm;
-    while (run0 < n_visit) {
-      if (ahead && lane == 0) pend = atomicAdd(a.next_psm, (unsigned long long)grab);
-      const int64_t pi_end = run0 + grab < n_visit ? run0 + grab : n_visit;
-      for (int64_t pi = run0; pi < pi_end; pi++) {
-        const int64_t p = a.order ? a.order[pi] : pi;
-        const int status = a.psm_status[p];
+    // Warps take one PSM at a time from a global cursor (the cost per PSM grows with its isoform count, so a
+    // static split leaves warps idle).
+    const int64_t n = *a.rest_count;
+    for (;;) {
+        unsigned long long pi = 0;
+        if (lane == 0) pi = atomicAdd(a.next_psm, 1ull);
+        pi = __shfl_sync(PA_FULL, pi, 0);
+        if ((int64_t)pi >= n) break;
+        const int64_t p = a.rest_list[pi];
         const int k = b.n_mod[p];
         const int64_t mo = a.mod_off[p];
         const int S = a.psm_S[p];
         const int64_t I = a.iso_off[p + 1] - a.iso_off[p];
         const int64_t ib = a.iso_off[p];
         if (lane == 0) {
-            if (a.psm_status_out) a.psm_status_out[p] = status;
+            if (a.psm_status_out) a.psm_status_out[p] = a.psm_status[p];
             if (a.n_iso) a.n_iso[p] = I;
             if (a.n_sites) a.n_sites[p] = S;
-        }
-        if (status != PA_PSM_OK || I == 0 || k >= S) {
-            // no isoform: best_sequence "" / best_score -1 (cpp/Ascore.cpp:273-295); k >= #sites is
-            // "unambiguous" (cpp/Ascore.cpp:38-51: ascores inf, no alternatives); errors report NaN
-            const bool ok = status == PA_PSM_OK;
-            const float fill = ok ? INF : __int_as_float(0x7fc00000);
-            if (lane == 0) {
-                uint64_t sig = 0; float sc = ok ? -1.f : fill;
-                if (ok && I > 0) { sig = (S >= 64) ? ~0ull : ((1ull << S) - 1ull); sc = a.iso.w[ib]; }
-                if (a.best_sig) a.best_sig[p] = sig;
-                if (a.best_score) a.best_score[p] = sc;
-                a.best_idx[p] = (ok && I > 0) ? 0u : 0xffffffffu;
-            }
-            for (int j = lane; j < k; j += 32) {
-                if (a.ascores) a.ascores[mo + j] = fill;
-                if (a.alt_sites) a.alt_sites[mo + j] = 0;
-                a.mod_psm[mo + j - a.mod_lo] = -1;
-                a.work_key[mo + j - a.mod_lo] = (uint16_t)PA_WORK_NONE;
-                a.work_val[mo + j - a.mod_lo] = (int32_t)(mo + j - a.mod_lo);
-            }
-            continue;
         }
         // residue positions of the sites: the distance between two sites is what an Ascore merge costs
         const int pep0 = b.pep_off[p], L = b.pep_off[p + 1] - pep0;
@@ -1676,34 +1603,26 @@ __global__ void __launch_bounds__(256) k_select(PaCfg cfg, PaBatchDev b, PaSelAr
         }
         uint32_t best = first_tie;
         if (ties > 1) {
-            const int64_t po = a.perm_off[S * 64 + k];
-            const uint32_t* perm = a.perm_pool + po;
-            if (I <= 16) {
-                // std::sort on <= 16 elements is a stable insertion sort: the first maximal element
-                // in hash-iteration order stays in front
-                uint32_t id = lane < I ? perm[lane] : 0u;
-                bool is = lane < I && a.iso.w[ib + id] == wmax;
-                unsigned bal = __ballot_sync(PA_FULL, is);
-                best = __shfl_sync(PA_FULL, id, __ffs(bal) - 1);
-            } else {
-                unsigned long long* arr = (I <= PA_SORTCAP) ? s_sort : a.g_sort + ib;
-                __syncwarp();
-                for (int64_t q = lane; q < I; q += 32) {
-                    uint32_t id = perm[q];
-                    arr[q] = ((unsigned long long)(uint32_t)__float_as_int(a.iso.w[ib + id]) << 32) | id;
-                }
-                __syncwarp();
-                if (I <= PA_SORTCAP) {       // shared-memory arena: one lane replays the partitions
-                    if (lane == 0) best = pa_gcc_sort_front(arr, (long)I);
-                    best = __shfl_sync(PA_FULL, best, 0);
-                } else best = pa_gcc_sort_front_warp(arr, (long)I, a.g_lr + ib + 2 * p);
-                __syncwarp();
+            // a tie among more than 16 isoforms: replay std::sort's partitions over the hash-iteration order
+            const uint32_t* perm = a.perm_pool + a.perm_off[S * 64 + k];
+            unsigned long long* arr = (I <= PA_SORTCAP) ? s_sort : a.g_sort + ib;
+            __syncwarp();
+            for (int64_t q = lane; q < I; q += 32) {
+                uint32_t id = perm[q];
+                arr[q] = ((unsigned long long)(uint32_t)__float_as_int(a.iso.w[ib + id]) << 32) | id;
             }
+            __syncwarp();
+            if (I <= PA_SORTCAP) {           // shared-memory arena: one lane replays the partitions
+                if (lane == 0) best = pa_gcc_sort_front(arr, (long)I);
+                best = __shfl_sync(PA_FULL, best, 0);
+            } else best = pa_gcc_sort_front_warp(arr, (long)I, a.g_lr + ib + 2 * p);
+            __syncwarp();
         }
         const uint64_t best_bits = pa_unrank(cfg.binom, S, k, best);
+        const float wb = a.iso.w[ib + best];
         if (lane == 0) {
             if (a.best_sig) a.best_sig[p] = best_bits;
-            if (a.best_score) a.best_score[p] = a.iso.w[ib + best];
+            if (a.best_score) a.best_score[p] = wb;
             a.best_idx[p] = best;
         }
         // ---- tied best competitors per modified site (cpp/Ascore.cpp:212-254) ---------------
@@ -1727,46 +1646,24 @@ __global__ void __launch_bounds__(256) k_select(PaCfg cfg, PaBatchDev b, PaSelAr
                 if (a.alt_sites) a.alt_sites[mo + j] = tie;
                 a.tie[mo + j - a.mod_lo] = tie;
                 a.mod_psm[mo + j - a.mod_lo] = (int32_t)p;
-                if (a.ascores) {
-                    // every tied competitor has exactly the score m; within 1e-6 of the best score the
-                    // ambiguity is 0 without looking at any ion (cpp/Ascore.cpp:161-163), so the Ascore
-                    // (the minimum over the tie set) is 0
-                    const float wb = a.iso.w[ib + best];
-                    if ((double)fabsf(__fsub_rn(wb, m)) < 1e-6) a.ascores[mo + j] = 0.f;
-                }
             }
             if (a.ascores) {
-                // everything else goes to k_ascore.  Every entry gets a sort key -- stream class (so that
-                // the lanes of a k_ascore warp run the same code), then the estimated number of merge trips,
-                // longest first: per tied competitor one trip per residue plus three per residue between the
-                // two sites, times the charges -- and the host sorts the entries by it, so that the lanes of a
-                // warp also finish together.
-                const float wb = a.iso.w[ib + best];
+                const bool zero = pa_asc_zero(wb, m);
                 uint32_t key = PA_WORK_NONE;
-                if (!((double)fabsf(__fsub_rn(wb, m)) < 1e-6)) {
-                    const int Z = b.max_charge[p];
-                    const int cls = cfg.has_nl ? 3 : (Z == 1 ? 0 : (Z == 2 ? 1 : (Z <= 4 ? 2 : 3)));
+                if (!zero) {
+                    int cls;
+                    key = pa_work_key(cfg, b.max_charge[p], L, site, tie, [&](int s) { return (int)s_pos[s]; }, cls);
                     int& qn = cls == 0 ? qn0 : (cls == 1 ? qn1 : (cls == 2 ? qn2 : qn3));
                     qn++;
-                    int work = 0;
-                    const int ps = s_pos[site < 64 ? site : 63];
-                    for (uint64_t tt = tie; tt; tt &= tt - 1) {
-                        const int pu = s_pos[__ffsll((long long)tt) - 1];
-                        work += (L - 1) + 3 * (pu > ps ? pu - ps : ps - pu);
-                    }
-                    work *= Z < 8 ? Z : 8;
-                    key = ((uint32_t)cls << 10) | (((uint32_t)(1023 - (work > 1023 ? 1023 : work)) >> PA_WORK_SHIFT) << PA_WORK_SHIFT);
                 }
                 if (lane == 0) {
+                    if (zero) a.ascores[mo + j] = 0.f;
                     a.work_key[mo + j - a.mod_lo] = (uint16_t)key;
                     a.work_val[mo + j - a.mod_lo] = (int32_t)(mo + j - a.mod_lo);
                 }
             }
         }
         __syncwarp();
-      }
-      if (!ahead && lane == 0) pend = atomicAdd(a.next_psm, (unsigned long long)grab);
-      run0 = (int64_t)__shfl_sync(PA_FULL, pend, 0);
     }
     if (a.ascores && lane == 0) {
         if (qn0) atomicAdd(a.work_count + 0, qn0);
@@ -1798,7 +1695,7 @@ struct PaAscArgs {
     const int32_t* psm_S;
     PaIso iso;
     float* ascores;              // absolute-indexed output (may be null)
-    const int32_t* work_sorted;  // mod entries sorted by k_select's key: class 0 first, longest merges first
+    const int32_t* work_sorted;  // mod entries sorted by K3a's key: class 0 first, longest merges first
     const int* work_count;       // [4] entries per stream class
     int32_t* generic_list;       // entries that need the generic kernel
     int* generic_count;

@@ -1258,20 +1258,16 @@ static int chunk_back(pa_scorer* s, int si, const pa_results* out, bool out_dev,
         sa.tie = sl.tie.as<unsigned long long>();
         sa.work_key = sl.work_key.as<uint16_t>(); sa.work_val = sl.work_val.as<int32_t>();
         sa.work_count = sl.generic_count.as<int>() + 1;
-        sa.order = nullptr;                      // PSMs in input order: the Ascore entries are sorted by key below
         sa.next_psm = sl.sched.as<unsigned long long>() + 1;
         // thread per PSM for the common shapes; what it declines (generic_count[5] PSMs in rest_list) goes to
         // the warp-per-PSM kernel, whose visit count is therefore only known on the device
         CK(sl.rest_list.ensure((size_t)std::max<int64_t>(np, 1) * 4));
         sa.rest_list = sl.rest_list.as<int32_t>(); sa.rest_count = sl.generic_count.as<int>() + 5;
-        sa.n_psm_dev = nullptr; sa.grab = 1;
         k_select_thread<<<(unsigned)((np + 127) / 128), 128, 0, st>>>(s->cfg, cs.b, sa);
         CK(cudaGetLastError());
         const int wpb = 8;
         const size_t sel_smem = wpb * PA_SORTCAP * sizeof(unsigned long long);
         int blocks = (int)std::min<int64_t>((np + wpb - 1) / wpb, (int64_t)s->sm_count * resident_blocks(k_select, wpb * 32, sel_smem));
-        sa.order = sl.rest_list.as<int32_t>(); sa.n_psm_dev = sl.generic_count.as<int>() + 5;
-        sa.grab = -1;                            // one PSM per visit, no reservation: the rest list is short
         k_select<<<blocks, wpb * 32, sel_smem, st>>>(s->cfg, cs.b, sa);
         CK(cudaGetLastError());
         s->ctr.kernel_launches += 2; s->ctr.launches_select += 2;
@@ -1285,7 +1281,7 @@ static int chunk_back(pa_scorer* s, int si, const pa_results* out, bool out_dev,
         aa.iso = iso; aa.ascores = cs.o_asc; aa.generic_list = sl.generic_list.as<int32_t>();
         aa.generic_count = sl.generic_count.as<int>();
         aa.work_sorted = sl.work_sorted.as<int32_t>(); aa.work_count = sl.generic_count.as<int>() + 1;
-        // Ascore entries by stream class, longest merges first (keys written by k_select)
+        // Ascore entries by stream class, longest merges first (keys written by K3a, pa_work_key)
         size_t tw = 0;
         CK(cub::DeviceRadixSort::SortPairs(nullptr, tw, sl.work_key.as<uint16_t>(), sl.work_key2.as<uint16_t>(),
                                            sl.work_val.as<int32_t>(), sl.work_sorted.as<int32_t>(), (int)nm, 0, PA_WORK_BITS, st));
