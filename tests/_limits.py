@@ -297,3 +297,158 @@ def fragments_per_isoform(pep, state, types, Z, nl):
         total += n * Z
     return total
 
+
+
+# ---- deep peak depths (n_top 11 .. 64).  The groups above hold at most 10 peaks per bin (even_bins) or a handful per
+# 100-Th bin (spectrum()), so at n_top > 10 they would give no rank >= 10 and K2d would only ever add zeros.  The helpers
+# below give a built group's spectra denser bins from their own generator; the groups above keep their draws.
+def at_n_top(g, n_top):
+    """group `g` scored at peak depth `n_top` (the scorer set-up with n_top overridden, the same PSMs)"""
+    out = Group(g.name, dict(g.meta["scorer"], n_top=n_top), g.meta["neutral_losses"])
+    out.psms, out.info = list(g.psms), list(g.info)
+    return out
+
+
+def densify_spectrum(rng, mz, inten, bin_size, n_top, cap=None, stronger=True):
+    """(mz, inten) with peaks added to the bins that hold peaks (bins as the reference counts them: from the spectrum's
+    lowest m/z rounded down to a multiple of 100), from the lowest bin up, until each holds 11 .. n_top peaks.  The added
+    peaks are stronger than every peak already in their bin, so those (the ions among them) move down by the number
+    added -- ten or more where n_top leaves room -- to ranks >= 10.  Half the bins stay within five peaks of that, so
+    that ions sit at depths near 10 as well as further down.  `cap`: stop before the retained peaks of the
+    spectrum pass it.  stronger=False: the added peaks are weaker than those in their bin instead (the ions keep their
+    ranks, the added peaks take 10 .. n_top-1).  Spectra of fewer than three peaks stay as they are."""
+    if mz.size < 3:
+        return mz, inten
+    bs = float(np.float32(bin_size))
+    lo, hi = np.floor(mz.min() / 100.) * 100., np.ceil(mz.max() / 100.) * 100.
+    nb = int(np.ceil(np.float32((hi - lo) / bs)))
+    b = np.minimum(np.floor((mz - lo) / bs).astype(np.int64), nb - 1)
+    count = np.bincount(b, minlength=nb)
+    retained = int(np.minimum(count, n_top).sum())
+    add_mz, add_it = [mz], [inten]
+    for q in np.flatnonzero((count > 0) & (count < n_top)):
+        c = int(count[q])
+        low = max(11, c + 10 if c + 10 <= n_top else c + 1)
+        want = int(rng.integers(low, (n_top if rng.random() < 0.5 else min(n_top, low + 5)) + 1))
+        if cap is not None and retained + want - c > cap:
+            break
+        a0 = lo + q * bs + 0.02 * bs
+        a1 = min(lo + (q + 1) * bs, hi) - 0.02 * bs
+        add_mz.append(rng.uniform(a0, a1, want - c))
+        f = np.exp(rng.uniform(0.01, 2., want - c))
+        add_it.append(inten[b == q].max() * f if stronger else inten[b == q].min() / f)
+        retained += want - c
+    mz, inten = np.concatenate(add_mz), np.concatenate(add_it)
+    assert np.unique(inten).size == inten.size                  # distinct intensities (ties are implementation-defined)
+    o = np.argsort(mz, kind="stable")
+    return np.ascontiguousarray(mz[o]), np.ascontiguousarray(inten[o])
+
+
+def densify(g, n_top, seed, cap=None, stronger=True):
+    """group `g` at peak depth `n_top` on densified spectra (densify_spectrum, generator seeded by (seed, n_top))"""
+    rng = np.random.default_rng([seed, n_top])
+    out = at_n_top(g, n_top)
+    bs = g.meta["scorer"]["bin_size"]
+    out.psms = []
+    for p in g.psms:
+        mz, it = densify_spectrum(rng, p["mz"], p["inten"], bs, n_top, cap, stronger)
+        out.psms.append(dict(p, mz=mz, inten=it))
+    return out
+
+
+def densify_batch(batch, bin_size, n_top, seed):
+    """densify_spectrum over every spectrum of a CSR batch"""
+    rng = np.random.default_rng([seed, n_top])
+    off = batch["spec_off"]
+    parts = [densify_spectrum(rng, batch["mz"][off[q]:off[q + 1]], batch["inten"][off[q]:off[q + 1]], bin_size, n_top)
+             for q in range(off.size - 1)]
+    out = dict(batch)
+    out["mz"] = np.ascontiguousarray(np.concatenate([m for m, _ in parts]))
+    out["inten"] = np.ascontiguousarray(np.concatenate([i for _, i in parts]))
+    out["spec_off"] = np.concatenate([[0], np.cumsum([m.size for m, _ in parts])]).astype(np.int64)
+    return out
+
+
+def add_one_residue_deep(g, rng, letter="S", Z=2):
+    """a one-residue PSM (k = 1) whose fragments (every loss variant of the group) sit at ranks 12 .. 13 of their bins:
+    twelve stronger peaks away from them fill each bin.  Only K2d's one-step walk (L = 1) counts these matches."""
+    m = _MASS[letter] + 79.966331
+    losses = [0.] + [mass for grp, mass in g.meta["neutral_losses"] if letter.lower() in grp]
+    ion = []
+    for t in g.meta["scorer"]["fragment_types"]:          # as ions(): residue sum + the ion type's shift
+        for nl in losses:
+            for z in range(1, Z + 1):
+                ion.append((m + _ION_SHIFT[t] - nl + z * 1.007825) / z)
+    ion = np.unique(np.round(np.array(ion), 4))
+    bs = float(np.float32(g.meta["scorer"]["bin_size"]))
+    mz, it = [ion + rng.normal(0., 0.05, ion.size)], [np.exp(3. + rng.random(ion.size))]
+    for q in np.unique(np.floor(ion / bs)):
+        a0, a1 = q * bs, (q + 1) * bs
+        cand = rng.uniform(a0 + 0.02 * bs, a1 - 0.02 * bs, 200)
+        cand = cand[np.min(np.abs(cand[:, None] - ion[None, :]), axis=1) > 3.][:12]
+        assert cand.size == 12
+        mz.append(cand)
+        it.append(np.exp(8. + rng.random(12)))
+    mz, it = np.concatenate(mz), np.concatenate(it)
+    o = np.argsort(mz)
+    g.add(letter, 1, Z, np.ascontiguousarray(mz[o]), np.ascontiguousarray(it[o]), one_residue_deep=True)
+
+
+def deep_peaks_group(n_top):
+    """254 / 255 / 256 retained peaks (straddling PA_RCAP) from 18 bins of 100 Th holding 14 or 15 peaks each, i.e. more
+    than ten retained peaks per bin, at peak depth n_top (>= 15)"""
+    rng = np.random.default_rng(2550 + n_top)
+    g = Group("peaks_deep", dict(PHOS, n_top=n_top))
+    n_bins = 18
+    for t in (254, 255, 256):
+        sites = [3, 7, 11, 15, 19, 22]
+        pep = peptide(rng, 25, sites)
+        per_bin = np.full(n_bins, t // n_bins)
+        per_bin[:t % n_bins] += 1
+        assert 10 < per_bin.min() and per_bin.max() <= n_top
+        mz, it = spectrum(rng, ions(pep, [7, 15], "by", 2), 100., 100., 100. + 100. * n_bins, per_bin=per_bin)
+        g.add(pep, 2, 2, mz, it, retained=t, n_bins=n_bins)
+    return g
+
+
+# the deep cases of tests/test_gpu_deep_limits.py (GPU against the oracle) and tests/test_oracle_deep_limits.py (their
+# reach, on the oracle alone)
+DEEP_SEED = 1164
+
+
+def deep_group(name, n_top):
+    """the shape group `name` at peak depth n_top with bins of 11 .. n_top peaks.  The length groups stay within PA_RCAP
+    retained peaks (their proof needs staged peaks), sites keeps its ions at the top ranks (its proof needs the true
+    sites past index 31 to stay the best isoform's), and length_nl gets a one-residue PSM matched at deep ranks."""
+    if name == "peaks_deep":
+        return deep_peaks_group(n_top)
+    build = {"length": length_group, "length_nl": lambda: length_group([("st", 97.9769)]), "sites": sites_group,
+             "charge_nl": lambda: charge_group([("ST", 18.01528)]), "fragments": frag_group,
+             "fragments_nl": frag_group_nl, "isoforms": isoform_group, "dense": dense_group}[name]
+    g = densify(build(), n_top, DEEP_SEED, cap=RCAP if name.startswith("length") else None, stronger=name != "sites")
+    if name == "length_nl":
+        add_one_residue_deep(g, np.random.default_rng([DEEP_SEED, n_top, 1]))
+    return g
+
+
+DEEP_SHAPES = [(n, t) for n in ("length", "length_nl", "sites", "charge_nl", "fragments", "fragments_nl", "isoforms",
+                                "dense") for t in (20, 64)] + [("peaks_deep", 20), ("peaks_deep", 40)]
+
+# the shape cases none of whose Ascores is taken at a depth >= 10 (every group but dense has one that is: in dense,
+# mz_error 1.5 over 10-Th bins, every 3-Th window holds peaks of rank < 10 and the score differences peak shallow)
+DEEP_SHALLOW_ASCORES = {("sites", 20), ("fragments_nl", 64), ("dense", 20), ("dense", 64)}
+
+# variant matrix at depth: every VARIANTS set-up at n_top 20, then the first set-up of each k_count_score
+# instantiation at 64
+DEEP_MATRIX = [(q, 20) for q in range(len(VARIANTS))] + \
+    [(q, 64) for q in sorted({k2_instantiation(*v): i for i, v in reversed(list(enumerate(VARIANTS)))}.values())]
+
+
+def deep_variant_case(q, n_top):
+    """(meta, batch) of variant q at n_top: 160 synthetic PSMs (7..20 residues, charges 1..2) on densified spectra"""
+    from pyascore_b200 import synth
+    ftypes, err, nl = VARIANTS[q]
+    w = dict(synth.WORKLOADS["lowres_phospho"], L=(7, 20), neutral_losses=nl,
+             scorer=dict(PHOS, fragment_types=ftypes, mz_error=err, n_top=n_top))
+    batch = synth.make_batch(w, 160, seed=2026, chunk_index=q)
+    return dict(scorer=w["scorer"], neutral_losses=nl), densify_batch(batch, 100., n_top, DEEP_SEED + q)
