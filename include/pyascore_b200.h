@@ -132,6 +132,20 @@ int pa_score_batch(pa_scorer* s, const pa_batch* in, const pa_results* out, uint
 int pa_score_range(pa_scorer* s, const pa_batch* in, const pa_results* out, int64_t psm_lo, int64_t psm_hi,
                    uint32_t flags);
 
+/* Several modification types in one call: scores each PSM p of `in` under the scorer s[psm_type[p]] -- its mod_group,
+ * mod_mass, neutral losses, mz_error and fragment_types.  The spectra are staged and binned ONCE for all types, so a run
+ * that localises, say, phospho on STY and acetyl on K pays one host-link transfer and one binning pass for its spectra;
+ * "the same spectrum scored for phospho and for acetyl" is two PSM rows of the batch.  Every scorer must be a scoring
+ * handle (not a binner) on the same device with the same bin_size and n_top (PA_ERR_ARG otherwise, also for n_types
+ * outside 1 .. 255); none may have an asynchronous call in flight (PA_ERR_STATE).  psm_type is on the same side (host /
+ * device) as the batch's arrays; NULL means every PSM is type 0.  A PSM whose type is >= n_types gets PA_PSM_BAD_INDEX.
+ * Results are written as by pa_score_batch: each PSM at its own position, ascores / alt_sites at mod_off; for the PSMs
+ * of type t they are bit-identical to pa_score_batch(s[t], ...) on a batch of the type-t rows alone.  PA_KEEP_ISOFORMS
+ * with n_types > 1 is PA_ERR_UNSUPPORTED.  pa_counters(s[0]) describes the call; pa_last_error(s[0]) has the text of
+ * a failure (pa_last_error(NULL) when s or s[0] is NULL). */
+int pa_score_typed(pa_scorer* const* s, int32_t n_types, const pa_batch* in, const uint8_t* psm_type,
+                   const pa_results* out, uint32_t flags);
+
 /* Asynchronous form of pa_score_range: returns once the work is handed to the scorer's own orchestration thread
  * (the path takes one host decision per chunk -- the plan totals size the isoform scratch -- so it cannot be a
  * pure stream enqueue).  `stream` (a cudaStream_t of the scorer's device, or NULL) is honoured as a dependency:

@@ -5,14 +5,17 @@
     parse identifications, sort by scan          (IdentificationParser.to_list)
     pack chunks of PSMs (hit_depth, mod split, charge rule)  ||  score previous chunk on the GPU
     format rows, write the TSV (same columns and number formatting)
+
+With --extra_mod, the spectra are parsed once and each batch holds the rows of every modification type, scored in
+one GPU call (score_typed); each type writes its own TSV.
 """
 import sys
 from datetime import datetime
 
 import numpy as np
 
-from .batch import MultiScorer, Scorer
-from .config import args_from_file, build_parser, validate_args
+from .batch import MultiScorer, Scorer, score_typed
+from .config import args_from_file, build_parser, parse_extra_mod, validate_args
 from .parsing import (COMMON_MODS, IdentificationParser, MassCorrector, SpectraParser, iter_batches, result_rows,
                       score_stream, write_tsv)
 
@@ -29,11 +32,14 @@ def static_mod_dict(args):
     return out
 
 
-def parse_identifications(args):
-    """reference: __main__.py:22-45 -> scan-sorted PSM records"""
+def parse_identifications(args, residues=None, mod_mass=None):
+    """reference: __main__.py:22-45 -> scan-sorted PSM records, mass-corrected for the variable modification
+    (residues, mod_mass) -- default: --residues / --mod_mass"""
+    residues = args.residues if residues is None else residues
+    mod_mass = args.mod_mass if mod_mass is None else mod_mass
     static_mods = static_mod_dict(args)
     mods = COMMON_MODS.copy()
-    mods.update({aa: args.mod_mass for aa in args.residues})
+    mods.update({aa: mod_mass for aa in residues})
     mods.update(static_mods)
     parser = IdentificationParser(args.ident_file, args.ident_file_type, MassCorrector(mod_mass_dict=mods),
                                   static_mods=static_mods)
@@ -53,7 +59,64 @@ def build_scorer(args):
     return scorer
 
 
+def mod_types(args):
+    """the modification types of a run: type 0 = --residues / --mod_mass / the neutral-loss flags / out_file, then one
+    per --extra_mod"""
+    return [dict(residues=args.residues, mod_mass=args.mod_mass, out_file=args.out_file,
+                 neutral_loss_groups=args.neutral_loss_groups, neutral_loss_masses=args.neutral_loss_masses)] + \
+        [parse_extra_mod(text) for text in args.extra_mod]
+
+
+def run_typed(args, log=print):
+    """A run with --extra_mod: the spectra are parsed once and every batch is scored for all modification types in
+    one GPU call (score_typed); each type's rows go to its own TSV, the same file a run of that type alone writes."""
+    types = mod_types(args)
+    log("{} -- Ascore Started".format(_stamp()))
+    log("{} -- Reading spectra from: {}".format(_stamp(), args.spec_file))
+    spectra = SpectraParser(args.spec_file, args.spec_file_type).to_csr()
+    log("{} -- Reading identifications from: {}".format(_stamp(), args.ident_file))
+    psms = [parse_identifications(args, t["residues"], t["mod_mass"]) for t in types]
+    log("{} -- Anlyzing PSMs".format(_stamp()))
+    scorers = []
+    rows = [[] for _ in types]
+    n_psm = [0] * len(types)
+    saved = []
+    try:
+        for t in types:
+            scorers.append(Scorer(100., 10, t["residues"], t["mod_mass"], args.mz_error, args.fragment_types,
+                                  device=args.device))
+            if t["neutral_loss_groups"] and t["neutral_loss_masses"]:
+                for g, m in zip(t["neutral_loss_groups"].split(","), t["neutral_loss_masses"].split(",")):
+                    scorers[-1].add_neutral_loss(g, float(m))
+        batches = iter_batches(spectra, psms, chunk_psms=args.chunk_psms,
+                               types=[(t["residues"], t["mod_mass"]) for t in types],
+                               mod_correction_tol=args.mod_correction_tol, zero_based=args.zero_based,
+                               max_fragment_charge=args.max_fragment_charge, hit_depth=args.hit_depth)
+        for scans, batch, res in score_stream(lambda b: score_typed(scorers, b, b["psm_type"]), batches):
+            for t, sc in enumerate(scorers):
+                sel = np.flatnonzero(batch["psm_type"] == t)
+                rows[t].extend(result_rows(sc, scans, batch, res, rows_of=sel))
+                n_psm[t] += int(sel.size)
+            if args.match_save:
+                saved.append((scans, batch))
+    finally:
+        for sc in scorers:
+            sc.close()
+    if args.match_save and saved:
+        scans, batch = saved[-1]
+        np.savez("dump_batch.npz", scans=scans, **{k: v for k, v in batch.items() if v is not None})
+    for t, typ in enumerate(types):
+        if len(rows[t]) != n_psm[t]:
+            log("{} -- {} of {} PSMs of {} could not be scored (see the warnings) and have no row in the output".format(
+                _stamp(), n_psm[t] - len(rows[t]), n_psm[t], typ["out_file"]))
+        write_tsv(typ["out_file"], rows[t])
+    log("{} -- Ascore Completed".format(_stamp()))
+    return rows
+
+
 def run(args, log=print):
+    if getattr(args, "extra_mod", None):
+        return run_typed(args, log)
     log("{} -- Ascore Started".format(_stamp()))
     log("{} -- Reading spectra from: {}".format(_stamp(), args.spec_file))
     spectra = SpectraParser(args.spec_file, args.spec_file_type).to_csr()

@@ -48,7 +48,7 @@ EXPORTS = ["pa_create", "pa_add_neutral_loss", "pa_destroy", "pa_last_error", "p
            "pa_fetch_pep_scores", "pa_calculate_ambiguity", "pa_format_sequence", "pa_site_positions",
            "pa_bin_spectra", "pa_tail_table", "pa_counters", "pa_alloc_pinned", "pa_free_pinned", "pa_version",
            "pa_create_binner", "pa_bin_spectra_ex", "pa_fragment_table", "pa_site_determining_ions", "pa_log_math",
-           "pa_power_set_sums", "pa_score_range", "pa_score_batch_async", "pa_wait", "pa_shard_ranges", "pa_shard_ranges_for", "pa_alloc_pinned_ex", "pa_narrow_mz"]
+           "pa_power_set_sums", "pa_score_range", "pa_score_batch_async", "pa_wait", "pa_shard_ranges", "pa_shard_ranges_for", "pa_alloc_pinned_ex", "pa_narrow_mz", "pa_score_typed"]
 
 _lib = None
 
@@ -73,6 +73,8 @@ def load():
     L.pa_last_error.argtypes = [vp]
     L.pa_score_batch.restype = C.c_int
     L.pa_score_batch.argtypes = [vp, C.POINTER(PaBatch), C.POINTER(PaResults), C.c_uint32]
+    L.pa_score_typed.restype = C.c_int
+    L.pa_score_typed.argtypes = [C.POINTER(vp), C.c_int32, C.POINTER(PaBatch), vp, C.POINTER(PaResults), C.c_uint32]
     L.pa_score_range.restype = C.c_int
     L.pa_score_range.argtypes = [vp, C.POINTER(PaBatch), C.POINTER(PaResults), C.c_int64, C.c_int64, C.c_uint32]
     L.pa_score_batch_async.restype = C.c_int

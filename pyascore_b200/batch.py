@@ -373,6 +373,39 @@ class MultiScorer:
         return self.scorers[0].site_positions(pep)
 
 
+def score_typed(scorers, batch, psm_type, out=None, want=_WANT_ALL):
+    """Score PSM i of `batch` under scorers[psm_type[i]] (pa_score_typed): several modification types in one call, with
+    the spectra copied and binned once for all of them.  `scorers`: `Scorer` objects on one device with the same
+    bin_size and n_top; `psm_type`: uint8 per PSM on the side of the batch's arrays (numpy / CUDA tensor), or None
+    (every PSM is type 0).  Returns the dict of `Scorer.score_batch`; the rows of type t equal scorers[t].score_batch on
+    those rows alone, and `format_results` takes scorers[psm_type[i]] for row i."""
+    scorers = list(scorers)
+    if not scorers:
+        raise ValueError("score_typed needs at least one scorer")
+    s0 = scorers[0]
+    pb, pr, out = s0._prepare(batch, out, want)
+    if psm_type is not None:
+        n_psm = int(batch["n_mod"].shape[0])
+        if tuple(psm_type.shape) != (n_psm,):
+            raise ValueError("psm_type must hold one entry per PSM (%d), not %s" % (n_psm, tuple(psm_type.shape)))
+        if isinstance(psm_type, np.ndarray):
+            if psm_type.dtype != np.uint8 or not psm_type.flags.c_contiguous:
+                raise ValueError("psm_type must be a C-contiguous uint8 array")
+            if not isinstance(batch["mz"], np.ndarray):
+                raise ValueError("psm_type must live where the batch's arrays live (a CUDA tensor here)")
+        else:
+            import torch
+            if psm_type.dtype != torch.uint8 or not psm_type.is_contiguous():
+                raise ValueError("psm_type must be a contiguous uint8 tensor")
+            if isinstance(batch["mz"], np.ndarray):
+                raise ValueError("psm_type must live where the batch's arrays live (a host array here)")
+    handles = (C.c_void_p * len(scorers))(*[sc.h for sc in scorers])
+    rc = s0.L.pa_score_typed(handles, len(scorers), C.byref(pb), _ptr(psm_type), C.byref(pr), 0)
+    if rc != 0:
+        s0._raise(rc)
+    return out
+
+
 def format_results(scorer, batch, res, i):
     """Reference-style view of PSM i: (best_sequence, best_score, ascores, alt_sites)."""
     pep = bytes(batch["pep"][batch["pep_off"][i]:batch["pep_off"][i + 1]])

@@ -1,6 +1,6 @@
 """Command-line options of `python -m pyascore_b200`: the reference's flag set
 (pyascore/config.py:19-93: same names, types and defaults, so parameter files and scripts carry
-over) plus `--device` / `--chunk_psms` for the GPU pipeline."""
+over) plus `--device` / `--chunk_psms` for the GPU pipeline and `--extra_mod` for more modification types per run."""
 import argparse
 import re
 
@@ -52,19 +52,59 @@ def build_parser():
     p.add_argument("--devices", type=str, default="", help="Comma separated CUDA device ordinals: every batch is "
                    "sharded over these GPUs (overrides --device).")
     p.add_argument("--chunk_psms", type=int, default=65536, help="PSMs packed per GPU batch.")
+    p.add_argument("--extra_mod", action="append", default=None, metavar="RESIDUES:MASS:OUT_FILE[:NL_GROUPS:NL_MASSES]",
+                   help="One more modification type to localise in the same run, written to its own OUT_FILE (the "
+                        "spectra are read, copied and binned once for all types). NL_GROUPS / NL_MASSES are comma "
+                        "separated as in --neutral_loss_groups / --neutral_loss_masses. Repeatable; in a parameter "
+                        "file, one 'extra_mod = ...' line per type. Not combinable with --devices.")
     p.add_argument("spec_file", type=str, help="MS spectra file.")
     p.add_argument("ident_file", type=str, help="Results of the database search.")
     p.add_argument("out_file", type=str, help="Destination of the tab-separated results.")
     return p
 
 
-def validate_args(args):
-    """reference: __main__.py:48-65"""
+def _validate_residues(residues):
+    """reference: __main__.py:49-53"""
     allowed_residues = "ncACDEFGHIKLMNOPQRSTUVWY"
-    for aa in args.residues:
+    for aa in residues:
         if aa not in allowed_residues:
             raise ValueError("The residue inputed, {}, is not allowed."
                              " Must be one of: {}".format(aa, allowed_residues))
+
+
+def parse_extra_mod(text):
+    """'RESIDUES:MASS:OUT_FILE[:NL_GROUPS:NL_MASSES]' -> dict(residues, mod_mass, out_file, neutral_loss_groups,
+    neutral_loss_masses)"""
+    parts = text.split(":")
+    if len(parts) not in (3, 5) or not parts[0] or not parts[2]:
+        raise ValueError("--extra_mod {!r}: expected RESIDUES:MASS:OUT_FILE or "
+                         "RESIDUES:MASS:OUT_FILE:NL_GROUPS:NL_MASSES".format(text))
+    try:
+        mass = float(parts[1])
+    except ValueError:
+        raise ValueError("--extra_mod {!r}: the mass {!r} is not a number".format(text, parts[1])) from None
+    groups, masses = (parts[3], parts[4]) if len(parts) == 5 else ("", "")
+    if len(groups.split(",")) != len(masses.split(",")):
+        raise ValueError("--extra_mod {!r}: {} neutral-loss groups but {} masses".format(
+            text, len(groups.split(",")), len(masses.split(","))))
+    for m in masses.split(",") if masses else ():
+        try:
+            float(m)
+        except ValueError:
+            raise ValueError("--extra_mod {!r}: the neutral-loss mass {!r} is not a number".format(text, m)) from None
+    return dict(residues=parts[0], mod_mass=mass, out_file=parts[2], neutral_loss_groups=groups,
+                neutral_loss_masses=masses)
+
+
+def validate_args(args):
+    """reference: __main__.py:48-65, plus the --extra_mod types"""
+    _validate_residues(args.residues)
+    extra = getattr(args, "extra_mod", None) or []
+    for text in extra:
+        _validate_residues(parse_extra_mod(text)["residues"])
+    if extra and getattr(args, "devices", ""):
+        raise ValueError("--extra_mod cannot be combined with --devices: a run with several modification types "
+                         "scores on one GPU (choose it with --device)")
     allowed_fragments = "cbyzZ"
     for frag in args.fragment_types:
         if frag not in allowed_fragments:

@@ -491,7 +491,14 @@ struct PaPlanOut {
     int* max_len;            // longest scored peptide of the chunk
 };
 
-__global__ void __launch_bounds__(256) k_plan(PaCfg cfg, PaBatchDev b, int64_t n_psm, PaPlanOut o) {
+// Status k_plan gives a PSM of a typed batch (pa_score_typed) that belongs to another type than the pass's: no
+// isoforms, no units, and k_select_thread<true> writes none of its results.  It never reaches the caller.
+#define PA_PSM_OTHER_TYPE 0x100
+
+// psm_type (typed batches, chunk-relative; null: every PSM is of the pass's type): PSMs of another type get
+// PA_PSM_OTHER_TYPE; the pass of type 0 reports a type >= n_types as PA_PSM_BAD_INDEX.
+__global__ void __launch_bounds__(256) k_plan(PaCfg cfg, PaBatchDev b, int64_t n_psm, PaPlanOut o,
+                                              const uint8_t* psm_type, int type, int n_types) {
     // chunk-wide maxima and the (S,k) combinations seen are collected per block in shared memory and
     // flushed once: a global atomic per PSM and field would queue up on four addresses
     __shared__ unsigned long long s_combo[64];
@@ -506,7 +513,9 @@ __global__ void __launch_bounds__(256) k_plan(PaCfg cfg, PaBatchDev b, int64_t n
         const int k = b.n_mod[p], Z = b.max_charge[p];
         const int sp = b.psm_spec[p];
         int status = PA_PSM_OK, S = 0;
-        if (sp < 0 || sp >= b.n_spec || k < 0 || Z < 1 || L < 1) status = PA_PSM_BAD_INDEX;  // Z == 0 crashes the reference
+        const int t = psm_type != nullptr ? (int)psm_type[p] : type;
+        if (t != type) status = (type == 0 && t >= n_types) ? PA_PSM_BAD_INDEX : PA_PSM_OTHER_TYPE;
+        else if (sp < 0 || sp >= b.n_spec || k < 0 || Z < 1 || L < 1) status = PA_PSM_BAD_INDEX;  // Z == 0 crashes the reference
         else if (L > PA_MAX_PEPTIDE) status = PA_PSM_TOO_LONG;
         else {
             for (int i = 0; i < L; i++) {
@@ -1420,8 +1429,12 @@ __device__ __forceinline__ uint32_t pa_work_key(const PaCfg& cfg, int Z, int L, 
 // the same steps serially (best isoform, per modified site the tied best competitors, Ascore-0 shortcut,
 // sort key of every Ascore entry).  PSMs whose best score is tied among more than 16 isoforms (the
 // reference's std::sort order decides, which takes the warp kernel's sort replay) or that have more than
-// PA_SEL_THREAD_MAX isoforms are left, untouched, to k_select through rest_list.
+// PA_SEL_THREAD_MAX isoforms are left, untouched, to k_select through rest_list.  TYPED (a pass of a typed batch):
+// a PSM of another type (PA_PSM_OTHER_TYPE) gets only the scratch entries that keep its Ascore entries out of K3b /
+// K3c, and none of the results, which belong to its own type's pass.  (k_select needs no gate: such a PSM is never
+// declined to it.)
 #define PA_SEL_THREAD_MAX 512
+template <bool TYPED>
 __global__ void __launch_bounds__(128) k_select_thread(PaCfg cfg, PaBatchDev b, PaSelArgs a) {
     __shared__ int s_cls[4];
     if (threadIdx.x < 4) s_cls[threadIdx.x] = 0;
@@ -1462,12 +1475,15 @@ __global__ void __launch_bounds__(128) k_select_thread(PaCfg cfg, PaBatchDev b, 
                 }
             }
         }
+        const bool own = !TYPED || status != PA_PSM_OTHER_TYPE;
         if (rest) {
             a.rest_list[atomicAdd(a.rest_count, 1)] = (int32_t)p;
         } else {
-            if (a.psm_status_out) a.psm_status_out[p] = status;
-            if (a.n_iso) a.n_iso[p] = I;
-            if (a.n_sites) a.n_sites[p] = S;
+            if (own) {
+                if (a.psm_status_out) a.psm_status_out[p] = status;
+                if (a.n_iso) a.n_iso[p] = I;
+                if (a.n_sites) a.n_sites[p] = S;
+            }
             if (none) {
                 // no isoform: best_sequence "" / best_score -1 (cpp/Ascore.cpp:273-295); k >= #sites is
                 // "unambiguous" (cpp/Ascore.cpp:38-51: ascores inf, no alternatives); errors report NaN
@@ -1475,12 +1491,16 @@ __global__ void __launch_bounds__(128) k_select_thread(PaCfg cfg, PaBatchDev b, 
                 const float fill = ok ? INF : __int_as_float(0x7fc00000);
                 uint64_t sig = 0; float sc = ok ? -1.f : fill;
                 if (ok && I > 0) { sig = (S >= 64) ? ~0ull : ((1ull << S) - 1ull); sc = a.iso.w[ib]; }
-                if (a.best_sig) a.best_sig[p] = sig;
-                if (a.best_score) a.best_score[p] = sc;
+                if (own) {
+                    if (a.best_sig) a.best_sig[p] = sig;
+                    if (a.best_score) a.best_score[p] = sc;
+                }
                 a.best_idx[p] = (ok && I > 0) ? 0u : 0xffffffffu;
                 for (int j = 0; j < k; j++) {
-                    if (a.ascores) a.ascores[mo + j] = fill;
-                    if (a.alt_sites) a.alt_sites[mo + j] = 0;
+                    if (own) {
+                        if (a.ascores) a.ascores[mo + j] = fill;
+                        if (a.alt_sites) a.alt_sites[mo + j] = 0;
+                    }
                     a.mod_psm[mo + j - a.mod_lo] = -1;
                     a.work_key[mo + j - a.mod_lo] = (uint16_t)PA_WORK_NONE;
                     a.work_val[mo + j - a.mod_lo] = (int32_t)(mo + j - a.mod_lo);

@@ -80,7 +80,7 @@ struct PlanTotals {          // device -> host after planning a chunk
 struct Slot {                // per-stream working set
     cudaStream_t st = nullptr;
     // staged inputs
-    DevBuf spec_off, mz, inten, inten32, psm_spec, pep_off, pep, n_mod, max_charge, aux_off, aux_pos, aux_mass, mod_off;
+    DevBuf spec_off, mz, inten, inten32, psm_spec, pep_off, pep, n_mod, max_charge, aux_off, aux_pos, aux_mass, mod_off, psm_type;
     // K1
     DevBuf rpk, rcount, ctab, chead, g_bin, g_tmp;
     // plan
@@ -877,13 +877,20 @@ __global__ void k_check_batch(const int32_t* psm_spec, const int32_t* pep_off, c
 
 struct ChunkRange { int64_t p0, p1, s0, s1; };
 
+struct PassEvents {               // one scoring pass of a chunk: one per type that has PSMs in it
+    cudaEvent_t e_plan0, e_plan1, e_cnt0, e_cnt1, e_sel1, e_asc1;
+    cudaEvent_t e_deep1 = nullptr;   // n_top > 10: end of K2d (which starts at e_cnt1)
+};
+
 struct ChunkState {              // what the back half of a chunk needs from the front half
     ChunkRange r;
     PaBatchDev b;
     int64_t mod_lo = 0, mod_hi = 0;
     const int64_t* mod_off_abs = nullptr;
-    cudaEvent_t e_bin0, e_bin1, e_plan1, e_cnt0, e_cnt1, e_sel1, e_asc1;
-    cudaEvent_t e_deep1 = nullptr;   // n_top > 10: end of K2d (which starts at e_cnt1)
+    const uint8_t* psm_type = nullptr;   // typed batches: chunk-relative view of the PSMs' types
+    std::vector<int> types;          // the types with PSMs in the chunk, in pass order (untyped: {0})
+    cudaEvent_t e_bin0, e_bin1;
+    std::vector<PassEvents> ev;      // [pass]
     uint64_t* o_sig; float* o_score; int64_t* o_niso; int32_t* o_nsites; float* o_asc; uint64_t* o_alt; int32_t* o_status;
     ChunkArray res[7];               // the result arrays (views: the o_* above)
     bool single_chunk = false;       // the call has one chunk
@@ -951,8 +958,12 @@ static int narrow_end(pa_scorer* s, NarrowStage& ns, const pa_batch* in) {
     return PA_OK;
 }
 
-static int chunk_front(pa_scorer* s, int si, const pa_batch* in, bool in_dev, const ChunkRange& r, int64_t mod_lo,
-                       int64_t mod_hi, int max_peaks, ChunkState& cs, const DevBounds* ends_dev, NarrowStage* nst = nullptr) {
+static int chunk_plan(pa_scorer* s, pa_scorer* ts, int si, ChunkState& cs, int pass, int n_types);
+
+// Staging of a chunk, K1 and the plan of the chunk's first pass.  psm_type: the typed batch's types (null: untyped).
+static int chunk_front(pa_scorer* s, pa_scorer* const* sc, int n_types, int si, const pa_batch* in, const uint8_t* psm_type,
+                       bool in_dev, const ChunkRange& r, int64_t mod_lo, int64_t mod_hi, int max_peaks, ChunkState& cs,
+                       const DevBounds* ends_dev, NarrowStage* nst = nullptr) {
     Slot& sl = s->slot[si];
     cudaStream_t st = sl.st;
     const int64_t np = r.p1 - r.p0, ns = r.s1 - r.s0;
@@ -984,6 +995,7 @@ static int chunk_front(pa_scorer* s, int si, const pa_batch* in, bool in_dev, co
         {in->aux_off ? in->aux_pos : nullptr, aux_lo, aux_hi - aux_lo, sl.aux_pos, b.aux_pos},
         {in->aux_off ? in->aux_mass : nullptr, aux_lo, aux_hi - aux_lo, sl.aux_mass, b.aux_mass},
         {in->mod_off, r.p0, np + 1, sl.mod_off, cs.mod_off_abs},
+        {psm_type, r.p0, psm_type ? np : 0, sl.psm_type, cs.psm_type},
     };
     const ChunkArray& mz_in = ins[1];
     // packed block bound: every array at full size, the absent ones too, and 16 bytes of alignment for each
@@ -1024,6 +1036,7 @@ static int chunk_front(pa_scorer* s, int si, const pa_batch* in, bool in_dev, co
     b.psm_spec += r.p0; b.pep_off += r.p0; b.n_mod += r.p0; b.max_charge += r.p0;
     if (b.aux_off) b.aux_off += r.p0;
     cs.mod_off_abs += r.p0;
+    if (cs.psm_type) cs.psm_type += r.p0;
     b.spec_base = 0; b.n_spec = r.s1;   // spectrum indices stay absolute (views are pre-offset)
 
     // K1 buffers, indexed by absolute peak / spectrum index
@@ -1049,7 +1062,7 @@ static int chunk_front(pa_scorer* s, int si, const pa_batch* in, bool in_dev, co
     size_t smem;
     bin_launch_shape(s->sm_count, max_peaks, ns, &cap, &wpb, &smem, &blocks);
     ba.cap = cap;
-    cs.e_bin0 = next_event(s); cs.e_bin1 = next_event(s); cs.e_plan1 = next_event(s);
+    cs.e_bin0 = next_event(s); cs.e_bin1 = next_event(s);
     CK(cudaEventRecord(cs.e_bin0, st));
     ba.list = nullptr; ba.list_n = nullptr;
     if (ns >= PA_ROWS_MIN_SPECTRA && s->bin_rows && s->n_top <= 31) {     // (a handful of spectra: one launch instead of two)
@@ -1077,8 +1090,20 @@ static int chunk_front(pa_scorer* s, int si, const pa_batch* in, bool in_dev, co
     CK(cudaEventRecord(cs.e_bin1, st));
     b.rpk = ba.rpk; b.rcount = sl.rcount.as<int32_t>() - r.s0;
     b.ctab = sl.ctab.as<uint8_t>() - (size_t)r.s0 * PA_NCELL; b.chead = sl.chead.as<float2>() - r.s0;
+    cs.ev.assign(cs.types.size(), PassEvents());
+    return chunk_plan(s, sc[cs.types[0]], si, cs, 0, n_types);
+}
 
-    // plan
+// Plan of pass `pass` of a chunk (the PSMs of type cs.types[pass], scored with ts's settings and tables), up to the
+// read-back of its totals.  s owns the slots and the counters.
+static int chunk_plan(pa_scorer* s, pa_scorer* ts, int si, ChunkState& cs, int pass, int n_types) {
+    Slot& sl = s->slot[si];
+    cudaStream_t st = sl.st;
+    const int64_t np = cs.r.p1 - cs.r.p0;
+    PassEvents& ev = cs.ev[pass];
+    ev.e_plan0 = cs.e_bin1;
+    if (pass > 0) { ev.e_plan0 = next_event(s); CK(cudaEventRecord(ev.e_plan0, st)); }
+    ev.e_plan1 = next_event(s);
     CK(sl.psm_S.ensure((size_t)(np + 1) * sizeof(int32_t)));
     CK(sl.psm_status.ensure((size_t)(np + 1) * sizeof(int32_t)));
     CK(sl.psm_I.ensure((size_t)(np + 1) * sizeof(int64_t)));
@@ -1095,7 +1120,7 @@ static int chunk_front(pa_scorer* s, int si, const pa_batch* in, bool in_dev, co
     PlanTotals* dt = sl.totals.as<PlanTotals>();
     po.combo_bits = dt->combo_bits; po.max_frag = &dt->max_frag; po.max_list = &dt->max_list; po.max_len = &dt->max_len;
     if (np > 0) {
-        k_plan<<<(unsigned)((np + 255) / 256), 256, 0, st>>>(s->cfg, b, np, po);
+        k_plan<<<(unsigned)((np + 255) / 256), 256, 0, st>>>(ts->cfg, cs.b, np, po, cs.psm_type, cs.types[pass], n_types);
         CK(cudaGetLastError());
         s->ctr.kernel_launches++;
     }
@@ -1111,108 +1136,17 @@ static int chunk_front(pa_scorer* s, int si, const pa_batch* in, bool in_dev, co
     CK(cudaMemcpyAsync(&dt->total_iso, sl.iso_off.as<int64_t>() + np, sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
     CK(cudaMemcpyAsync(&dt->total_units, sl.unit_off.as<int32_t>() + np, sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
     CK(cudaMemcpyAsync(sl.h_totals.p, dt, sizeof(PlanTotals), cudaMemcpyDeviceToHost, st));
-    CK(cudaEventRecord(cs.e_plan1, st));
+    CK(cudaEventRecord(ev.e_plan1, st));
     CK(cudaEventRecord(sl.ev_plan, st));
     return PA_OK;
 }
 
-static int chunk_back(pa_scorer* s, int si, const pa_results* out, bool out_dev, ChunkState& cs, bool keep) {
+// The result arrays of a chunk: device views that every pass of the chunk writes into, read back once after the last.
+static int stage_results(pa_scorer* s, int si, const pa_results* out, bool out_dev, ChunkState& cs) {
     Slot& sl = s->slot[si];
     cudaStream_t st = sl.st;
     const ChunkRange& r = cs.r;
     const int64_t np = r.p1 - r.p0;
-    CK(cudaEventSynchronize(sl.ev_plan));
-    PlanTotals T = *sl.h_totals.as<PlanTotals>();
-    const int64_t total_iso = T.total_iso;
-    const int n_units = T.total_units;
-    // tables that depend on what the chunk contains
-    int rc = ensure_table(s, std::max(T.max_frag, 1));
-    if (rc != PA_OK) return rc;
-    for (int S = 0; S < 64; S++)
-        for (int k = 0; k < 64; k++)
-            if ((T.combo_bits[S] >> k) & 1ull) { rc = ensure_perm(s, S, k); if (rc != PA_OK) return rc; }
-    rc = upload_perms(s);
-    if (rc != PA_OK) return rc;
-    // scratch
-    CK(sl.iso_lo.ensure((size_t)std::max<int64_t>(total_iso, 1) * 8));
-    CK(sl.iso_hi.ensure((size_t)std::max<int64_t>(total_iso, 1) * 8));
-    CK(sl.iso_n.ensure((size_t)std::max<int64_t>(total_iso, 1) * 4));
-    CK(sl.iso_w.ensure((size_t)std::max<int64_t>(total_iso, 1) * 4));
-    CK(sl.g_sort.ensure((size_t)std::max<int64_t>(total_iso, 1) * 8));
-    CK(sl.g_lr.ensure((size_t)(std::max<int64_t>(total_iso, 1) + 2 * np + 2) * 4));
-    CK(sl.unit_psm.ensure((size_t)std::max(n_units, 1) * 4));
-    PaIso iso;
-    iso.lo = sl.iso_lo.as<unsigned long long>(); iso.hi = sl.iso_hi.as<unsigned long long>();
-    iso.nfrag = sl.iso_n.as<uint32_t>(); iso.w = sl.iso_w.as<float>();
-    cs.e_cnt0 = next_event(s); cs.e_cnt1 = next_event(s); cs.e_sel1 = next_event(s);
-    CK(sl.sched.ensure(16));                          // work cursors of k_count_score [0] and k_select [1]
-    CK(cudaMemsetAsync(sl.sched.p, 0, 16, st));
-    if (np > 0) {
-        k_expand_units<<<(unsigned)((np + 255) / 256), 256, 0, st>>>(np, sl.unit_off.as<int32_t>(), sl.unit_psm.as<int32_t>());
-        CK(cudaGetLastError());
-        s->ctr.kernel_launches++;
-    }
-    CK(cudaEventRecord(cs.e_cnt0, st));
-    if (n_units > 0) {
-        PaCountArgs ca;
-        ca.n_units = n_units; ca.unit_psm = sl.unit_psm.as<int32_t>(); ca.unit_off = sl.unit_off.as<int32_t>();
-        ca.iso_off = sl.iso_off.as<int64_t>(); ca.psm_S = sl.psm_S.as<int32_t>(); ca.psm_status = sl.psm_status.as<int32_t>();
-        ca.iso = iso; ca.n_lookups = sl.lookups.as<unsigned long long>();
-        const int wpb = 8;
-        const bool pair = s->cfg.n_types == 2;
-        size_t smem = wpb * sizeof(PsmSmem);
-        ca.next_unit = sl.sched.as<unsigned long long>();
-        const int64_t want = ((int64_t)n_units + wpb - 1) / wpb;
-        // template switches: neutral losses configured, exactly two ion types, mz_error > 0.5.
-        // One resident wave of blocks; the warps pull units from the cursor.
-#define PA_K2_LAUNCH(NL, PR, EG) { \
-            int blocks = (int)std::min<int64_t>(want, (int64_t)s->sm_count * resident_blocks(k_count_score<NL, PR, EG>, wpb * 32, smem)); \
-            ca.grab = grab_size(n_units, (int64_t)blocks * wpb, PA_K2_GRAB); \
-            k_count_score<NL, PR, EG><<<blocks, wpb * 32, smem, st>>>(s->cfg, cs.b, ca); }
-        const int variant = (s->cfg.has_nl ? 4 : 0) | (pair ? 2 : 0) | (s->cfg.err_gt_half ? 1 : 0);
-        switch (variant) {
-            case 0: PA_K2_LAUNCH(false, false, false) break;
-            case 1: PA_K2_LAUNCH(false, false, true) break;
-            case 2: PA_K2_LAUNCH(false, true, false) break;
-            case 3: PA_K2_LAUNCH(false, true, true) break;
-            case 4: PA_K2_LAUNCH(true, false, false) break;
-            case 5: PA_K2_LAUNCH(true, false, true) break;
-            case 6: PA_K2_LAUNCH(true, true, false) break;
-            default: PA_K2_LAUNCH(true, true, true) break;
-        }
-#undef PA_K2_LAUNCH
-        CK(cudaGetLastError());
-        s->ctr.kernel_launches++; s->ctr.launches_count++;
-    }
-    CK(cudaEventRecord(cs.e_cnt1, st));
-    // K2d: depths 10 .. n_top-1 (n_top > 10 only)
-    PaDeep deep;
-    deep.nd = s->n_deep; deep.T = s->d_T_deep.as<float>(); deep.cnt = nullptr;
-    if (deep.nd > 0) {
-        CK(sl.iso_deep.ensure((size_t)std::max<int64_t>(total_iso, 1) * deep.nd * sizeof(uint16_t)));
-        deep.cnt = sl.iso_deep.as<uint16_t>();
-        cs.e_deep1 = next_event(s);
-        if (n_units > 0) {
-            PaDeepCountArgs da;
-            da.n_units = n_units; da.unit_psm = sl.unit_psm.as<int32_t>(); da.unit_off = sl.unit_off.as<int32_t>();
-            da.iso_off = sl.iso_off.as<int64_t>(); da.psm_S = sl.psm_S.as<int32_t>(); da.iso_hi = iso.hi;
-            da.cnt = sl.iso_deep.as<uint16_t>(); da.nd = deep.nd;
-            const int wpb = 4;
-            const size_t smem = wpb * (sizeof(PsmSmem) + 32 * deep.nd * sizeof(uint16_t));
-            const int64_t want = ((int64_t)n_units + wpb - 1) / wpb;
-            if (s->cfg.has_nl) {
-                const int blocks = (int)std::min<int64_t>(want, (int64_t)s->sm_count * resident_blocks(k_count_deep<true>, wpb * 32, smem));
-                k_count_deep<true><<<blocks, wpb * 32, smem, st>>>(s->cfg, cs.b, da);
-            } else {
-                const int blocks = (int)std::min<int64_t>(want, (int64_t)s->sm_count * resident_blocks(k_count_deep<false>, wpb * 32, smem));
-                k_count_deep<false><<<blocks, wpb * 32, smem, st>>>(s->cfg, cs.b, da);
-            }
-            CK(cudaGetLastError());
-            s->ctr.kernel_launches++; s->ctr.launches_deep++;
-        }
-        CK(cudaEventRecord(cs.e_deep1, st));
-    }
-    // outputs
     const int64_t nm = cs.mod_hi - cs.mod_lo;
     ChunkArray* res = cs.res;
     res[0] = {out->best_sig, r.p0, np, sl.o_sig, cs.o_sig};
@@ -1232,6 +1166,109 @@ static int chunk_back(pa_scorer* s, int si, const pa_results* out, bool out_dev,
     } else {
         for (int i = 0; i < 7; i++) CK(stage(res[i], out_dev, st, nullptr));
     }
+    return PA_OK;
+}
+
+// Pass `pass` of a chunk once its plan is on the host: K2, K2d, K3a, K3b / K3c for the PSMs of type cs.types[pass],
+// with ts's settings and device tables; s owns the slots (scratch reused in stream order) and the counters.
+static int chunk_pass(pa_scorer* s, pa_scorer* ts, int si, ChunkState& cs, int pass, bool keep) {
+    Slot& sl = s->slot[si];
+    cudaStream_t st = sl.st;
+    const ChunkRange& r = cs.r;
+    const int64_t np = r.p1 - r.p0;
+    PassEvents& ev = cs.ev[pass];
+    CK(cudaEventSynchronize(sl.ev_plan));
+    PlanTotals T = *sl.h_totals.as<PlanTotals>();
+    const int64_t total_iso = T.total_iso;
+    const int n_units = T.total_units;
+    // tables that depend on what the chunk contains (errors are reported on s, the handle of the call)
+    int rc = ensure_table(ts, std::max(T.max_frag, 1));
+    for (int S = 0; S < 64 && rc == PA_OK; S++)
+        for (int k = 0; k < 64 && rc == PA_OK; k++)
+            if ((T.combo_bits[S] >> k) & 1ull) rc = ensure_perm(ts, S, k);
+    if (rc == PA_OK) rc = upload_perms(ts);
+    if (rc != PA_OK) { if (ts != s) s->error = ts->error; return rc; }
+    // scratch
+    CK(sl.iso_lo.ensure((size_t)std::max<int64_t>(total_iso, 1) * 8));
+    CK(sl.iso_hi.ensure((size_t)std::max<int64_t>(total_iso, 1) * 8));
+    CK(sl.iso_n.ensure((size_t)std::max<int64_t>(total_iso, 1) * 4));
+    CK(sl.iso_w.ensure((size_t)std::max<int64_t>(total_iso, 1) * 4));
+    CK(sl.g_sort.ensure((size_t)std::max<int64_t>(total_iso, 1) * 8));
+    CK(sl.g_lr.ensure((size_t)(std::max<int64_t>(total_iso, 1) + 2 * np + 2) * 4));
+    CK(sl.unit_psm.ensure((size_t)std::max(n_units, 1) * 4));
+    PaIso iso;
+    iso.lo = sl.iso_lo.as<unsigned long long>(); iso.hi = sl.iso_hi.as<unsigned long long>();
+    iso.nfrag = sl.iso_n.as<uint32_t>(); iso.w = sl.iso_w.as<float>();
+    ev.e_cnt0 = next_event(s); ev.e_cnt1 = next_event(s); ev.e_sel1 = next_event(s);
+    CK(sl.sched.ensure(16));                          // work cursors of k_count_score [0] and k_select [1]
+    CK(cudaMemsetAsync(sl.sched.p, 0, 16, st));
+    if (np > 0) {
+        k_expand_units<<<(unsigned)((np + 255) / 256), 256, 0, st>>>(np, sl.unit_off.as<int32_t>(), sl.unit_psm.as<int32_t>());
+        CK(cudaGetLastError());
+        s->ctr.kernel_launches++;
+    }
+    CK(cudaEventRecord(ev.e_cnt0, st));
+    if (n_units > 0) {
+        PaCountArgs ca;
+        ca.n_units = n_units; ca.unit_psm = sl.unit_psm.as<int32_t>(); ca.unit_off = sl.unit_off.as<int32_t>();
+        ca.iso_off = sl.iso_off.as<int64_t>(); ca.psm_S = sl.psm_S.as<int32_t>(); ca.psm_status = sl.psm_status.as<int32_t>();
+        ca.iso = iso; ca.n_lookups = sl.lookups.as<unsigned long long>();
+        const int wpb = 8;
+        const bool pair = ts->cfg.n_types == 2;
+        size_t smem = wpb * sizeof(PsmSmem);
+        ca.next_unit = sl.sched.as<unsigned long long>();
+        const int64_t want = ((int64_t)n_units + wpb - 1) / wpb;
+        // template switches: neutral losses configured, exactly two ion types, mz_error > 0.5.
+        // One resident wave of blocks; the warps pull units from the cursor.
+#define PA_K2_LAUNCH(NL, PR, EG) { \
+            int blocks = (int)std::min<int64_t>(want, (int64_t)s->sm_count * resident_blocks(k_count_score<NL, PR, EG>, wpb * 32, smem)); \
+            ca.grab = grab_size(n_units, (int64_t)blocks * wpb, PA_K2_GRAB); \
+            k_count_score<NL, PR, EG><<<blocks, wpb * 32, smem, st>>>(ts->cfg, cs.b, ca); }
+        const int variant = (ts->cfg.has_nl ? 4 : 0) | (pair ? 2 : 0) | (ts->cfg.err_gt_half ? 1 : 0);
+        switch (variant) {
+            case 0: PA_K2_LAUNCH(false, false, false) break;
+            case 1: PA_K2_LAUNCH(false, false, true) break;
+            case 2: PA_K2_LAUNCH(false, true, false) break;
+            case 3: PA_K2_LAUNCH(false, true, true) break;
+            case 4: PA_K2_LAUNCH(true, false, false) break;
+            case 5: PA_K2_LAUNCH(true, false, true) break;
+            case 6: PA_K2_LAUNCH(true, true, false) break;
+            default: PA_K2_LAUNCH(true, true, true) break;
+        }
+#undef PA_K2_LAUNCH
+        CK(cudaGetLastError());
+        s->ctr.kernel_launches++; s->ctr.launches_count++;
+    }
+    CK(cudaEventRecord(ev.e_cnt1, st));
+    // K2d: depths 10 .. n_top-1 (n_top > 10 only)
+    PaDeep deep;
+    deep.nd = ts->n_deep; deep.T = ts->d_T_deep.as<float>(); deep.cnt = nullptr;
+    if (deep.nd > 0) {
+        CK(sl.iso_deep.ensure((size_t)std::max<int64_t>(total_iso, 1) * deep.nd * sizeof(uint16_t)));
+        deep.cnt = sl.iso_deep.as<uint16_t>();
+        ev.e_deep1 = next_event(s);
+        if (n_units > 0) {
+            PaDeepCountArgs da;
+            da.n_units = n_units; da.unit_psm = sl.unit_psm.as<int32_t>(); da.unit_off = sl.unit_off.as<int32_t>();
+            da.iso_off = sl.iso_off.as<int64_t>(); da.psm_S = sl.psm_S.as<int32_t>(); da.iso_hi = iso.hi;
+            da.cnt = sl.iso_deep.as<uint16_t>(); da.nd = deep.nd;
+            const int wpb = 4;
+            const size_t smem = wpb * (sizeof(PsmSmem) + 32 * deep.nd * sizeof(uint16_t));
+            const int64_t want = ((int64_t)n_units + wpb - 1) / wpb;
+            if (ts->cfg.has_nl) {
+                const int blocks = (int)std::min<int64_t>(want, (int64_t)s->sm_count * resident_blocks(k_count_deep<true>, wpb * 32, smem));
+                k_count_deep<true><<<blocks, wpb * 32, smem, st>>>(ts->cfg, cs.b, da);
+            } else {
+                const int blocks = (int)std::min<int64_t>(want, (int64_t)s->sm_count * resident_blocks(k_count_deep<false>, wpb * 32, smem));
+                k_count_deep<false><<<blocks, wpb * 32, smem, st>>>(ts->cfg, cs.b, da);
+            }
+            CK(cudaGetLastError());
+            s->ctr.kernel_launches++; s->ctr.launches_deep++;
+        }
+        CK(cudaEventRecord(ev.e_deep1, st));
+    }
+    // K3a .. K3c (the result views: stage_results)
+    const int64_t nm = cs.mod_hi - cs.mod_lo;
     CK(sl.best_idx.ensure((size_t)std::max<int64_t>(np, 1) * 4));
     CK(sl.mod_psm.ensure((size_t)std::max<int64_t>(nm, 1) * 4));
     CK(sl.tie.ensure((size_t)std::max<int64_t>(nm, 1) * 8));
@@ -1240,12 +1277,12 @@ static int chunk_back(pa_scorer* s, int si, const pa_results* out, bool out_dev,
     CK(sl.work_val.ensure((size_t)std::max<int64_t>(nm, 1) * 4)); CK(sl.work_sorted.ensure((size_t)std::max<int64_t>(nm, 1) * 4));
     CK(sl.generic_count.ensure(32));                 // [0] generic entries, [1..4] k_ascore work entries by class
     CK(cudaMemsetAsync(sl.generic_count.p, 0, 32, st));
-    cs.e_asc1 = next_event(s);
+    ev.e_asc1 = next_event(s);
     if (np > 0) {
         PaSelArgs sa;
         sa.n_psm = np; sa.iso_off = sl.iso_off.as<int64_t>(); sa.psm_S = sl.psm_S.as<int32_t>();
         sa.psm_status = sl.psm_status.as<int32_t>(); sa.iso = iso;
-        sa.perm_off = s->d_perm_off.as<int64_t>(); sa.perm_pool = s->d_perm_pool.as<uint32_t>();
+        sa.perm_off = ts->d_perm_off.as<int64_t>(); sa.perm_pool = ts->d_perm_pool.as<uint32_t>();
         sa.mod_off = cs.mod_off_abs;
         sa.best_sig = cs.o_sig ? cs.o_sig + r.p0 : nullptr;
         sa.best_score = cs.o_score ? cs.o_score + r.p0 : nullptr;
@@ -1263,16 +1300,17 @@ static int chunk_back(pa_scorer* s, int si, const pa_results* out, bool out_dev,
         // the warp-per-PSM kernel, whose visit count is therefore only known on the device
         CK(sl.rest_list.ensure((size_t)std::max<int64_t>(np, 1) * 4));
         sa.rest_list = sl.rest_list.as<int32_t>(); sa.rest_count = sl.generic_count.as<int>() + 5;
-        k_select_thread<<<(unsigned)((np + 127) / 128), 128, 0, st>>>(s->cfg, cs.b, sa);
+        if (cs.psm_type) k_select_thread<true><<<(unsigned)((np + 127) / 128), 128, 0, st>>>(ts->cfg, cs.b, sa);
+        else k_select_thread<false><<<(unsigned)((np + 127) / 128), 128, 0, st>>>(ts->cfg, cs.b, sa);
         CK(cudaGetLastError());
         const int wpb = 8;
         const size_t sel_smem = wpb * PA_SORTCAP * sizeof(unsigned long long);
         int blocks = (int)std::min<int64_t>((np + wpb - 1) / wpb, (int64_t)s->sm_count * resident_blocks(k_select, wpb * 32, sel_smem));
-        k_select<<<blocks, wpb * 32, sel_smem, st>>>(s->cfg, cs.b, sa);
+        k_select<<<blocks, wpb * 32, sel_smem, st>>>(ts->cfg, cs.b, sa);
         CK(cudaGetLastError());
         s->ctr.kernel_launches += 2; s->ctr.launches_select += 2;
     }
-    CK(cudaEventRecord(cs.e_sel1, st));
+    CK(cudaEventRecord(ev.e_sel1, st));
     if (np > 0 && nm > 0 && cs.o_asc != nullptr) {
         PaAscArgs aa;
         aa.n_entries = nm; aa.mod_lo = cs.mod_lo; aa.mod_psm = sl.mod_psm.as<int32_t>();
@@ -1301,22 +1339,22 @@ static int chunk_back(pa_scorer* s, int si, const pa_results* out, bool out_dev,
         ia.item_cnt = sl.item_cnt.as<int32_t>(); ia.item_off = sl.item_off.as<int32_t>();
         ia.cursor = sl.asc_cursor.as<unsigned long long>(); ia.gen_flag = sl.gen_flag.as<int>();
         k_asc_item_count<<<(unsigned)((nm + 1 + 255) / 256), 256, 0, st>>>(aa, ia);
-        size_t ts = 0;
-        CK(cub::DeviceScan::ExclusiveSum(nullptr, ts, ia.item_cnt, sl.item_off.as<int32_t>(), (int)(nm + 1), st));
-        CK(sl.cub_tmp.ensure(ts + 256));
-        ts = sl.cub_tmp.cap;
-        CK(cub::DeviceScan::ExclusiveSum(sl.cub_tmp.p, ts, ia.item_cnt, sl.item_off.as<int32_t>(), (int)(nm + 1), st));
+        size_t tsz = 0;
+        CK(cub::DeviceScan::ExclusiveSum(nullptr, tsz, ia.item_cnt, sl.item_off.as<int32_t>(), (int)(nm + 1), st));
+        CK(sl.cub_tmp.ensure(tsz + 256));
+        tsz = sl.cub_tmp.cap;
+        CK(cub::DeviceScan::ExclusiveSum(sl.cub_tmp.p, tsz, ia.item_cnt, sl.item_off.as<int32_t>(), (int)(nm + 1), st));
         s->ctr.kernel_launches += 2;
         // (n_top > 10: the DEEP instantiations, whose depth argmax goes on over depths 10 .. n_top-1)
 #define PA_PAIRS_LAUNCH(NQ, CLS, SMEM) { \
             if (deep.nd > 0) { \
                 const int blocks = (int)std::min<int64_t>(ab, (int64_t)s->sm_count * resident_blocks(k_ascore_pairs<NQ, CLS, true>, 128, SMEM)); \
-                k_ascore_pairs<NQ, CLS, true><<<blocks, 128, SMEM, st>>>(s->cfg, cs.b, aa, ia, deep); \
+                k_ascore_pairs<NQ, CLS, true><<<blocks, 128, SMEM, st>>>(ts->cfg, cs.b, aa, ia, deep); \
             } else { \
                 const int blocks = (int)std::min<int64_t>(ab, (int64_t)s->sm_count * resident_blocks(k_ascore_pairs<NQ, CLS, false>, 128, SMEM)); \
-                k_ascore_pairs<NQ, CLS, false><<<blocks, 128, SMEM, st>>>(s->cfg, cs.b, aa, ia, deep); \
+                k_ascore_pairs<NQ, CLS, false><<<blocks, 128, SMEM, st>>>(ts->cfg, cs.b, aa, ia, deep); \
             } }
-        if (!s->cfg.has_nl) {
+        if (!ts->cfg.has_nl) {
             PA_PAIRS_LAUNCH(1, 0, 0) PA_PAIRS_LAUNCH(2, 1, 0) PA_PAIRS_LAUNCH(4, 2, 0)
             s->ctr.kernel_launches += 3;
         }
@@ -1328,19 +1366,12 @@ static int chunk_back(pa_scorer* s, int si, const pa_results* out, bool out_dev,
         int64_t stride = 32;
         while (stride < T.max_list) stride <<= 1;
         if (T.max_list > PA_LCAP) CK(sl.g_lists.ensure((size_t)blocks * wpb * 4 * stride * sizeof(float)));
-        if (deep.nd > 0) k_ascore_generic<true><<<blocks, wpb * 32, wpb * sizeof(SelSmem), st>>>(s->cfg, cs.b, aa, sl.g_lists.as<float>(), stride, deep);
-        else k_ascore_generic<false><<<blocks, wpb * 32, wpb * sizeof(SelSmem), st>>>(s->cfg, cs.b, aa, sl.g_lists.as<float>(), stride, deep);
+        if (deep.nd > 0) k_ascore_generic<true><<<blocks, wpb * 32, wpb * sizeof(SelSmem), st>>>(ts->cfg, cs.b, aa, sl.g_lists.as<float>(), stride, deep);
+        else k_ascore_generic<false><<<blocks, wpb * 32, wpb * sizeof(SelSmem), st>>>(ts->cfg, cs.b, aa, sl.g_lists.as<float>(), stride, deep);
         CK(cudaGetLastError());
         s->ctr.kernel_launches += 2; s->ctr.launches_ascore += 2;
     }
-    CK(cudaEventRecord(cs.e_asc1, st));
-    int64_t* d2h = &s->ctr.bytes_d2h;
-    if (cs.packed_res) {         // (score_impl copies the block into the caller's arrays once the stream is done)
-        CK(cudaMemcpyAsync(sl.h_opack.p, sl.d_opack.p, cs.packed_res_bytes, cudaMemcpyDeviceToHost, st));
-        *d2h += (int64_t)cs.packed_res_bytes;
-    } else {
-        for (int i = 0; i < 7; i++) CK(copy_back(res[i], out_dev, st, d2h));
-    }
+    CK(cudaEventRecord(ev.e_asc1, st));
     s->ctr.n_isoforms += total_iso;
     if (keep) {
         s->kept.b = cs.b; s->kept.n_psm = np; s->kept.psm_lo = r.p0;
@@ -1348,6 +1379,26 @@ static int chunk_back(pa_scorer* s, int si, const pa_results* out, bool out_dev,
         s->kept.psm_status = sl.psm_status.as<int32_t>(); s->kept.iso = iso; s->kept.max_list = T.max_list;
         s->kept.iso_deep = deep.cnt;
         s->kept.valid = true; s->kept.slot = si;
+    }
+    return PA_OK;
+}
+
+static int chunk_back(pa_scorer* s, pa_scorer* const* sc, int n_types, int si, const pa_results* out, bool out_dev,
+                      ChunkState& cs, bool keep) {
+    Slot& sl = s->slot[si];
+    cudaStream_t st = sl.st;
+    int rc = stage_results(s, si, out, out_dev, cs);
+    for (size_t pass = 0; pass < cs.types.size() && rc == PA_OK; pass++) {
+        if (pass > 0) rc = chunk_plan(s, sc[cs.types[pass]], si, cs, (int)pass, n_types);
+        if (rc == PA_OK) rc = chunk_pass(s, sc[cs.types[pass]], si, cs, (int)pass, keep);
+    }
+    if (rc != PA_OK) return rc;
+    int64_t* d2h = &s->ctr.bytes_d2h;
+    if (cs.packed_res) {         // (score_impl copies the block into the caller's arrays once the stream is done)
+        CK(cudaMemcpyAsync(sl.h_opack.p, sl.d_opack.p, cs.packed_res_bytes, cudaMemcpyDeviceToHost, st));
+        *d2h += (int64_t)cs.packed_res_bytes;
+    } else {
+        for (int i = 0; i < 7; i++) CK(copy_back(cs.res[i], out_dev, st, d2h));
     }
     return PA_OK;
 }
@@ -1368,8 +1419,26 @@ static const char* check_host_range(const pa_batch* in, int64_t p0, int64_t p1, 
     return nullptr;
 }
 
-static int score_impl(pa_scorer* s, const pa_batch* in, const pa_results* out, int64_t p_lo, int64_t p_hi, uint32_t flags) {
+// Types of PSMs [p_lo, p_hi) of a typed batch: count[t] PSMs of type t, a type >= n_types counted as type 0 (whose
+// pass reports it).
+__global__ void k_type_count(const uint8_t* psm_type, int64_t p_lo, int64_t p_hi, int n_types, unsigned int* count) {
+    __shared__ unsigned int c[256];
+    for (int i = threadIdx.x; i < 256; i += blockDim.x) c[i] = 0;
+    __syncthreads();
+    for (int64_t p = p_lo + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < p_hi; p += (int64_t)gridDim.x * blockDim.x) {
+        const int t = psm_type[p];
+        atomicAdd(&c[t < n_types ? t : 0], 1u);
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < 256; i += blockDim.x) if (c[i]) atomicAdd(&count[i], c[i]);
+}
+
+// sc[0 .. n_types) (typed batches, pa_score_typed; null: s alone) score the PSMs of each type; s == sc[0] owns the
+// slots, the counters and the error text.  psm_type: on the side of the batch's arrays, null = every PSM is type 0.
+static int score_impl(pa_scorer* s, const pa_batch* in, const pa_results* out, int64_t p_lo, int64_t p_hi, uint32_t flags,
+                      pa_scorer* const* sc = nullptr, int n_types = 1, const uint8_t* psm_type = nullptr) {
     if (!s) return PA_ERR_ARG;
+    if (!sc) sc = &s;
     if (!in || !out) return fail(s, PA_ERR_ARG, "NULL batch or results");
     if (s->binner_only) return fail(s, PA_ERR_STATE, "this handle was made by pa_create_binner: it only bins spectra");
     if (in->n_psm < 0 || in->n_spec < 0) return fail(s, PA_ERR_ARG, "negative sizes");
@@ -1404,12 +1473,13 @@ static int score_impl(pa_scorer* s, const pa_batch* in, const pa_results* out, i
     std::vector<int> chunk_maxp;
     std::vector<int64_t> mod_lo, mod_hi;
     DevBounds hb;
+    unsigned int dev_type_n[256];
     if (in_dev) {
         // Device-resident batch: one chunk (see DevBounds).  One small kernel gathers the range ends the host needs,
         // a second checks the CSR arrays (and that psm_spec is non-decreasing: the spectrum range relies on it), a
         // third finds the largest spectrum: one device -> host copy instead of one per value.
         DevBuf& tb = s->slot[0].totals;
-        CK(tb.ensure(sizeof(PlanTotals) + sizeof(DevBounds)));
+        CK(tb.ensure(sizeof(PlanTotals) + sizeof(DevBounds) + 256 * sizeof(unsigned int)));
         DevBounds* d_b = (DevBounds*)tb.p;
         CK(cudaMemset(d_b, 0, sizeof(DevBounds)));
         k_dev_bounds<<<1, 1>>>(in->spec_off, in->psm_spec, in->pep_off, in->aux_off, in->mod_off, p_lo, p_hi, in->n_spec, d_b);
@@ -1427,6 +1497,14 @@ static int score_impl(pa_scorer* s, const pa_batch* in, const pa_results* out, i
             CK(cudaMemcpy(&hb.peak1, in->spec_off + in->n_spec, 8, cudaMemcpyDeviceToHost));
         }
         chunks.push_back({p_lo, p_hi, hb.s0, hb.s1});
+        if (psm_type) {          // the types present: one more small kernel and copy
+            unsigned int* d_cnt = (unsigned int*)(d_b + 1);
+            CK(cudaMemset(d_cnt, 0, 256 * sizeof(unsigned int)));
+            k_type_count<<<(unsigned)std::min<int64_t>((n_range + 255) / 256, 1184), 256>>>(psm_type, p_lo, p_hi, n_types, d_cnt);
+            CK(cudaGetLastError());
+            s->ctr.kernel_launches++;
+            CK(cudaMemcpy(dev_type_n, d_cnt, sizeof(dev_type_n), cudaMemcpyDeviceToHost));
+        }
         mod_lo.push_back(hb.mod0); mod_hi.push_back(hb.mod1);
         chunk_maxp.push_back(hb.max_peaks);
         s->ctr.n_peaks += hb.peak1 - hb.peak0;
@@ -1480,6 +1558,14 @@ static int score_impl(pa_scorer* s, const pa_batch* in, const pa_results* out, i
 
     // ---- two-slot software pipeline ----
     std::vector<ChunkState> cs(chunks.size());
+    // the passes of each chunk: one per type with PSMs in it (a type >= n_types goes with type 0, whose pass reports it)
+    for (size_t c = 0; c < chunks.size(); c++) {
+        if (!psm_type) { cs[c].types = {0}; continue; }
+        std::vector<int64_t> n(256, 0);
+        if (in_dev) for (int t = 0; t < 256; t++) n[t] = dev_type_n[t];
+        else for (int64_t p = chunks[c].p0; p < chunks[c].p1; p++) n[psm_type[p] < n_types ? psm_type[p] : 0]++;
+        for (int t = 0; t < n_types; t++) if (n[t] > 0) cs[c].types.push_back(t);
+    }
     s->ctr.n_chunks = (int64_t)chunks.size();
     cs[0].single_chunk = chunks.size() == 1;
     // The m/z narrowing of a host chunk (narrow_begin / narrow_end) runs on the pool one chunk AHEAD of the copies: the
@@ -1500,8 +1586,8 @@ static int score_impl(pa_scorer* s, const pa_batch* in, const pa_results* out, i
         rc = narrow_begin(s, nstage(0), in, chunks[0]);           // (chunk_front waits for it, after the chunk's other copies)
         if (rc != PA_OK) return bail(rc);
     }
-    rc = chunk_front(s, 0, in, in_dev, chunks[0], mod_lo[0], mod_hi[0], chunk_maxp[0], cs[0], in_dev ? &hb : nullptr,
-                     may_narrow ? &nstage(0) : nullptr);
+    rc = chunk_front(s, sc, n_types, 0, in, psm_type, in_dev, chunks[0], mod_lo[0], mod_hi[0], chunk_maxp[0], cs[0],
+                     in_dev ? &hb : nullptr, may_narrow ? &nstage(0) : nullptr);
     if (rc != PA_OK) return bail(rc);
     if (may_narrow && chunks.size() > 1) { rc = narrow_begin(s, nstage(1), in, chunks[1]); if (rc != PA_OK) return bail(rc); }
     for (size_t c = 0; c < chunks.size(); c++) {
@@ -1511,12 +1597,13 @@ static int score_impl(pa_scorer* s, const pa_batch* in, const pa_results* out, i
                 if (why) { bail(0); return fail(s, PA_ERR_ARG, "inconsistent batch: %s", why); }
             }
             // slot (c+1)&1 was last used by chunk c-1: its stream order keeps buffers safe
-            rc = chunk_front(s, (int)((c + 1) & 1), in, in_dev, chunks[c + 1], mod_lo[c + 1], mod_hi[c + 1],
-                             chunk_maxp[c + 1], cs[c + 1], in_dev ? &hb : nullptr, may_narrow ? &nstage(c + 1) : nullptr);
+            rc = chunk_front(s, sc, n_types, (int)((c + 1) & 1), in, psm_type, in_dev, chunks[c + 1], mod_lo[c + 1],
+                             mod_hi[c + 1], chunk_maxp[c + 1], cs[c + 1], in_dev ? &hb : nullptr,
+                             may_narrow ? &nstage(c + 1) : nullptr);
             if (rc != PA_OK) return bail(rc);
             if (may_narrow && c + 2 < chunks.size()) { rc = narrow_begin(s, nstage(c + 2), in, chunks[c + 2]); if (rc != PA_OK) return bail(rc); }
         }
-        rc = chunk_back(s, (int)(c & 1), out, out_dev, cs[c], keep);
+        rc = chunk_back(s, sc, n_types, (int)(c & 1), out, out_dev, cs[c], keep);
         if (rc != PA_OK) return bail(rc);
     }
     for (int i = 0; i < 2; i++)
@@ -1534,11 +1621,13 @@ static int score_impl(pa_scorer* s, const pa_batch* in, const pa_results* out, i
     for (size_t c = 0; c < chunks.size(); c++) {
         float ms = 0.f;
         cudaEventElapsedTime(&ms, cs[c].e_bin0, cs[c].e_bin1); s->ctr.ms_bin += ms;
-        cudaEventElapsedTime(&ms, cs[c].e_bin1, cs[c].e_plan1); s->ctr.ms_plan += ms;
-        cudaEventElapsedTime(&ms, cs[c].e_cnt0, cs[c].e_cnt1); s->ctr.ms_count += ms;
-        if (cs[c].e_deep1) { cudaEventElapsedTime(&ms, cs[c].e_cnt1, cs[c].e_deep1); s->ctr.ms_deep += ms; }
-        cudaEventElapsedTime(&ms, cs[c].e_deep1 ? cs[c].e_deep1 : cs[c].e_cnt1, cs[c].e_sel1); s->ctr.ms_select += ms;
-        cudaEventElapsedTime(&ms, cs[c].e_sel1, cs[c].e_asc1); s->ctr.ms_ascore += ms;
+        for (const PassEvents& ev : cs[c].ev) {
+            cudaEventElapsedTime(&ms, ev.e_plan0, ev.e_plan1); s->ctr.ms_plan += ms;
+            cudaEventElapsedTime(&ms, ev.e_cnt0, ev.e_cnt1); s->ctr.ms_count += ms;
+            if (ev.e_deep1) { cudaEventElapsedTime(&ms, ev.e_cnt1, ev.e_deep1); s->ctr.ms_deep += ms; }
+            cudaEventElapsedTime(&ms, ev.e_deep1 ? ev.e_deep1 : ev.e_cnt1, ev.e_sel1); s->ctr.ms_select += ms;
+            cudaEventElapsedTime(&ms, ev.e_sel1, ev.e_asc1); s->ctr.ms_ascore += ms;
+        }
     }
     cudaEventElapsedTime(&s->ctr.ms_total, e_all0, e_all1);
     s->ctr.n_fragment_lookups = (int64_t)*s->slot[0].h_lookups.as<unsigned long long>() + (int64_t)*s->slot[1].h_lookups.as<unsigned long long>();
@@ -1564,6 +1653,26 @@ extern "C" int pa_score_range(pa_scorer* s, const pa_batch* in, const pa_results
     if (!s) return PA_ERR_ARG;
     if (s->busy) return busy_error(s);
     return score_impl(s, in, out, psm_lo, psm_hi, flags);
+}
+
+extern "C" int pa_score_typed(pa_scorer* const* s, int32_t n_types, const pa_batch* in, const uint8_t* psm_type,
+                              const pa_results* out, uint32_t flags) {
+    if (!s || !s[0]) return fail(nullptr, PA_ERR_ARG, "pa_score_typed: NULL scorer list or NULL first handle");
+    pa_scorer* s0 = s[0];
+    if (n_types < 1 || n_types > 255) return fail(s0, PA_ERR_ARG, "pa_score_typed: n_types = %d outside 1 .. 255", (int)n_types);
+    for (int t = 0; t < n_types; t++) {
+        if (!s[t]) return fail(s0, PA_ERR_ARG, "pa_score_typed: handle of type %d is NULL", t);
+        if (s[t]->binner_only) return fail(s0, PA_ERR_ARG, "pa_score_typed: handle of type %d was made by pa_create_binner: it only bins spectra", t);
+        if (s[t]->device != s0->device) return fail(s0, PA_ERR_ARG, "pa_score_typed: handle of type %d is on device %d, type 0 on device %d", t, s[t]->device, s0->device);
+        if (s[t]->bin_size != s0->bin_size || s[t]->n_top != s0->n_top)
+            return fail(s0, PA_ERR_ARG, "pa_score_typed: handle of type %d bins with bin_size %g / n_top %d, type 0 with %g / %d: the "
+                        "spectra are binned once for every type", t, (double)s[t]->bin_size, s[t]->n_top, (double)s0->bin_size, s0->n_top);
+    }
+    for (int t = 0; t < n_types; t++)
+        if (s[t]->busy) return fail(s0, PA_ERR_STATE, "pa_score_typed: handle of type %d has an asynchronous call in flight: call pa_wait first", t);
+    if ((flags & PA_KEEP_ISOFORMS) && n_types > 1)
+        return fail(s0, PA_ERR_UNSUPPORTED, "pa_score_typed: PA_KEEP_ISOFORMS is not supported with more than one type");
+    return score_impl(s0, in, out, 0, in ? in->n_psm : 0, flags, s, n_types, psm_type);
 }
 
 // The path has one host decision per chunk (the plan totals size the isoform scratch), so "asynchronous" means a

@@ -41,31 +41,40 @@ def fragment_charge(match_charge, precursor_charge, max_fragment_charge):
 
 
 class PsmPacker:
-    """Accumulates the PSMs that will be scored (n_variable > 0) of scan-sorted match records."""
+    """Accumulates the PSMs that will be scored (n_variable > 0) of scan-sorted match records.
+
+    `types` (default: the one type (residues, mod_mass)) lists the (residues, mod_mass) of every modification type of
+    a typed batch (`score_typed`): a record added as type t is split by process_mods with types[t], and with more
+    than one type every flushed batch carries `psm_type` (uint8, one per row)."""
 
     def __init__(self, spectra, residues="STY", mod_mass=79.966331, mod_correction_tol=1., zero_based=False,
-                 max_fragment_charge=5, hit_depth=1):
+                 max_fragment_charge=5, hit_depth=1, types=None):
         self.spectra = spectra
-        self.residues, self.mod_mass, self.tol = residues, mod_mass, mod_correction_tol
+        self.types = list(types) if types is not None else [(residues, mod_mass)]
+        self.residues, self.mod_mass = self.types[0]
+        self.tol = mod_correction_tol
         self.zero_based, self.max_z, self.hit_depth = zero_based, max_fragment_charge, hit_depth
         self._reset()
 
     def _reset(self):
         self.scans, self.psm_spec, self.peps, self.n_mod, self.max_charge = [], [], [], [], []
-        self.aux_pos, self.aux_mass = [], []
+        self.aux_pos, self.aux_mass, self.psm_type = [], [], []
 
     def __len__(self):
         return len(self.scans)
 
-    def add(self, match):
-        """pack one PSM record; returns True when it carries variable mods (i.e. will be scored)"""
+    def add(self, match, t=0):
+        """pack one PSM record as type t; returns True when it carries variable mods of that type (i.e. will be
+        scored)"""
         idx = self.spectra.index_of(match["scan"])
         if idx < 0:
             raise KeyError(match["scan"])            # the reference indexes spectra_map[scan] (:133)
-        cpos, cmass, n_var = process_mods(self.residues, self.mod_mass, self.tol, self.zero_based,
+        residues, mod_mass = self.types[t]
+        cpos, cmass, n_var = process_mods(residues, mod_mass, self.tol, self.zero_based,
                                           match["peptide"], match["mod_positions"], match["mod_masses"])
         if n_var <= 0:
             return False
+        self.psm_type.append(t)
         self.scans.append(int(match["scan"]))
         self.psm_spec.append(idx)
         self.peps.append(match["peptide"].encode("ascii"))
@@ -100,27 +109,48 @@ class PsmPacker:
             n_mod=np.array(self.n_mod, np.int32), max_charge=np.array(self.max_charge, np.int32), aux_off=aux_off,
             aux_pos=np.concatenate(self.aux_pos).astype(np.uint32) if n else np.zeros(0, np.uint32),
             aux_mass=np.concatenate(self.aux_mass).astype(np.float32) if n else np.zeros(0, np.float32))
+        if len(self.types) > 1:
+            batch["psm_type"] = np.array(self.psm_type, np.uint8)
         scans = np.array(self.scans, np.int64)
         self._reset()
         return scans, batch
 
 
 def iter_batches(spectra, psms, chunk_psms=65536, **packer_kw):
-    """scan-sorted PSM records -> (scans, batch) chunks cut on scan boundaries"""
+    """scan-sorted PSM records -> (scans, batch) chunks cut on scan boundaries.
+
+    With `types` of more than one entry (see PsmPacker), `psms` holds one scan-sorted record list per type -- the
+    same identifications, mass-corrected for that type -- and every scan contributes its hit_depth hits of type 0,
+    then those of type 1, and so on: psm_spec stays non-decreasing."""
     packer = PsmPacker(spectra, **packer_kw)
-    for _, group in groupby(psms, lambda m: m["scan"]):
-        for ind, match in enumerate(group):
-            if ind == packer.hit_depth:
-                break
-            packer.add(match)
-        if len(packer) >= chunk_psms:
-            yield packer.flush()
+    if len(packer.types) == 1:
+        for _, group in groupby(psms, lambda m: m["scan"]):
+            for ind, match in enumerate(group):
+                if ind == packer.hit_depth:
+                    break
+                packer.add(match)
+            if len(packer) >= chunk_psms:
+                yield packer.flush()
+    else:
+        if len(psms) != len(packer.types):
+            raise ValueError("%d record lists for %d modification types" % (len(psms), len(packer.types)))
+        for groups in zip(*(groupby(p, lambda m: m["scan"]) for p in psms), strict=True):
+            if any(scan != groups[0][0] for scan, _ in groups):
+                raise ValueError("the record lists of the modification types do not list the same scans")
+            for t, (_, group) in enumerate(groups):
+                for ind, match in enumerate(group):
+                    if ind == packer.hit_depth:
+                        break
+                    packer.add(match, t)
+            if len(packer) >= chunk_psms:
+                yield packer.flush()
     if len(packer):
         yield packer.flush()
 
 
 def score_stream(scorer, batches, depth=2):
-    """Score (scans, batch) chunks on the GPU while a producer thread packs the next ones.
+    """Score (scans, batch) chunks on the GPU while a producer thread packs the next ones.  `scorer`: a Scorer /
+    MultiScorer, or a function batch -> results (e.g. around `score_typed`).
 
     `pa_score_batch` is a blocking C call that releases the GIL (ctypes), so host-side
     parsing/packing of chunk c+1 overlaps the H2D copies and kernels of chunk c.  Yields
@@ -157,20 +187,21 @@ def score_stream(scorer, batches, depth=2):
             if isinstance(item, BaseException):
                 raise item
             scans, batch = item
-            yield scans, batch, scorer.score_batch(batch)
+            yield scans, batch, (scorer(batch) if callable(scorer) else scorer.score_batch(batch))
     finally:
         stop.set()
         t.join(timeout=30)
 
 
-def result_rows(scorer, scans, batch, res):
+def result_rows(scorer, scans, batch, res, rows_of=None):
     """-> [scan, LocalizedSequence, PepScore, Ascores, AltSites] rows with the reference's string
     formatting (__main__.py:158-164): ascores `str(np.float32)` joined by ';', alternative sites
-    joined by ',' inside a mod and ';' between mods"""
+    joined by ',' inside a mod and ';' between mods.  rows_of: the batch rows to format (default: all), e.g. the rows
+    of one type of a typed batch, formatted with that type's scorer"""
     from ..batch import format_results
     from .._lib import PSM_STATUS
     rows = []
-    for i in range(scans.size):
+    for i in range(scans.size) if rows_of is None else rows_of:
         status = int(res["psm_status"][i])
         if status != 0:
             import warnings

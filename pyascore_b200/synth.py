@@ -250,3 +250,44 @@ def psm_view(batch, i):
     x, y = int(batch["aux_off"][i]), int(batch["aux_off"][i + 1])
     return (batch["mz"][a:b], batch["inten"][a:b], pep, int(batch["n_mod"][i]), int(batch["max_charge"][i]),
             batch["aux_pos"][x:y], batch["aux_mass"][x:y])
+
+
+def _ragged(off, rows):
+    """indices into the data of a CSR array for rows `rows`, and their offsets"""
+    lens = (off[1:] - off[:-1])[rows].astype(np.int64)
+    new_off = np.zeros(rows.size + 1, np.int64)
+    np.cumsum(lens, out=new_off[1:])
+    return np.repeat(off[:-1][rows].astype(np.int64) - new_off[:-1], lens) + np.arange(new_off[-1]), new_off
+
+
+def select_rows(batch, rows, n_mod=None):
+    """host batch of PSM rows `rows` of `batch` (in that order, repeats allowed) over the same spectra arrays; n_mod:
+    the rows' n_mod (default: theirs)"""
+    rows = np.asarray(rows, np.int64)
+    out = {k: batch[k] for k in ("spec_off", "mz", "inten", "inten32") if k in batch}
+    out["psm_spec"] = np.ascontiguousarray(batch["psm_spec"][rows])
+    idx, off = _ragged(batch["pep_off"], rows)
+    out["pep"], out["pep_off"] = np.ascontiguousarray(batch["pep"][idx]), off.astype(np.int32)
+    idx, off = _ragged(batch["aux_off"], rows)
+    out["aux_pos"], out["aux_mass"] = np.ascontiguousarray(batch["aux_pos"][idx]), np.ascontiguousarray(batch["aux_mass"][idx])
+    out["aux_off"] = off.astype(np.int32)
+    out["n_mod"] = np.ascontiguousarray(batch["n_mod"][rows] if n_mod is None else np.asarray(n_mod, np.int32))
+    out["max_charge"] = np.ascontiguousarray(batch["max_charge"][rows])
+    return out
+
+
+def typed_batch(batch, groups, skip_below=0):
+    """A batch of several modification types (pyascore_b200.score_typed) over the spectra of `batch`: type 0 = every
+    PSM of `batch`; type t >= 1 = for every PSM at index >= skip_below whose peptide has a letter of groups[t-1], a row
+    on the same spectrum with one such modification, right after the PSM's rows of the types before (psm_spec stays
+    non-decreasing).  -> (batch, psm_type uint8)"""
+    n = batch["n_mod"].size
+    pep, off = batch["pep"], batch["pep_off"]
+    rows, n_mod, typ = [np.arange(n)], [batch["n_mod"]], [np.zeros(n, np.uint8)]
+    for t, letters in enumerate(groups, start=1):
+        cs = np.concatenate([[0], np.cumsum(np.isin(pep, np.frombuffer(letters.encode(), np.uint8)))])
+        r = np.flatnonzero((cs[off[1:]] - cs[off[:-1]] > 0) & (np.arange(n) >= skip_below))
+        rows.append(r); n_mod.append(np.ones(r.size, np.int32)); typ.append(np.full(r.size, t, np.uint8))
+    rows, n_mod, typ = np.concatenate(rows), np.concatenate(n_mod), np.concatenate(typ)
+    order = np.lexsort((typ, rows))
+    return select_rows(batch, rows[order], n_mod[order]), np.ascontiguousarray(typ[order])
