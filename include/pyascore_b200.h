@@ -282,6 +282,60 @@ void pa_free_pinned(void* p);
 #define PA_PINNED_PORTABLE 2u
 void* pa_alloc_pinned_ex(int64_t bytes, uint32_t flags);
 
+/* ---- mzML spectra decoded on the GPU ----
+ * pa_mzml_index (host, no GPU) reads the XML structure of an mzML file held in memory; pa_decode_arrays decodes the
+ * binary arrays it lists (base64, zlib, dtype conversion) on the GPU, straight into CSR peak arrays.  Together they give
+ * what the stdlib reader gives for SpectraParser(path, "mzML").to_csr() (reference: spec_parsers.py:49-110, :175-282). */
+#define PA_MZML_F64 0          /* MS:1000523 */
+#define PA_MZML_F32 1          /* MS:1000521 */
+#define PA_MZML_I32 2          /* MS:1000519 */
+#define PA_MZML_I64 3          /* MS:1000522 */
+#define PA_MZML_ZLIB 1         /* pa_mzml_array.flags: MS:1000574 */
+#define PA_MZML_INTENSITY 2    /* pa_mzml_array.flags: intensity array (else m/z) */
+
+typedef struct {
+    int64_t text_off;   /* byte offset of the <binary> element's text in the file */
+    int64_t text_len;   /* its length in bytes */
+    int64_t out_off;    /* first element of the array in the output: spec_off of its spectrum */
+    int64_t count;      /* expected elements: arrayLength of the binaryDataArray, else defaultArrayLength of the spectrum */
+    int64_t spec;       /* its spectrum: position in the sorted index */
+    int32_t dtype;      /* PA_MZML_F64 .. PA_MZML_I64 */
+    int32_t flags;      /* PA_MZML_ZLIB | PA_MZML_INTENSITY */
+} pa_mzml_array;
+
+typedef struct {
+    int64_t n_spec;                  /* retained spectra (ms_level filter), stably sorted by scan */
+    const int64_t* scan;             /* [n_spec] scan= number of the id attribute, -1 without one */
+    const int32_t* ms_level;         /* [n_spec] */
+    const double* precursor_mz;      /* [n_spec] NaN = missing */
+    const int32_t* precursor_charge; /* [n_spec] 0 = missing */
+    const int64_t* spec_off;         /* [n_spec+1] peak ranges laid out from the expected counts */
+    int64_t n_arrays;                /* two per spectrum with both arrays (m/z then intensity, in spectrum order) */
+    const pa_mzml_array* arrays;
+} pa_mzml_index_t;
+
+/* Replaces the XML half of MzMLExtractor (spec_parsers.py:49-110) and SpectraParser._get_spectra (:175-282) for the
+ * `n` bytes of an mzML file at `bytes`: spectra of level ms_level (0 = all), referenceableParamGroup references resolved,
+ * sorted by scan (ties in file order).  Payloads of spectra the filter drops are skipped, never decoded.  Returns PA_OK
+ * and *out (free it with pa_mzml_index_free), or PA_ERR_ARG with the text in err[0, err_cap): for the files the stdlib
+ * reader rejects with a ValueError (several precursors, numpress) the same text, otherwise why this path refuses the
+ * file (markup inside <binary>, m/z and intensity counts that differ, a missing array length ...).  Needs no GPU. */
+int pa_mzml_index(const uint8_t* bytes, int64_t n, int32_t ms_level, pa_mzml_index_t** out, char* err, int32_t err_cap);
+void pa_mzml_index_free(pa_mzml_index_t* index);
+
+/* Decodes the n_arrays binary arrays of `arrays` (host memory) on CUDA device `device`: file_dev holds the file bytes on
+ * that device; array j goes to (PA_MZML_INTENSITY ? inten_out : mz_out)[out_off, out_off + count) as float64.
+ * status_out[j] (device): 0 = decoded, 1 = base64 text b64decode rejects (or refused: non-ASCII, '&', data after padding),
+ * 2 = a zlib stream zlib.decompress rejects, 3 = decoded length other than `count` elements.  *inexact_out (device) = 1
+ * when some decoded intensity is not exactly a float32 value.  Synchronous.  Returns PA_OK or a negative pa_status (text
+ * in err). */
+int pa_decode_arrays(int device, const uint8_t* file_dev, const pa_mzml_array* arrays, int64_t n_arrays, double* mz_out,
+                     double* inten_out, int32_t* status_out, int32_t* inexact_out, char* err, int32_t err_cap);
+
+/* The inflate core of pa_decode_arrays built for the CPU: zlib.decompress(in) into out[0, cap).  Returns the output
+ * length, -1 for a stream zlib rejects (header, blocks, truncation, Adler-32), -2 when the output exceeds cap. */
+int64_t pa_inflate_host(const uint8_t* in, int64_t n_in, uint8_t* out, int64_t cap);
+
 /* Library/ABI version. */
 int pa_version(void);
 

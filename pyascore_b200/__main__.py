@@ -7,14 +7,15 @@
     format rows, write the TSV (same columns and number formatting)
 
 With --extra_mod, the spectra are parsed once and each batch holds the rows of every modification type, scored in
-one GPU call (score_typed); each type writes its own TSV.
+one GPU call (score_typed); each type writes its own TSV.  With --gpu_decode, the spectra of an mzML file are decoded on
+the GPU (SpectraParser.to_device) and every batch is scored from device memory.
 """
 import sys
 from datetime import datetime
 
 import numpy as np
 
-from .batch import MultiScorer, Scorer, score_typed
+from .batch import MultiScorer, Scorer, add_mod_off, score_typed
 from .config import args_from_file, build_parser, parse_extra_mod, validate_args
 from .parsing import (COMMON_MODS, IdentificationParser, MassCorrector, SpectraParser, iter_batches, result_rows,
                       score_stream, write_tsv)
@@ -59,6 +60,38 @@ def build_scorer(args):
     return scorer
 
 
+def read_spectra(args, log=print):
+    """The run's spectra: with --gpu_decode decoded on the GPU (--device), else -- or when that path refuses the file, which
+    is logged -- the pinned CSR block of the stdlib reader"""
+    parser = SpectraParser(args.spec_file, args.spec_file_type)
+    if getattr(args, "gpu_decode", False):
+        try:
+            return parser.to_device(args.device)
+        except ValueError as e:
+            log("{} -- GPU decoding refused, reading the spectra on the host: {}".format(_stamp(), e))
+    return parser.to_csr()
+
+
+def score_on_device(score, spectra):
+    """`score` (batch -> results) as the CLI calls it: unchanged for host spectra; for spectra on a GPU each batch's PSM
+    arrays go to that device, `score` takes the device-resident path and the results come back to the host"""
+    if isinstance(spectra.mz, np.ndarray):
+        return score
+    import torch
+    dev = spectra.mz.device
+
+    def run(batch):
+        add_mod_off(batch)
+        on_dev = {k: torch.from_numpy(v).to(dev) if isinstance(v, np.ndarray) else v for k, v in batch.items()}
+        torch.cuda.current_stream(dev).synchronize()
+        return {k: v.cpu().numpy() for k, v in score(on_dev).items()}
+    return run
+
+
+def _host_arrays(batch):
+    return {k: v if isinstance(v, np.ndarray) else v.cpu().numpy() for k, v in batch.items() if v is not None}
+
+
 def mod_types(args):
     """the modification types of a run: type 0 = --residues / --mod_mass / the neutral-loss flags / out_file, then one
     per --extra_mod"""
@@ -73,7 +106,7 @@ def run_typed(args, log=print):
     types = mod_types(args)
     log("{} -- Ascore Started".format(_stamp()))
     log("{} -- Reading spectra from: {}".format(_stamp(), args.spec_file))
-    spectra = SpectraParser(args.spec_file, args.spec_file_type).to_csr()
+    spectra = read_spectra(args, log)
     log("{} -- Reading identifications from: {}".format(_stamp(), args.ident_file))
     psms = [parse_identifications(args, t["residues"], t["mod_mass"]) for t in types]
     log("{} -- Anlyzing PSMs".format(_stamp()))
@@ -92,7 +125,8 @@ def run_typed(args, log=print):
                                types=[(t["residues"], t["mod_mass"]) for t in types],
                                mod_correction_tol=args.mod_correction_tol, zero_based=args.zero_based,
                                max_fragment_charge=args.max_fragment_charge, hit_depth=args.hit_depth)
-        for scans, batch, res in score_stream(lambda b: score_typed(scorers, b, b["psm_type"]), batches):
+        score = score_on_device(lambda b: score_typed(scorers, b, b["psm_type"]), spectra)
+        for scans, batch, res in score_stream(score, batches):
             for t, sc in enumerate(scorers):
                 sel = np.flatnonzero(batch["psm_type"] == t)
                 rows[t].extend(result_rows(sc, scans, batch, res, rows_of=sel))
@@ -104,7 +138,7 @@ def run_typed(args, log=print):
             sc.close()
     if args.match_save and saved:
         scans, batch = saved[-1]
-        np.savez("dump_batch.npz", scans=scans, **{k: v for k, v in batch.items() if v is not None})
+        np.savez("dump_batch.npz", scans=scans, **_host_arrays(batch))
     for t, typ in enumerate(types):
         if len(rows[t]) != n_psm[t]:
             log("{} -- {} of {} PSMs of {} could not be scored (see the warnings) and have no row in the output".format(
@@ -119,7 +153,7 @@ def run(args, log=print):
         return run_typed(args, log)
     log("{} -- Ascore Started".format(_stamp()))
     log("{} -- Reading spectra from: {}".format(_stamp(), args.spec_file))
-    spectra = SpectraParser(args.spec_file, args.spec_file_type).to_csr()
+    spectra = read_spectra(args, log)
     log("{} -- Reading identifications from: {}".format(_stamp(), args.ident_file))
     psms = parse_identifications(args)
     log("{} -- Anlyzing PSMs".format(_stamp()))
@@ -132,7 +166,7 @@ def run(args, log=print):
     saved = []
     n_psm = 0
     try:
-        for scans, batch, res in score_stream(scorer, batches):
+        for scans, batch, res in score_stream(score_on_device(scorer.score_batch, spectra), batches):
             rows.extend(result_rows(scorer, scans, batch, res))
             n_psm += int(scans.size)
             if args.match_save:
@@ -141,7 +175,7 @@ def run(args, log=print):
         scorer.close()
     if args.match_save and saved:
         scans, batch = saved[-1]
-        np.savez("dump_batch.npz", scans=scans, **{k: v for k, v in batch.items() if v is not None})
+        np.savez("dump_batch.npz", scans=scans, **_host_arrays(batch))
     if len(rows) != n_psm:
         # the reference would have written a row for these (or crashed on them): make the difference visible
         log("{} -- {} of {} PSMs could not be scored (see the warnings) and have no row in the output".format(

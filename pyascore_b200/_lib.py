@@ -35,6 +35,16 @@ class PaResults(C.Structure):
                 ("alt_sites", vp), ("psm_status", vp)]
 
 
+class PaMzmlArray(C.Structure):
+    _fields_ = [("text_off", C.c_int64), ("text_len", C.c_int64), ("out_off", C.c_int64), ("count", C.c_int64),
+                ("spec", C.c_int64), ("dtype", C.c_int32), ("flags", C.c_int32)]
+
+
+class PaMzmlIndex(C.Structure):
+    _fields_ = [("n_spec", C.c_int64), ("scan", vp), ("ms_level", vp), ("precursor_mz", vp), ("precursor_charge", vp),
+                ("spec_off", vp), ("n_arrays", C.c_int64), ("arrays", C.POINTER(PaMzmlArray))]
+
+
 class PaCounters(C.Structure):
     _fields_ = [(n, C.c_int64) for n in ("n_psm", "n_spec", "n_peaks", "n_retained", "n_isoforms",
                                          "n_fragment_lookups", "bytes_h2d", "bytes_d2h", "kernel_launches")] + \
@@ -48,7 +58,8 @@ EXPORTS = ["pa_create", "pa_add_neutral_loss", "pa_destroy", "pa_last_error", "p
            "pa_fetch_pep_scores", "pa_calculate_ambiguity", "pa_format_sequence", "pa_site_positions",
            "pa_bin_spectra", "pa_tail_table", "pa_counters", "pa_alloc_pinned", "pa_free_pinned", "pa_version",
            "pa_create_binner", "pa_bin_spectra_ex", "pa_fragment_table", "pa_site_determining_ions", "pa_log_math",
-           "pa_power_set_sums", "pa_score_range", "pa_score_batch_async", "pa_wait", "pa_shard_ranges", "pa_shard_ranges_for", "pa_alloc_pinned_ex", "pa_narrow_mz", "pa_score_typed"]
+           "pa_power_set_sums", "pa_score_range", "pa_score_batch_async", "pa_wait", "pa_shard_ranges", "pa_shard_ranges_for", "pa_alloc_pinned_ex", "pa_narrow_mz", "pa_score_typed",
+           "pa_mzml_index", "pa_mzml_index_free", "pa_decode_arrays", "pa_inflate_host"]
 
 _lib = None
 
@@ -121,6 +132,14 @@ def load():
     L.pa_log_math.argtypes = [vp, C.c_int32, C.c_int32, vp, vp, vp, vp, C.c_float, vp]
     L.pa_power_set_sums.restype = C.c_int64
     L.pa_power_set_sums.argtypes = [vp, C.c_int32, C.c_int32, vp, C.c_int64]
+    L.pa_mzml_index.restype = C.c_int
+    L.pa_mzml_index.argtypes = [vp, C.c_int64, C.c_int32, C.POINTER(C.POINTER(PaMzmlIndex)), C.c_char_p, C.c_int32]
+    L.pa_mzml_index_free.restype = None
+    L.pa_mzml_index_free.argtypes = [C.POINTER(PaMzmlIndex)]
+    L.pa_decode_arrays.restype = C.c_int
+    L.pa_decode_arrays.argtypes = [C.c_int, vp, vp, C.c_int64, vp, vp, vp, vp, C.c_char_p, C.c_int32]
+    L.pa_inflate_host.restype = C.c_int64
+    L.pa_inflate_host.argtypes = [vp, C.c_int64, vp, C.c_int64]
     _lib = L
     return L
 

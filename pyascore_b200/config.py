@@ -1,6 +1,7 @@
 """Command-line options of `python -m pyascore_b200`: the reference's flag set
 (pyascore/config.py:19-93: same names, types and defaults, so parameter files and scripts carry
-over) plus `--device` / `--chunk_psms` for the GPU pipeline and `--extra_mod` for more modification types per run."""
+over) plus `--device` / `--chunk_psms` for the GPU pipeline, `--extra_mod` for more modification types per run and `--gpu_decode`
+to decode mzML spectra on the GPU."""
 import argparse
 import re
 
@@ -27,6 +28,9 @@ _OPTIONS = [
 ]
 
 
+_SWITCHES = ("gpu_decode",)     # flags without a value on the command line
+
+
 def args_from_file(file_path):
     """'name = value' lines ('#' starts a comment) -> ['--name', 'value', ...] (config.py:5-17)"""
     out = []
@@ -34,7 +38,10 @@ def args_from_file(file_path):
         for line in src:
             m = re.search(r"^([^\s]+)\s*=\s*([^\s]+)$", line.split("#")[0].strip())
             if m is not None:
-                out += ["--" + m.group(1), m.group(2)]
+                if m.group(1) in _SWITCHES:          # 'gpu_decode = 1' turns the switch on, '= 0' leaves it off
+                    out += ["--" + m.group(1)] if m.group(2) not in ("0", "False", "false") else []
+                else:
+                    out += ["--" + m.group(1), m.group(2)]
     return out
 
 
@@ -57,6 +64,11 @@ def build_parser():
                         "spectra are read, copied and binned once for all types). NL_GROUPS / NL_MASSES are comma "
                         "separated as in --neutral_loss_groups / --neutral_loss_masses. Repeatable; in a parameter "
                         "file, one 'extra_mod = ...' line per type. Not combinable with --devices.")
+    p.add_argument("--gpu_decode", action="store_true",
+                   help="Decode the mzML spectra on the GPU (--device): the host reads the XML structure, the GPU the "
+                        "binary arrays, and every batch is scored from device memory. Same output; a file this path "
+                        "cannot decode exactly is read by the standard reader instead. 'gpu_decode = 1' in a parameter "
+                        "file. Not combinable with --devices or mzXML.")
     p.add_argument("spec_file", type=str, help="MS spectra file.")
     p.add_argument("ident_file", type=str, help="Results of the database search.")
     p.add_argument("out_file", type=str, help="Destination of the tab-separated results.")
@@ -105,6 +117,12 @@ def validate_args(args):
     if extra and getattr(args, "devices", ""):
         raise ValueError("--extra_mod cannot be combined with --devices: a run with several modification types "
                          "scores on one GPU (choose it with --device)")
+    if getattr(args, "gpu_decode", False):
+        if getattr(args, "devices", ""):
+            raise ValueError("--gpu_decode cannot be combined with --devices: the spectra are decoded into the memory of "
+                             "one GPU (choose it with --device)")
+        if args.spec_file_type != "mzML":
+            raise ValueError("--gpu_decode reads mzML files only, not {}".format(args.spec_file_type))
     allowed_fragments = "cbyzZ"
     for frag in args.fragment_types:
         if frag not in allowed_fragments:

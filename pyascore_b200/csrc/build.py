@@ -12,7 +12,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 OUT = os.path.join(os.path.dirname(HERE), "libpyascore_b200.so")
-SRCS = ["pa_lib.cu", "pa_host.cpp"]
+SRCS = ["pa_lib.cu", "pa_host.cpp", "pa_decode.cu", "pa_mzml.cpp"]
 DEPS = sorted(f for f in os.listdir(HERE) if f.endswith((".cu", ".cuh", ".cpp"))) + ["../../include/pyascore_b200.h"]
 
 

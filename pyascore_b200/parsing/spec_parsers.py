@@ -112,3 +112,16 @@ class SpectraParser:
         pmz = np.array([np.nan if r["precursor_mz"] is None else r["precursor_mz"] for r in recs], np.float64)
         pz = np.array([0 if r["precursor_charge"] is None else r["precursor_charge"] for r in recs], np.int32)
         return SpectraCSR(scans, pmz, pz, spec_off, mz, None if narrow else inten, inten if narrow else None)
+
+    def to_device(self, device=0, narrow_intensity=True):
+        """The CSR block of `to_csr(narrow_intensity=...)`, bit for bit, decoded on CUDA device `device`: the host reads
+        the XML structure only, the GPU decodes the binary arrays (parsing/mzml_gpu.py).  `spec_off`, `mz` and `inten` /
+        `inten32` are CUDA tensors; `scans`, `precursor_mz` and `precursor_charge` numpy arrays.  mzML only, without a
+        custom_filter (it runs on decoded arrays in Python); a file this path cannot decode exactly as the stdlib reader
+        does raises ValueError with the reason, and `to_csr()` reads it."""
+        if self._reader is not _xml.iter_mzml:
+            raise ValueError("to_device decodes mzML files only; read mzXML with to_csr()")
+        if self.custom_filter is not None:
+            raise ValueError("to_device cannot apply a custom_filter (it runs in Python on decoded arrays); use to_csr()")
+        from .mzml_gpu import mzml_to_device
+        return mzml_to_device(self._path, self.ms_level, device, narrow_intensity)
